@@ -276,6 +276,35 @@ def oracle_stream_digests(words, n_reads, threads, slab=1_000_000):
     return (xa, sa), (xh, sh)
 
 
+DUMP_SAMPLE = 1 << 20  # k-mers per stream written by --dump-outputs: 5 float64 arrays of 8 MiB
+DUMP_SEED = 20240611
+
+
+def dump_outputs(path, ctx, d_canon, d_hash, n_kmers):
+    """Writes what the timed call returned, for comparing two builds output for output: a fixed seeded sample of
+    DUMP_SAMPLE k-mer positions (all of them for a smaller run) of the canonical and the hash stream, and the
+    fingerprints of both full streams.  A u64 is split into its upper and lower 32 bits, each exact as a float64."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    if n_kmers <= DUMP_SAMPLE:
+        idx = np.arange(n_kmers, dtype=np.int64)
+    else:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n_kmers, DUMP_SAMPLE, replace=False)).astype(np.int64)
+    d_idx = torch.from_numpy(idx).cuda()
+
+    def halves(x):
+        x = np.asarray(x, dtype=np.uint64)
+        return (x >> np.uint64(32)).astype(np.float64), (x & np.uint64(0xFFFFFFFF)).astype(np.float64)
+    arrays = {"kmer_index": idx.astype(np.float64)}
+    for name, d in (("canon", d_canon), ("hash", d_hash)):
+        arrays[f"{name}_hi"], arrays[f"{name}_lo"] = halves(d[d_idx].cpu().numpy().view(np.uint64))
+    # rows: canonical xor, canonical wrapping sum, hash xor, hash wrapping sum; columns: upper, lower 32 bits
+    dg = [*ctx.digest(d_canon.data_ptr(), n_kmers), *ctx.digest(d_hash.data_ptr(), n_kmers)]
+    arrays["stream_digest"] = np.stack(halves(dg), axis=1)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def splitmix_words(first, count, seed):
     """words[first : first + count) of the counter-based stream word[j] = splitmix64(seed + j)."""
     out = np.empty(count, dtype=np.uint64)
@@ -558,6 +587,8 @@ def run_ours(args, rank, local_rank, world):
     kernel_ms = [a.elapsed_time(b) for a, b in ev]
     clocks = sampler.stop(wall0, wall1) if rank == 0 else None
     assert res.n_written == n_kmers
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ctx, d_canon, d_hash, n_kmers)
 
     # The same launch with idle gaps (outside the timed region, reported beside the roofline): back to back the
     # kernel runs into the board's power cap and the SM clock drops (tools/diag_power.py: 1000 W, ~1650 of 1965 MHz);
@@ -814,7 +845,13 @@ def main():
     ap.add_argument("--leg-steps", type=int, default=10)
     ap.add_argument("--c5-reads", type=int, default=25_000_000, help="reads per GPU of the c5 leg")
     ap.add_argument("--c5-bits", type=int, default=28)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write rank 0's outputs of the last step as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
