@@ -260,6 +260,18 @@ int32_t kmc_kmer_table_merge(kmc_ctx *ctx, uint64_t *keys, uint32_t *vals, uint3
 /* The table's entries as two dense device arrays (unordered); *n_out = how many. */
 int32_t kmc_kmer_table_export(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
                               uint64_t *out_keys, uint32_t *out_vals, uint64_t capacity, uint64_t *n_out);
+/* The same table for two-limb k-mers: forward (KMC_FW, K = 33..63) or canonical (KMC_CANON, K = 33..64) k-mers of a
+ * 2-bit source.  keys: device u64[2^log2_capacity][2], 16-byte aligned, each entry Kmer{A,K,2}.data (head limb
+ * first, unused top bits of limb 0 zero); free slot = both limbs ~0 (initialise with kmc_memset(keys, 0xff, 16 << cap));
+ * vals u32[2^log2_capacity] (zeroed).  fx_hash of the k-mer picks the slot, linear probing; a free slot is claimed
+ * with one 128-bit compare-and-swap.  Results and status as for kmc_kmer_count. */
+int32_t kmc_kmer_count2(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t mode, uint64_t *keys /* [2^cap][2] */,
+                        uint32_t *vals, uint32_t log2_capacity, kmc_result *result);
+/* kmc_kmer_table_merge / kmc_kmer_table_export of two-limb tables: src_keys u64[n_src][2], out_keys u64[capacity][2] */
+int32_t kmc_kmer_table2_merge(kmc_ctx *ctx, uint64_t *keys, uint32_t *vals, uint32_t log2_capacity,
+                              const uint64_t *src_keys /* [n_src][2] */, const uint32_t *src_vals, uint64_t n_src, uint64_t *n_new);
+int32_t kmc_kmer_table2_export(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
+                               uint64_t *out_keys /* [capacity][2] */, uint32_t *out_vals, uint64_t capacity, uint64_t *n_out);
 
 /* ---- multi-GPU (SURVEY.md 8b / 8e) ---------------------------------------------------------------
  * The reference has no collective (it is single-threaded Julia); north_star shards reads over the GPUs of a box
@@ -294,6 +306,11 @@ int32_t kmc_bucket_count_merge(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, in
 uint32_t kmc_kmer_owner(uint64_t key, uint32_t n_ranks);
 int32_t kmc_kmer_table_exchange(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
                                 uint64_t *owned_keys, uint32_t *owned_vals, uint32_t owned_log2_capacity, uint64_t *n_owned);
+/* The same for two-limb tables (kmc_kmer_count2): the owner of {limb0, limb1} is the same second mix taken over
+ * fx_hash of both limbs; entries travel as 2n u64, the owner merges with kmc_kmer_table2_merge. */
+uint32_t kmc_kmer_owner2(uint64_t limb0, uint64_t limb1, uint32_t n_ranks);
+int32_t kmc_kmer_table2_exchange(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
+                                 uint64_t *owned_keys, uint32_t *owned_vals, uint32_t owned_log2_capacity, uint64_t *n_owned);
 
 /* devices == NULL selects devices 0 .. n-1 */
 int32_t kmc_group_create(int32_t n, const int32_t *devices, kmc_group **group);
@@ -317,6 +334,9 @@ int32_t kmc_group_extract_host(kmc_group *group, const kmc_seqs *host_seqs, int3
 int32_t kmc_group_kmer_table_exchange(kmc_group *group, const uint64_t *const *keys, const uint32_t *const *vals,
                                       uint32_t log2_capacity, uint64_t *const *owned_keys, uint32_t *const *owned_vals,
                                       uint32_t owned_log2_capacity, uint64_t *n_owned);
+int32_t kmc_group_kmer_table2_exchange(kmc_group *group, const uint64_t *const *keys, const uint32_t *const *vals,
+                                       uint32_t log2_capacity, uint64_t *const *owned_keys, uint32_t *const *owned_vals,
+                                       uint32_t owned_log2_capacity, uint64_t *n_owned);
 
 /* XOR and wrapping sum of n u64 words in device memory -> out[0], out[1] (host).  A cheap
  * fingerprint of a device-resident stream: parity checks and result read-back at sizes where

@@ -698,36 +698,47 @@ function minimizers(it::Union{FwKmers{A, K}, CanonicalKmers{A, K}}, W::Integer; 
 end
 
 """
-    count_kmers(FwKmers{A,K}(seq) | CanonicalKmers{A,K}(seq); log2_capacity) -> Dict{Kmer{A,K,1}, Int}
+    count_kmers(FwKmers{A,K}(seq) | CanonicalKmers{A,K}(seq); log2_capacity) -> Dict{Kmer{A,K,N}, Int}
 
 Exact k-mer counts -- the `Dict` a loop over the iterator would build -- through `kmc_kmer_count` (open addressing
-in device memory keyed by the k-mer, K <= 31, or K = 32 for canonical k-mers) and `kmc_kmer_table_export`.
+in device memory keyed by the k-mer, K <= 31, or K = 32 for canonical k-mers) and `kmc_kmer_table_export`; two-limb
+k-mers (K = 33..63, or K = 64 for canonical k-mers) through `kmc_kmer_count2` and `kmc_kmer_table2_export`.
 `log2_capacity` defaults to twice the number of windows, rounded up to a power of two.
 """
 function count_kmers(it::Union{FwKmers{A, K}, CanonicalKmers{A, K}};
         log2_capacity::Integer = max(10, ceil(Int, log2(2 * max(1, length(source(it)))))),
         ctx::Context = default_context()) where {A <: NucleicAcidAlphabet{2}, K}
-    K <= 32 || throw(ArgumentError("count_kmers handles one-limb k-mers (K <= 32)"))
+    K <= 64 || throw(ArgumentError("count_kmers handles k-mers of one or two limbs (K <= 64)"))
     T = derive_type(Kmer{A, K})
+    N = K <= 32 ? 1 : 2                         # UInt64 limbs per key
     slots = 1 << log2_capacity
     res = KmcResult()
-    dk, dv = DeviceVector{UInt64}(ctx, slots), DeviceVector{UInt32}(ctx, slots)
-    zero!(dk, 0xff)   # free slot = ~0
+    dk, dv = DeviceVector{UInt64}(ctx, N * slots), DeviceVector{UInt32}(ctx, slots)
+    zero!(dk, 0xff)   # free slot = ~0 in every limb
     zero!(dv)
     with_device_sequence(ctx, source(it)) do d
-        st = ccall((:kmc_kmer_count, LIB[]), Int32,
-            (Ptr{Cvoid}, Ptr{KmcSeqs}, Int32, Int32, Ptr{Cvoid}, Ptr{Cvoid}, UInt32, Ref{KmcResult}),
-            ctx.handle, d, K, mode_of(typeof(it)), dk.ptr, dv.ptr, UInt32(log2_capacity), res)
+        st = N == 1 ?
+            ccall((:kmc_kmer_count, LIB[]), Int32,
+                (Ptr{Cvoid}, Ptr{KmcSeqs}, Int32, Int32, Ptr{Cvoid}, Ptr{Cvoid}, UInt32, Ref{KmcResult}),
+                ctx.handle, d, K, mode_of(typeof(it)), dk.ptr, dv.ptr, UInt32(log2_capacity), res) :
+            ccall((:kmc_kmer_count2, LIB[]), Int32,
+                (Ptr{Cvoid}, Ptr{KmcSeqs}, Int32, Int32, Ptr{Cvoid}, Ptr{Cvoid}, UInt32, Ref{KmcResult}),
+                ctx.handle, d, K, mode_of(typeof(it)), dk.ptr, dv.ptr, UInt32(log2_capacity), res)
         st == KMC_OK || throw_status(ctx, st, res, A)
     end
     n = Int(res.digest[1])                      # keys this call added = every key of a fresh table
-    ok, ov, nout = DeviceVector{UInt64}(ctx, n), DeviceVector{UInt32}(ctx, n), Ref{UInt64}(0)
-    check(ctx, ccall((:kmc_kmer_table_export, LIB[]), Int32,
-        (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, UInt32, Ptr{Cvoid}, Ptr{Cvoid}, UInt64, Ptr{UInt64}),
-        ctx.handle, dk.ptr, dv.ptr, UInt32(log2_capacity), ok.ptr, ov.ptr, n, nout))
+    ok, ov, nout = DeviceVector{UInt64}(ctx, N * n), DeviceVector{UInt32}(ctx, n), Ref{UInt64}(0)
+    check(ctx, N == 1 ?
+        ccall((:kmc_kmer_table_export, LIB[]), Int32,
+            (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, UInt32, Ptr{Cvoid}, Ptr{Cvoid}, UInt64, Ptr{UInt64}),
+            ctx.handle, dk.ptr, dv.ptr, UInt32(log2_capacity), ok.ptr, ov.ptr, n, nout) :
+        ccall((:kmc_kmer_table2_export, LIB[]), Int32,
+            (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, UInt32, Ptr{Cvoid}, Ptr{Cvoid}, UInt64, Ptr{UInt64}),
+            ctx.handle, dk.ptr, dv.ptr, UInt32(log2_capacity), ok.ptr, ov.ptr, n, nout))
     keys, vals = Array(ok), Array(ov)
     foreach(free!, (dk, dv, ok, ov))
-    kmers = reinterpret(T, keys)               # Kmer{A,K,1} is one UInt64 limb
+    # Kmer{A,K,N} is N UInt64 limbs, head first: the [N, n] export is a vector of n k-mers
+    kmers = reinterpret(T, keys)
     return Dict{T, Int}(kmers[i] => Int(vals[i]) for i in eachindex(vals))
 end
 

@@ -36,6 +36,25 @@ end
     @test sum(t) == length(s) - 10
 end
 
+@testset "count_kmers of two-limb k-mers (K = 33..64) == Dict loop" begin
+    genome = randdnaseq(RNG, 2_000)
+    s = LongDNA{2}(reduce(*, [genome[i:i+299] for i in rand(RNG, 1:1700, 20)]))   # repeated k-mers
+    for (K, canonical) in ((33, false), (47, true), (63, false), (63, true), (64, true))
+        it = canonical ? CanonicalDNAMers{K}(s) : FwDNAMers{K}(s)
+        want = Dict{eltype(it), Int}()
+        for m in it
+            want[m] = get(want, m, 0) + 1
+        end
+        got = KmersCUDA.count_kmers(it)
+        @test got == want
+        @test keytype(got) == Kmer{DNAAlphabet{2}, K, 2}
+    end
+    pal = LongDNA{2}("T"^32 * "A"^32)                  # its own reverse complement, head limb all ones
+    @test KmersCUDA.count_kmers(CanonicalDNAMers{64}(pal)) == Dict(first(CanonicalDNAMers{64}(pal)) => 1)
+    @test_throws ErrorException KmersCUDA.count_kmers(FwDNAMers{64}(s))   # KMC_E_UNSUPPORTED: all-T is {~0, ~0}
+    @test_throws ArgumentError KmersCUDA.count_kmers(CanonicalDNAMers{65}(s))
+end
+
 @testset "LongSubSeq views (reference: test/runtests.jl:154-169)" begin
     s2 = LongDNA{2}(randdnaseq(RNG, 1000))
     s4 = LongDNA{4}(s2); s4[500] = DNA_N

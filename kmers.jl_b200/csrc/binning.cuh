@@ -2,7 +2,8 @@
 //
 // Used where a table is too large for L2 and random updates to it would run at DRAM latency: the
 // updates are first sorted by the table slice they touch, then applied slice after slice
-// (buckets.cu: 32-bit bucket ids; sketch.cu: 64-bit k-mers of the exact count table).
+// (buckets.cu: 32-bit bucket ids; sketch.cu: 64-bit one-limb and 128-bit two-limb (ulonglong2) k-mers of the
+// exact count tables).
 //
 // One block owns a chunk of the input.  Pass 1 counts the chunk's keys per bin (count matrix
 // [bin][block]), an exclusive scan of the matrix gives every (bin, block) its place in the output, pass
@@ -28,6 +29,7 @@
 #include <type_traits>
 
 #include "kmc_internal.h"
+#include "table_keys.cuh"
 
 namespace kmc {
 namespace binning {
@@ -61,9 +63,15 @@ struct KmerHashBin {
     }
 };
 
+// bin of a two-limb k-mer: the high bits of the hash that picks its table slot (table_keys.cuh)
+struct KmerHashBin2 {
+    int shift; // 64 - P
+    __device__ __forceinline__ uint32_t operator()(ulonglong2 kmer) const { return static_cast<uint32_t>(key_hash(kmer) >> shift); }
+};
+
 // Loads this thread's keys of the iteration starting at it_base: warp w owns the keys [w * 32 * kPerThread,
 // + 32 * kPerThread) of the iteration as four rows of one 128-bit vector per lane.  `in` must be 16-byte
-// aligned; the tail of the array is loaded key by key.
+// aligned; the tail of the array is loaded key by key (16-byte keys: a row is one key).
 template <typename Key>
 __device__ __forceinline__ void load_iter(const Key *__restrict__ in, uint64_t n, uint64_t it_base,
                                           Key (&key)[Shape<Key>::kPerThread], uint32_t &ok_mask)
@@ -81,11 +89,15 @@ __device__ __forceinline__ void load_iter(const Key *__restrict__ in, uint64_t n
                 key[V * r + 1] = v.y;
                 key[V * r + 2] = v.z;
                 key[V * r + 3] = v.w;
-            } else {
+            } else if constexpr (sizeof(Key) == 8) {
                 key[V * r + 0] = (static_cast<uint64_t>(v.y) << 32) | v.x;
                 key[V * r + 1] = (static_cast<uint64_t>(v.w) << 32) | v.z;
+            } else {
+                key[r] = make_ulonglong2((static_cast<uint64_t>(v.y) << 32) | v.x, (static_cast<uint64_t>(v.w) << 32) | v.z);
             }
             ok_mask |= ((1u << V) - 1u) << (V * r);
+        } else if constexpr (V == 1) {
+            key[r] = Key{};
         } else {
 #pragma unroll
             for (int q = 0; q < V; ++q) {
@@ -165,7 +177,7 @@ template <typename Key> struct Scatter64Smem {
     uint32_t off[kTpGroups * 2][kBlock];  // keys of the bin held by the threads before this one: two 16-bit fields per
                                           // word, bin b in word [(b >> 2) * 2 + (b & 1)], field (b >> 1) & 1
     Key keys[Shape<Key>::kPerIter];
-    uint8_t bins[sizeof(Key) == 8 ? Shape<Key>::kPerIter : 16]; // 64-bit keys: the bin of every staged key
+    uint8_t bins[sizeof(Key) >= 8 ? Shape<Key>::kPerIter : 16]; // 64- and 128-bit keys: the bin of every staged key
     uint64_t dst[kTpBins];                // output index of staging slot 0 of each bin (wraps; only sums are used)
     uint64_t glob[kTpBins];               // where the block's next key of each bin goes
     uint32_t start[kTpBins + 1];
@@ -179,8 +191,12 @@ template <typename Key> __device__ __forceinline__ void st_binned(Key *p, Key v)
 {
     if constexpr (sizeof(Key) == 4)
         asm volatile("st.global.L1::no_allocate.L2::cache_hint.u32 [%0], %1, %2;" ::"l"(p), "r"(v), "l"(0x12F0000000000000ull) : "memory");
-    else
+    else if constexpr (sizeof(Key) == 8)
         asm volatile("st.global.L1::no_allocate.L2::cache_hint.u64 [%0], %1, %2;" ::"l"(p), "l"(v), "l"(0x12F0000000000000ull) : "memory");
+    else
+        asm volatile("st.global.L1::no_allocate.L2::cache_hint.v2.u64 [%0], {%1, %2}, %3;" ::"l"(p), "l"(v.x), "l"(v.y),
+                     "l"(0x12F0000000000000ull)
+                     : "memory");
 }
 
 // One iteration of the 64-bin scatter: the block's kPerIter keys (PT per thread, in registers) are counted per bin,
@@ -196,7 +212,7 @@ __device__ __forceinline__ void scatter64_iter(Scatter64Smem<Key> &sm, const Key
     using S = Shape<Key>;
     constexpr int PT = S::kPerThread;
     static_assert(PT * kBlock == S::kPerIter, "the write-out of a full iteration takes PT keys per thread");
-    constexpr bool kStageBins = sizeof(Key) == 8; // recomputing a hash bin at write-out costs more than a byte of staging
+    constexpr bool kStageBins = sizeof(Key) >= 8; // recomputing a hash bin at write-out costs more than a byte of staging
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll
     for (int g = 0; g < kTpGroups; ++g) sm.cnt[g][threadIdx.x] = 0;

@@ -25,6 +25,7 @@
 #include <vector>
 
 #include "plan.h"
+#include "table_keys.cuh"
 
 namespace kmc {
 
@@ -161,22 +162,27 @@ int32_t comm_finish_init(kmc_ctx *ctx, ncclComm_t comm, int rank, int n_ranks)
 }
 
 // ---- the exact k-mer table across GPUs: entries -> owner ranks ---------------------------------------------------
-constexpr uint64_t kEmptyKey = ~0ull;       // sketch.cu: a free slot of a k-mer table
+// (keys: uint64_t for one-limb tables, ulonglong2 for two-limb ones; table_keys.cuh)
 constexpr int kMaxRanks = 64;
 
 // The owner of a key: a second mix of its fx_hash (the table's slot is the TOP bits of fx_hash; an owner taken from
 // the same bits would leave every owner's table with a 1/n_ranks sliver of its slots in use), range-reduced by a
-// multiply-shift.  Host and device agree (kmc_kmer_owner).
-__host__ __device__ inline uint32_t owner_of(uint64_t key, uint32_t n_ranks)
+// multiply-shift.  Host and device agree (kmc_kmer_owner, kmc_kmer_owner2).
+__host__ __device__ inline uint32_t owner_of_hash(uint64_t h, uint32_t n_ranks)
 {
-    uint64_t h = key * FX_CONSTANT; // fx_hash of a one-limb k-mer with h0 = 0: (rotl(0,5) ^ key) * FX
     h ^= h >> 32;
     h *= 0x9E3779B97F4A7C15ull;
     return static_cast<uint32_t>(((h >> 32) * n_ranks) >> 32);
 }
+__host__ __device__ inline uint32_t owner_of(uint64_t key, uint32_t n_ranks)
+{
+    return owner_of_hash(key * FX_CONSTANT, n_ranks); // fx_hash of a one-limb k-mer with h0 = 0: (rotl(0,5) ^ key) * FX
+}
+__host__ __device__ inline uint32_t owner_of(ulonglong2 key, uint32_t n_ranks) { return owner_of_hash(key_hash(key), n_ranks); }
 
 // pass 1: entries per owner
-__global__ void __launch_bounds__(256) owner_count_kernel(const uint64_t *__restrict__ keys, uint64_t n_slots, uint32_t n_ranks,
+template <typename Key>
+__global__ void __launch_bounds__(256) owner_count_kernel(const Key *__restrict__ keys, uint64_t n_slots, uint32_t n_ranks,
                                                           unsigned long long *__restrict__ counts)
 {
     __shared__ uint32_t s_cnt[kMaxRanks];
@@ -184,8 +190,8 @@ __global__ void __launch_bounds__(256) owner_count_kernel(const uint64_t *__rest
     __syncthreads();
     for (uint64_t i = static_cast<uint64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < n_slots;
          i += static_cast<uint64_t>(gridDim.x) * blockDim.x) {
-        const uint64_t key = keys[i];
-        if (key != kEmptyKey) atomicAdd(s_cnt + owner_of(key, n_ranks), 1u);
+        const Key key = keys[i];
+        if (!key_free(key)) atomicAdd(s_cnt + owner_of(key, n_ranks), 1u);
     }
     __syncthreads();
     if (threadIdx.x < n_ranks && s_cnt[threadIdx.x]) atomicAdd(counts + threadIdx.x, static_cast<unsigned long long>(s_cnt[threadIdx.x]));
@@ -193,9 +199,10 @@ __global__ void __launch_bounds__(256) owner_count_kernel(const uint64_t *__rest
 
 // pass 2: the entries, grouped by owner (segment o starts at base[o]); one block reserves a run per owner for the
 // chunk of slots it handles, so the global cursors see one atomic per (block, chunk, owner)
-__global__ void __launch_bounds__(256) owner_scatter_kernel(const uint64_t *__restrict__ keys, const uint32_t *__restrict__ vals,
+template <typename Key>
+__global__ void __launch_bounds__(256) owner_scatter_kernel(const Key *__restrict__ keys, const uint32_t *__restrict__ vals,
                                                             uint64_t n_slots, uint32_t n_ranks, const uint64_t *__restrict__ base,
-                                                            unsigned long long *__restrict__ cursor, uint64_t *__restrict__ out_keys,
+                                                            unsigned long long *__restrict__ cursor, Key *__restrict__ out_keys,
                                                             uint32_t *__restrict__ out_vals)
 {
     __shared__ uint32_t s_cnt[kMaxRanks];
@@ -205,13 +212,16 @@ __global__ void __launch_bounds__(256) owner_scatter_kernel(const uint64_t *__re
     for (uint64_t c0 = static_cast<uint64_t>(blockIdx.x) * chunk; c0 < n_slots; c0 += static_cast<uint64_t>(gridDim.x) * chunk) {
         if (threadIdx.x < kMaxRanks) s_cnt[threadIdx.x] = 0;
         __syncthreads();
-        uint64_t key[kPer];
+        Key key[kPer];
         uint32_t val[kPer], own[kPer], rank[kPer];
 #pragma unroll
         for (int j = 0; j < kPer; ++j) {
             const uint64_t i = c0 + static_cast<uint64_t>(j) * 256 + threadIdx.x;
-            key[j] = i < n_slots ? keys[i] : kEmptyKey;
-            if (key[j] != kEmptyKey) {
+            if constexpr (sizeof(Key) == 8)
+                key[j] = i < n_slots ? keys[i] : kEmptyKey;
+            else
+                key[j] = i < n_slots ? keys[i] : make_ulonglong2(kEmptyKey, kEmptyKey);
+            if (!key_free(key[j])) {
                 val[j] = vals[i];
                 own[j] = owner_of(key[j], n_ranks);
                 rank[j] = atomicAdd(s_cnt + own[j], 1u);
@@ -223,7 +233,7 @@ __global__ void __launch_bounds__(256) owner_scatter_kernel(const uint64_t *__re
         __syncthreads();
 #pragma unroll
         for (int j = 0; j < kPer; ++j)
-            if (key[j] != kEmptyKey) {
+            if (!key_free(key[j])) {
                 const uint64_t at = s_base[own[j]] + rank[j];
                 out_keys[at] = key[j];
                 out_vals[at] = val[j];
@@ -232,7 +242,7 @@ __global__ void __launch_bounds__(256) owner_scatter_kernel(const uint64_t *__re
     }
 }
 
-// what one local rank holds during an exchange
+// what one local rank holds during an exchange (keys: n_limbs u64 per entry)
 struct ExchangeRank {
     kmc_ctx *ctx;
     const uint64_t *keys;
@@ -246,9 +256,11 @@ struct ExchangeRank {
 
 // The exchange for the local ranks `rs` (one per context of this process: all of the communicator's ranks in the
 // single-process group, exactly one under one-process-per-GPU launchers).  Every rank of the communicator must make
-// the call (it is a collective).
+// the call (it is a collective).  Key: uint64_t (one-limb tables) or ulonglong2 (two-limb tables, sent as 2n u64).
+template <typename Key>
 int32_t table_exchange(std::vector<ExchangeRank> &rs, uint32_t log2_capacity, uint32_t owned_log2_capacity, uint64_t *n_owned)
 {
+    constexpr uint64_t NL = sizeof(Key) / 8;
     kmc_ctx *c0 = rs[0].ctx;
     int32_t st = need_nccl(c0);
     if (st) return st;
@@ -267,7 +279,8 @@ int32_t table_exchange(std::vector<ExchangeRank> &rs, uint32_t log2_capacity, ui
         CU(r.matrix_dev.alloc(ctx, 8ull * n_ranks * n_ranks, s));
         CU(cudaMemsetAsync(r.counts_dev.p, 0, 8 * n_ranks, s));
         const uint64_t blocks = std::min<uint64_t>((n_slots + 255) / 256, static_cast<uint64_t>(ctx->sm_count) * 16);
-        owner_count_kernel<<<static_cast<unsigned>(blocks), 256, 0, s>>>(r.keys, n_slots, n_ranks, r.counts_dev.as<unsigned long long>());
+        owner_count_kernel<Key><<<static_cast<unsigned>(blocks), 256, 0, s>>>(reinterpret_cast<const Key *>(r.keys), n_slots, n_ranks,
+                                                                             r.counts_dev.as<unsigned long long>());
         CU(cudaGetLastError());
     }
     if (grouped) NC(c0, N.GroupStart());
@@ -304,18 +317,18 @@ int32_t table_exchange(std::vector<ExchangeRank> &rs, uint32_t log2_capacity, ui
             if (q != me) r.n_recv += r.matrix[static_cast<size_t>(q) * n_ranks + me];
         CU(r.base_dev.alloc(ctx, 8 * (n_ranks + 1), s));
         CU(r.cursor_dev.alloc(ctx, 8 * n_ranks, s));
-        CU(r.send_keys.alloc(ctx, 8 * r.n_entries, s));
+        CU(r.send_keys.alloc(ctx, 8 * NL * r.n_entries, s));
         CU(r.send_vals.alloc(ctx, 4 * r.n_entries, s));
-        CU(r.recv_keys.alloc(ctx, 8 * r.n_recv, s));
+        CU(r.recv_keys.alloc(ctx, 8 * NL * r.n_recv, s));
         CU(r.recv_vals.alloc(ctx, 4 * r.n_recv, s));
         // (base is a host vector that dies with this iteration: a synchronous copy)
         CU(cudaMemcpyAsync(r.base_dev.p, base.data(), 8 * (n_ranks + 1), cudaMemcpyHostToDevice, s));
         CU(cudaStreamSynchronize(s));
         CU(cudaMemsetAsync(r.cursor_dev.p, 0, 8 * n_ranks, s));
         const uint64_t blocks = std::min<uint64_t>((n_slots + 2047) / 2048, static_cast<uint64_t>(ctx->sm_count) * 8);
-        owner_scatter_kernel<<<static_cast<unsigned>(blocks), 256, 0, s>>>(r.keys, r.vals, n_slots, n_ranks, r.base_dev.as<uint64_t>(),
-                                                                          r.cursor_dev.as<unsigned long long>(),
-                                                                          r.send_keys.as<uint64_t>(), r.send_vals.as<uint32_t>());
+        owner_scatter_kernel<Key><<<static_cast<unsigned>(blocks), 256, 0, s>>>(
+            reinterpret_cast<const Key *>(r.keys), r.vals, n_slots, n_ranks, r.base_dev.as<uint64_t>(), r.cursor_dev.as<unsigned long long>(),
+            r.send_keys.as<Key>(), r.send_vals.as<uint32_t>());
         CU(cudaGetLastError());
     }
 
@@ -329,13 +342,13 @@ int32_t table_exchange(std::vector<ExchangeRank> &rs, uint32_t log2_capacity, ui
         for (uint32_t q = 0; q < n_ranks; ++q) {
             const uint64_t ns = r.counts[q];
             if (q != me && ns) {
-                NC(ctx, N.Send(r.send_keys.as<uint64_t>() + send_at, ns, ncclUint64, static_cast<int>(q), ctx->comm->comm, ctx->stream));
+                NC(ctx, N.Send(r.send_keys.as<uint64_t>() + NL * send_at, NL * ns, ncclUint64, static_cast<int>(q), ctx->comm->comm, ctx->stream));
                 NC(ctx, N.Send(r.send_vals.as<uint32_t>() + send_at, ns, ncclUint32, static_cast<int>(q), ctx->comm->comm, ctx->stream));
             }
             send_at += ns;
             const uint64_t nr = q != me ? r.matrix[static_cast<size_t>(q) * n_ranks + me] : 0;
             if (nr) {
-                NC(ctx, N.Recv(r.recv_keys.as<uint64_t>() + recv_at, nr, ncclUint64, static_cast<int>(q), ctx->comm->comm, ctx->stream));
+                NC(ctx, N.Recv(r.recv_keys.as<uint64_t>() + NL * recv_at, NL * nr, ncclUint64, static_cast<int>(q), ctx->comm->comm, ctx->stream));
                 NC(ctx, N.Recv(r.recv_vals.as<uint32_t>() + recv_at, nr, ncclUint32, static_cast<int>(q), ctx->comm->comm, ctx->stream));
                 recv_at += nr;
             }
@@ -351,11 +364,12 @@ int32_t table_exchange(std::vector<ExchangeRank> &rs, uint32_t log2_capacity, ui
         uint64_t own0 = 0;
         for (uint32_t o = 0; o < me; ++o) own0 += r.counts[o];
         uint64_t added = 0, a2 = 0;
-        st = kmc_kmer_table_merge(ctx, r.owned_keys, r.owned_vals, owned_log2_capacity, r.send_keys.as<uint64_t>() + own0,
-                                  r.send_vals.as<uint32_t>() + own0, r.counts[me], &added);
+        auto merge = NL == 1 ? kmc_kmer_table_merge : kmc_kmer_table2_merge;
+        st = merge(ctx, r.owned_keys, r.owned_vals, owned_log2_capacity, r.send_keys.as<uint64_t>() + NL * own0,
+                   r.send_vals.as<uint32_t>() + own0, r.counts[me], &added);
         if (st) return st;
-        st = kmc_kmer_table_merge(ctx, r.owned_keys, r.owned_vals, owned_log2_capacity, r.recv_keys.as<uint64_t>(),
-                                  r.recv_vals.as<uint32_t>(), r.n_recv, &a2);
+        st = merge(ctx, r.owned_keys, r.owned_vals, owned_log2_capacity, r.recv_keys.as<uint64_t>(), r.recv_vals.as<uint32_t>(),
+                   r.n_recv, &a2);
         if (st) return st;
         if (n_owned) n_owned[i] = added + a2;
     }
@@ -564,13 +578,23 @@ int32_t kmc_bucket_count_merge(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, in
 
 uint32_t kmc_kmer_owner(uint64_t key, uint32_t n_ranks) { return n_ranks ? owner_of(key, n_ranks) : 0; }
 
-int32_t kmc_kmer_table_exchange(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
-                                uint64_t *owned_keys, uint32_t *owned_vals, uint32_t owned_log2_capacity, uint64_t *n_owned)
+uint32_t kmc_kmer_owner2(uint64_t limb0, uint64_t limb1, uint32_t n_ranks)
+{
+    return n_ranks ? owner_of(make_ulonglong2(limb0, limb1), n_ranks) : 0;
+}
+
+} // extern "C"
+
+template <typename Key>
+static int32_t kmer_table_exchange(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity, uint64_t *owned_keys,
+                                   uint32_t *owned_vals, uint32_t owned_log2_capacity, uint64_t *n_owned)
 {
     if (!ctx) return KMC_E_BAD_ARG;
     if (!keys || !vals || !owned_keys || !owned_vals) return fail(ctx, KMC_E_BAD_ARG, "NULL table");
     if (log2_capacity < 1 || log2_capacity > 40 || owned_log2_capacity < 1 || owned_log2_capacity > 40)
         return fail(ctx, KMC_E_BAD_ARG, "log2_capacity must be in 1..40");
+    if (sizeof(Key) == 16 && (reinterpret_cast<uintptr_t>(keys) % 16 || reinterpret_cast<uintptr_t>(owned_keys) % 16))
+        return fail(ctx, KMC_E_BAD_ARG, "the two-limb keys must be 16-byte aligned");
     if (!ctx->comm) return fail(ctx, KMC_E_BAD_ARG, "the context has no communicator (kmc_comm_init_rank / kmc_group_create)");
     std::vector<ExchangeRank> rs(1);
     rs[0].ctx = ctx;
@@ -578,7 +602,47 @@ int32_t kmc_kmer_table_exchange(kmc_ctx *ctx, const uint64_t *keys, const uint32
     rs[0].vals = vals;
     rs[0].owned_keys = owned_keys;
     rs[0].owned_vals = owned_vals;
-    return table_exchange(rs, log2_capacity, owned_log2_capacity, n_owned);
+    return table_exchange<Key>(rs, log2_capacity, owned_log2_capacity, n_owned);
+}
+
+template <typename Key>
+static int32_t group_kmer_table_exchange(kmc_group *g, const uint64_t *const *keys, const uint32_t *const *vals, uint32_t log2_capacity,
+                                         uint64_t *const *owned_keys, uint32_t *const *owned_vals, uint32_t owned_log2_capacity,
+                                         uint64_t *n_owned)
+{
+    if (!g || !keys || !vals || !owned_keys || !owned_vals) return KMC_E_BAD_ARG;
+    const size_t n = g->ctx.size();
+    if (sizeof(Key) == 16)
+        for (size_t i = 0; i < n; ++i)
+            if (reinterpret_cast<uintptr_t>(keys[i]) % 16 || reinterpret_cast<uintptr_t>(owned_keys[i]) % 16)
+                return fail(g->ctx[i], KMC_E_BAD_ARG, "the two-limb keys must be 16-byte aligned");
+    if (n == 1) { // one owner: the exchange is a merge into the owned table
+        auto merge = sizeof(Key) == 8 ? kmc_kmer_table_merge : kmc_kmer_table2_merge;
+        return merge(g->ctx[0], owned_keys[0], owned_vals[0], owned_log2_capacity, keys[0], vals[0], 1ull << log2_capacity, n_owned);
+    }
+    std::vector<ExchangeRank> rs(n);
+    for (size_t i = 0; i < n; ++i) {
+        rs[i].ctx = g->ctx[i];
+        rs[i].keys = keys[i];
+        rs[i].vals = vals[i];
+        rs[i].owned_keys = owned_keys[i];
+        rs[i].owned_vals = owned_vals[i];
+    }
+    return table_exchange<Key>(rs, log2_capacity, owned_log2_capacity, n_owned);
+}
+
+extern "C" {
+
+int32_t kmc_kmer_table_exchange(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
+                                uint64_t *owned_keys, uint32_t *owned_vals, uint32_t owned_log2_capacity, uint64_t *n_owned)
+{
+    return kmer_table_exchange<uint64_t>(ctx, keys, vals, log2_capacity, owned_keys, owned_vals, owned_log2_capacity, n_owned);
+}
+
+int32_t kmc_kmer_table2_exchange(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
+                                 uint64_t *owned_keys, uint32_t *owned_vals, uint32_t owned_log2_capacity, uint64_t *n_owned)
+{
+    return kmer_table_exchange<ulonglong2>(ctx, keys, vals, log2_capacity, owned_keys, owned_vals, owned_log2_capacity, n_owned);
 }
 
 // ---- one process, several GPUs (what a Julia session is) -------------------------------------------------------------
@@ -703,21 +767,14 @@ int32_t kmc_group_kmer_table_exchange(kmc_group *g, const uint64_t *const *keys,
                                       uint64_t *const *owned_keys, uint32_t *const *owned_vals, uint32_t owned_log2_capacity,
                                       uint64_t *n_owned)
 {
-    if (!g || !keys || !vals || !owned_keys || !owned_vals) return KMC_E_BAD_ARG;
-    const size_t n = g->ctx.size();
-    if (n == 1) { // one owner: the exchange is a merge into the owned table
-        return kmc_kmer_table_merge(g->ctx[0], owned_keys[0], owned_vals[0], owned_log2_capacity, keys[0], vals[0],
-                                    1ull << log2_capacity, n_owned);
-    }
-    std::vector<ExchangeRank> rs(n);
-    for (size_t i = 0; i < n; ++i) {
-        rs[i].ctx = g->ctx[i];
-        rs[i].keys = keys[i];
-        rs[i].vals = vals[i];
-        rs[i].owned_keys = owned_keys[i];
-        rs[i].owned_vals = owned_vals[i];
-    }
-    return table_exchange(rs, log2_capacity, owned_log2_capacity, n_owned);
+    return group_kmer_table_exchange<uint64_t>(g, keys, vals, log2_capacity, owned_keys, owned_vals, owned_log2_capacity, n_owned);
+}
+
+int32_t kmc_group_kmer_table2_exchange(kmc_group *g, const uint64_t *const *keys, const uint32_t *const *vals, uint32_t log2_capacity,
+                                       uint64_t *const *owned_keys, uint32_t *const *owned_vals, uint32_t owned_log2_capacity,
+                                       uint64_t *n_owned)
+{
+    return group_kmer_table_exchange<ulonglong2>(g, keys, vals, log2_capacity, owned_keys, owned_vals, owned_log2_capacity, n_owned);
 }
 
 } // extern "C"

@@ -11,6 +11,8 @@
 //                       open-addressing table in device memory (fx_hash of the k-mer picks the slot,
 //                       linear probing, 64-bit compare-and-swap on the key, 32-bit add on the count);
 //                       kmc_kmer_table_merge / _export move entries between tables (multi-GPU merge)
+//   kmc_kmer_count2     the same table for two-limb k-mers, K = 33..64 (table_keys.cuh): 16-byte keys, claimed by
+//                       one 128-bit compare-and-swap; kmc_kmer_table2_merge / _export
 //
 // Both run consume_kernel: the same (read, group slot) work items, block load and static funnel
 // shifts as extract_kernel (kmer_core.cuh), with the stores replaced by a small functor.
@@ -30,14 +32,16 @@
 
 #include "binning.cuh"
 #include "plan.h"
+#include "table_keys.cuh"
 
 namespace kmc {
 
 namespace {
 
-enum : int { OP_HASH_HIST = 0, OP_HASH_BELOW = 1, OP_COMPOSITION = 2, OP_COMPOSITION_SHARED = 3, OP_TABLE = 4 };
+enum : int { OP_HASH_HIST = 0, OP_HASH_BELOW = 1, OP_COMPOSITION = 2, OP_COMPOSITION_SHARED = 3, OP_TABLE = 4, OP_TABLE2 = 5 };
 
-constexpr uint64_t kEmptyKey = ~0ull; // never a k-mer: K <= 31, or K = 32 canonical (the all-T 32-mer is not canonical)
+// kEmptyKey (table_keys.cuh) is never a k-mer: one limb, K <= 31, or K = 32 canonical (the all-T 32-mer is not
+// canonical); two limbs {~0, ~0}, K <= 63, or K = 64 canonical.
 
 // table[key] += inc.  Returns kTableFull when no slot is left, kTableNew when the key was not in the table
 // before.  Most k-mers of a read set are already in the table, so the slot is read before the
@@ -68,6 +72,35 @@ __device__ __forceinline__ int table_add(unsigned long long *keys, uint32_t *val
     return kTableFull;
 }
 
+// The same for a two-limb key.  The slot is read with one 16-byte load, but a vector load is not promised to be
+// single-copy atomic: a slot being claimed could be seen half written, and a half-written slot has a limb that is
+// still ~0.  So a slot with any ~0 limb is read again through the compare-and-swap itself, which claims it if it is
+// free and returns its true content otherwise (keys whose limbs are ~0 -- the all-T tail of a k-mer -- are rare).
+__device__ __forceinline__ int table_add(ulonglong2 *keys, uint32_t *vals, uint32_t log2cap, ulonglong2 key, uint64_t hash,
+                                         uint32_t inc)
+{
+    const uint64_t mask = (1ull << log2cap) - 1;
+    const ulonglong2 empty = make_ulonglong2(kEmptyKey, kEmptyKey);
+    uint64_t slot = hash >> (64 - log2cap);
+    for (uint64_t probes = 0; probes <= mask; ++probes) {
+        ulonglong2 cur = keys[slot];
+        int st = kTableCounted;
+        if (cur.x == kEmptyKey || cur.y == kEmptyKey) {
+            cur = atomicCAS(keys + slot, empty, key);
+            if (key_free(cur)) {
+                st = kTableNew;
+                cur = key;
+            }
+        }
+        if (cur.x == key.x && cur.y == key.y) {
+            atomicAdd(vals + slot, inc);
+            return st;
+        }
+        slot = (slot + 1) & mask;
+    }
+    return kTableFull;
+}
+
 // adds the new keys a thread has seen to *distinct: one atomic per warp (all 32 lanes must call)
 __device__ __forceinline__ void add_distinct(unsigned long long *distinct, uint32_t n_new)
 {
@@ -87,7 +120,8 @@ struct ConsumeParams {
     unsigned long long *keys;      // OP_TABLE: u64[2^log2cap] keys (kEmptyKey = free), vals = table
     uint32_t log2cap;
     unsigned long long *distinct;  // OP_TABLE: keys in the table
-    uint32_t *overflow;            // OP_TABLE: set when a k-mer found no slot
+    uint32_t *overflow;            // OP_TABLE*: set when a k-mer found no slot
+    ulonglong2 *keys2;             // OP_TABLE2: two-limb keys, ulonglong2[2^log2cap] ({~0, ~0} = free), vals = table
 };
 
 constexpr int kSharedCompositionMax = 4096; // 4^6 counters = 16 KB of shared memory
@@ -111,7 +145,7 @@ __global__ void __launch_bounds__(kBlockThreads) consume_kernel(const ExtractPar
     TileCursor<RAGGED, G> cur;
     if (!ALIGNED) cur.init(p, tile_base, sh, threadIdx.x); // (block-wide barriers inside: also orders the zeroing above)
     if (SHARED_HIST) __syncthreads();
-    uint32_t n_new = 0; // OP_TABLE: keys this thread put into the table
+    uint32_t n_new = 0; // OP_TABLE*: keys this thread put into the table
     const AlignedItems<G, 2> items(p);
     const uint32_t n_items32 = static_cast<uint32_t>(p.items);
     bool inside = false;
@@ -161,6 +195,11 @@ __global__ void __launch_bounds__(kBlockThreads) consume_kernel(const ExtractPar
                     const int st = table_add(c.keys, c.table, c.log2cap, a[N - 1], fx_hash<N>(a, 0), 1u);
                     if (st == kTableFull) *c.overflow = 1u;
                     n_new += st == kTableNew;
+                } else if (OP == OP_TABLE2) {
+                    const ulonglong2 key = make_ulonglong2(a[0], a[N - 1]);
+                    const int st = table_add(c.keys2, c.table, c.log2cap, key, key_hash(key), 1u);
+                    if (st == kTableFull) *c.overflow = 1u;
+                    n_new += st == kTableNew;
                 } else if (OP == OP_COMPOSITION) {
                     atomicAdd(c.table + a[N - 1], 1u); // as_integer(kmer): K <= 14, one limb
                 } else {
@@ -170,7 +209,7 @@ __global__ void __launch_bounds__(kBlockThreads) consume_kernel(const ExtractPar
         }
         if (!ALIGNED) cur.advance(p);
     }
-    if (OP == OP_TABLE) add_distinct(c.distinct, n_new);
+    if (OP == OP_TABLE || OP == OP_TABLE2) add_distinct(c.distinct, n_new);
     if (SHARED_HIST) {
         __syncthreads();
         for (uint32_t i = threadIdx.x; i < c.table_entries; i += kBlockThreads) {
@@ -230,18 +269,18 @@ ConsumeLaunchFn consume_launcher(const Geometry &ge, bool ragged, bool canon)
 }
 
 // every non-empty (key, count) of a source table / entry list into the destination table
-__global__ void __launch_bounds__(256) table_merge_kernel(unsigned long long *keys, uint32_t *vals, uint32_t log2cap,
-                                                          const unsigned long long *__restrict__ src_keys,
+// (Key: unsigned long long for one-limb tables, ulonglong2 for two-limb ones)
+template <typename Key>
+__global__ void __launch_bounds__(256) table_merge_kernel(Key *keys, uint32_t *vals, uint32_t log2cap, const Key *__restrict__ src_keys,
                                                           const uint32_t *__restrict__ src_vals, uint64_t n,
                                                           unsigned long long *distinct, uint32_t *overflow)
 {
     uint32_t n_new = 0;
     for (uint64_t i = static_cast<uint64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < n;
          i += static_cast<uint64_t>(gridDim.x) * blockDim.x) {
-        const uint64_t key = src_keys[i];
-        if (key == kEmptyKey) continue;
-        const uint64_t d[1] = {key};
-        const int st = table_add(keys, vals, log2cap, key, fx_hash<1>(d, 0), src_vals[i]);
+        const Key key = src_keys[i];
+        if (key_free(key)) continue;
+        const int st = table_add(keys, vals, log2cap, key, key_hash(key), src_vals[i]);
         if (st == kTableFull) *overflow = 1u;
         n_new += st == kTableNew;
     }
@@ -252,34 +291,34 @@ __global__ void __launch_bounds__(256) table_merge_kernel(unsigned long long *ke
 // L2-resident table).  So the k-mers are written out, partitioned by the high bits of their slot (binning.cuh)
 // and inserted slice after slice, each slice pulled into L2 first.  The k-mers of bin `bin` are
 // binned[offs[bin * n_blocks] .. offs[(bin + 1) * n_blocks]); one launch inserts the bins [bin, bin_end).
-__global__ void __launch_bounds__(256) bin_insert_kernel(const uint64_t *__restrict__ binned, const uint64_t *__restrict__ offs,
-                                                         uint64_t n_blocks, int bin, int bin_end, unsigned long long *keys,
-                                                         uint32_t *vals, uint32_t log2cap, unsigned long long *distinct,
-                                                         uint32_t *overflow)
+template <typename Key>
+__global__ void __launch_bounds__(256) bin_insert_kernel(const Key *__restrict__ binned, const uint64_t *__restrict__ offs,
+                                                         uint64_t n_blocks, int bin, int bin_end, Key *keys, uint32_t *vals,
+                                                         uint32_t log2cap, unsigned long long *distinct, uint32_t *overflow)
 {
     const uint64_t begin = __ldg(offs + static_cast<uint64_t>(bin) * n_blocks);
     const uint64_t end = __ldg(offs + static_cast<uint64_t>(bin_end) * n_blocks);
     uint32_t n_new = 0;
     for (uint64_t i = begin + static_cast<uint64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < end;
          i += static_cast<uint64_t>(gridDim.x) * blockDim.x) {
-        const uint64_t key = __ldg(binned + i);
-        const uint64_t d[1] = {key};
-        const int st = table_add(keys, vals, log2cap, key, fx_hash<1>(d, 0), 1u);
+        const Key key = __ldg(binned + i);
+        const int st = table_add(keys, vals, log2cap, key, key_hash(key), 1u);
         if (st == kTableFull) *overflow = 1u;
         n_new += st == kTableNew;
     }
     add_distinct(distinct, n_new);
 }
 
-__global__ void __launch_bounds__(256) table_export_kernel(const unsigned long long *__restrict__ keys,
-                                                           const uint32_t *__restrict__ vals, uint64_t n_slots,
-                                                           uint64_t *__restrict__ out_keys, uint32_t *__restrict__ out_vals,
-                                                           uint64_t capacity, unsigned long long *cursor)
+template <typename Key>
+__global__ void __launch_bounds__(256) table_export_kernel(const Key *__restrict__ keys, const uint32_t *__restrict__ vals,
+                                                           uint64_t n_slots, Key *__restrict__ out_keys,
+                                                           uint32_t *__restrict__ out_vals, uint64_t capacity,
+                                                           unsigned long long *cursor)
 {
     for (uint64_t i = static_cast<uint64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < n_slots;
          i += static_cast<uint64_t>(gridDim.x) * blockDim.x) {
-        const uint64_t key = keys[i];
-        if (key == kEmptyKey) continue;
+        const Key key = keys[i];
+        if (key_free(key)) continue;
         const uint32_t active = __activemask(); // warp-aggregated append: one atomic per converged group
         const int leader = __ffs(active) - 1;
         unsigned long long base = 0;
@@ -448,23 +487,24 @@ static int32_t table_status(kmc_ctx *ctx, cudaStream_t stream, unsigned long lon
     return KMC_OK;
 }
 
-extern "C" int32_t kmc_kmer_count(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t mode, uint64_t *keys, uint32_t *vals,
-                                  uint32_t log2_capacity, kmc_result *result)
+// The key of a table of NL limbs (table_keys.cuh), and the same k-mer as binning.cuh partitions it
+template <int NL> using TableKey = typename std::conditional<NL == 1, unsigned long long, ulonglong2>::type;
+template <int NL> using BinKey = typename std::conditional<NL == 1, uint64_t, ulonglong2>::type;
+
+// kmc_kmer_count (NL = 1) and kmc_kmer_count2 (NL = 2) past their K checks
+template <int NL>
+static int32_t kmer_count(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t mode, uint64_t *keys, uint32_t *vals,
+                          uint32_t log2_capacity, kmc_result *result)
 {
-    int32_t st = check_common(ctx, seqs, k);
-    if (st) return st;
-    if (!keys || !vals || !result) return fail(ctx, KMC_E_BAD_ARG, "keys / vals / result is NULL");
-    if (mode != KMC_FW && mode != KMC_CANON) return fail(ctx, KMC_E_BAD_ARG, "mode must be KMC_FW or KMC_CANON");
-    if (seqs->src_bits != 2) return fail(ctx, KMC_E_UNSUPPORTED, "the k-mer table needs a 2-bit source");
-    if (k > 32 || (k == 32 && mode == KMC_FW))
-        return fail(ctx, KMC_E_UNSUPPORTED, "the k-mer table supports K <= 31, and K = 32 for canonical k-mers");
+    using Key = TableKey<NL>;
     if (log2_capacity < 1 || log2_capacity > 40) return fail(ctx, KMC_E_BAD_ARG, "log2_capacity must be in 1..40");
     CU(cudaSetDevice(ctx->device));
     memset(result, 0, sizeof *result);
     const Geometry ge = geometry(k);
+    if (ge.n_limbs != NL) return fail(ctx, KMC_E_UNSUPPORTED, "no kernel for this K");
     cudaStream_t stream = ctx->stream;
     CU(cudaEventRecord(ctx->ev_k0, stream));
-    st = ensure_scratch(ctx, layout_scratch_bytes(seqs) + 1024);
+    int32_t st = ensure_scratch(ctx, layout_scratch_bytes(seqs) + 1024);
     if (st) return st;
     st = ensure_host_small(ctx);
     if (st) return st;
@@ -477,26 +517,32 @@ extern "C" int32_t kmc_kmer_count(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k,
     result->n_written = L.total;
     if (L.total == 0) return KMC_OK;
     ExtractParams p = base_params(seqs, k, ge, L, 0);
+    Key *table_keys = reinterpret_cast<Key *>(keys);
     ConsumeParams c{};
     c.table = vals;
-    c.keys = reinterpret_cast<unsigned long long *>(keys);
+    if constexpr (NL == 1)
+        c.keys = table_keys;
+    else
+        c.keys2 = table_keys;
     c.log2cap = log2_capacity;
     c.distinct = distinct;
     c.overflow = overflow;
     CU(cudaMemsetAsync(distinct, 0, 16, stream));
-    // A table beyond L2 (12 bytes per slot): write the k-mers out, bin them by the table slice they fall into and
-    // insert slice after slice (bin_insert_kernel).  Needs 16 bytes per k-mer of temporary memory; without it the
-    // k-mers are inserted as they are produced.
-    const uint64_t table_bytes = 12ull << log2_capacity;
-    int bin_bits = static_cast<int>(log2_capacity) - 20; // <= 2^20 slots = 12 MB per slice
+    // A table beyond L2 (12 bytes per slot for one limb, 20 for two): write the k-mers out, bin them by the table slice
+    // they fall into and insert slice after slice (bin_insert_kernel), a group of slices -- 72 MB of one-limb table, 60 MB
+    // of two-limb table -- per launch.  Needs 16 (32) bytes per k-mer of temporary memory; without it the k-mers are
+    // inserted as they are produced.
+    const uint64_t slot_bytes = 8 * NL + 4;
+    const uint64_t table_bytes = slot_bytes << log2_capacity;
+    int bin_bits = static_cast<int>(log2_capacity) - 20; // <= 2^20 slots = 12 (20) MB per slice
     bin_bits = std::max(binning::kMinBits, std::min(binning::kMaxBits, bin_bits));
     bool binned = table_bytes > (96ull << 20) && static_cast<int>(log2_capacity) > bin_bits;
     AsyncBuf kmers_buf, binned_buf, matrix_buf, offs_buf, scan_buf;
     const uint64_t n_flat = (L.items + 1) * static_cast<uint64_t>(ge.g); // flat windows, rounded up to whole groups
     if (binned) {
-        const uint64_t cells = binning::matrix_cells<uint64_t>(L.total, bin_bits);
-        cudaError_t e = kmers_buf.alloc(ctx, round_up(n_flat * 8, 256), stream);
-        if (e == cudaSuccess) e = binned_buf.alloc(ctx, round_up(n_flat * 8, 256), stream);
+        const uint64_t cells = binning::matrix_cells<BinKey<NL>>(L.total, bin_bits);
+        cudaError_t e = kmers_buf.alloc(ctx, round_up(n_flat * sizeof(Key), 256), stream);
+        if (e == cudaSuccess) e = binned_buf.alloc(ctx, round_up(n_flat * sizeof(Key), 256), stream);
         if (e == cudaSuccess) e = matrix_buf.alloc(ctx, (cells + 1) * 8, stream);
         if (e == cudaSuccess) e = offs_buf.alloc(ctx, (cells + 2) * 8, stream);
         if (e == cudaSuccess) e = scan_buf.alloc(ctx, (scan_tmp_elems(cells) + 1) * 8, stream);
@@ -511,25 +557,31 @@ extern "C" int32_t kmc_kmer_count(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k,
         ExtractLaunchFn xfn = get_launcher(ge, mode == KMC_CANON ? MODE_CANON : MODE_FW, false, !L.uniform_len);
         if (!xfn) return fail(ctx, KMC_E_UNSUPPORTED, "no kernel for this K");
         CU(xfn(p, ctx->sm_count, stream));
-        const uint64_t *kmers = static_cast<const uint64_t *>(kmers_buf.p);
-        uint64_t *sorted = static_cast<uint64_t *>(binned_buf.p);
+        const BinKey<NL> *kmers = static_cast<const BinKey<NL> *>(kmers_buf.p);
+        BinKey<NL> *sorted = static_cast<BinKey<NL> *>(binned_buf.p);
         uint64_t *offs = static_cast<uint64_t *>(offs_buf.p);
-        CU(binning::partition<uint64_t>(kmers, L.total, bin_bits, binning::KmerHashBin{64 - bin_bits}, sorted,
-                                        static_cast<uint64_t *>(matrix_buf.p), offs, static_cast<uint64_t *>(scan_buf.p), stream));
-        const uint64_t n_blocks = binning::blocks_for<uint64_t>(L.total);
+        if constexpr (NL == 1)
+            CU(binning::partition<BinKey<NL>>(kmers, L.total, bin_bits, binning::KmerHashBin{64 - bin_bits}, sorted,
+                                       static_cast<uint64_t *>(matrix_buf.p), offs, static_cast<uint64_t *>(scan_buf.p), stream));
+        else
+            CU(binning::partition<BinKey<NL>>(kmers, L.total, bin_bits, binning::KmerHashBin2{64 - bin_bits}, sorted,
+                                       static_cast<uint64_t *>(matrix_buf.p), offs, static_cast<uint64_t *>(scan_buf.p), stream));
+        const uint64_t n_blocks = binning::blocks_for<BinKey<NL>>(L.total);
         const uint64_t slice = 1ull << (log2_capacity - bin_bits); // slots per bin
-        const int group = apply_group(6);
+        const int group = apply_group(NL == 1 ? 6 : 3);
         for (int b = 0; b < (1 << bin_bits); b += group) {
             const int b_end = std::min(b + group, 1 << bin_bits);
             const uint64_t slots = slice * static_cast<uint64_t>(b_end - b);
-            CU(warm_table(reinterpret_cast<const uint32_t *>(keys + static_cast<uint64_t>(b) * slice), 2 * slots, ctx->sm_count, warm_sink(ctx), stream));
+            CU(warm_table(reinterpret_cast<const uint32_t *>(table_keys + static_cast<uint64_t>(b) * slice), 2 * NL * slots, ctx->sm_count,
+                          warm_sink(ctx), stream));
             CU(warm_table(vals + static_cast<uint64_t>(b) * slice, slots, ctx->sm_count, warm_sink(ctx), stream));
-            bin_insert_kernel<<<static_cast<unsigned>(ctx->sm_count * 16), 256, 0, stream>>>(
-                sorted, offs, n_blocks, b, b_end, c.keys, vals, log2_capacity, distinct, overflow);
+            bin_insert_kernel<Key><<<static_cast<unsigned>(ctx->sm_count * 16), 256, 0, stream>>>(
+                reinterpret_cast<const Key *>(sorted), offs, n_blocks, b, b_end, table_keys, vals, log2_capacity, distinct, overflow);
         }
         CU(cudaGetLastError());
     } else {
-        ConsumeLaunchFn fn = consume_launcher<OP_TABLE>(ge, !L.uniform_len, mode == KMC_CANON);
+        const bool ragged = !L.uniform_len, canon = mode == KMC_CANON;
+        ConsumeLaunchFn fn = NL == 1 ? consume_launcher<OP_TABLE>(ge, ragged, canon) : pick_consume_nx<2, OP_TABLE2>(ge.nx, ragged, canon);
         if (!fn) return fail(ctx, KMC_E_UNSUPPORTED, "no kernel for this K");
         CU(fn(p, c, stream));
     }
@@ -539,9 +591,11 @@ extern "C" int32_t kmc_kmer_count(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k,
     return st;
 }
 
-extern "C" int32_t kmc_kmer_table_merge(kmc_ctx *ctx, uint64_t *keys, uint32_t *vals, uint32_t log2_capacity,
-                                        const uint64_t *src_keys, const uint32_t *src_vals, uint64_t n_src, uint64_t *n_new)
+template <int NL>
+static int32_t kmer_table_merge(kmc_ctx *ctx, uint64_t *keys, uint32_t *vals, uint32_t log2_capacity, const uint64_t *src_keys,
+                                const uint32_t *src_vals, uint64_t n_src, uint64_t *n_new)
 {
+    using Key = TableKey<NL>;
     if (!ctx) return KMC_E_BAD_ARG;
     if (!keys || !vals || (n_src && (!src_keys || !src_vals))) return fail(ctx, KMC_E_BAD_ARG, "NULL table");
     if (log2_capacity < 1 || log2_capacity > 40) return fail(ctx, KMC_E_BAD_ARG, "log2_capacity must be in 1..40");
@@ -556,10 +610,9 @@ extern "C" int32_t kmc_kmer_table_merge(kmc_ctx *ctx, uint64_t *keys, uint32_t *
     CU(cudaMemsetAsync(distinct, 0, 16, stream));
     if (n_src) {
         const uint64_t blocks = std::min<uint64_t>((n_src + 255) / 256, static_cast<uint64_t>(ctx->sm_count) * 16);
-        table_merge_kernel<<<static_cast<unsigned>(blocks), 256, 0, stream>>>(reinterpret_cast<unsigned long long *>(keys), vals,
-                                                                              log2_capacity,
-                                                                              reinterpret_cast<const unsigned long long *>(src_keys),
-                                                                              src_vals, n_src, distinct, overflow);
+        table_merge_kernel<Key><<<static_cast<unsigned>(blocks), 256, 0, stream>>>(reinterpret_cast<Key *>(keys), vals, log2_capacity,
+                                                                                   reinterpret_cast<const Key *>(src_keys), src_vals,
+                                                                                   n_src, distinct, overflow);
         CU(cudaGetLastError());
     }
     kmc_result r{};
@@ -568,9 +621,11 @@ extern "C" int32_t kmc_kmer_table_merge(kmc_ctx *ctx, uint64_t *keys, uint32_t *
     return st;
 }
 
-extern "C" int32_t kmc_kmer_table_export(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
-                                         uint64_t *out_keys, uint32_t *out_vals, uint64_t capacity, uint64_t *n_out)
+template <int NL>
+static int32_t kmer_table_export(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity, uint64_t *out_keys,
+                                 uint32_t *out_vals, uint64_t capacity, uint64_t *n_out)
 {
+    using Key = TableKey<NL>;
     if (!ctx) return KMC_E_BAD_ARG;
     if (!keys || !vals || !n_out || (capacity && (!out_keys || !out_vals))) return fail(ctx, KMC_E_BAD_ARG, "NULL buffer");
     if (log2_capacity < 1 || log2_capacity > 40) return fail(ctx, KMC_E_BAD_ARG, "log2_capacity must be in 1..40");
@@ -584,12 +639,68 @@ extern "C" int32_t kmc_kmer_table_export(kmc_ctx *ctx, const uint64_t *keys, con
     CU(cudaMemsetAsync(cursor, 0, 8, stream));
     const uint64_t n_slots = 1ull << log2_capacity;
     const uint64_t blocks = std::min<uint64_t>((n_slots + 255) / 256, static_cast<uint64_t>(ctx->sm_count) * 16);
-    table_export_kernel<<<static_cast<unsigned>(blocks), 256, 0, stream>>>(reinterpret_cast<const unsigned long long *>(keys), vals,
-                                                                           n_slots, out_keys, out_vals, capacity, cursor);
+    table_export_kernel<Key><<<static_cast<unsigned>(blocks), 256, 0, stream>>>(reinterpret_cast<const Key *>(keys), vals, n_slots,
+                                                                                 reinterpret_cast<Key *>(out_keys), out_vals, capacity,
+                                                                                 cursor);
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(&ctx->host_small[100], cursor, 8, cudaMemcpyDeviceToHost, stream));
     CU(cudaStreamSynchronize(stream));
     *n_out = ctx->host_small[100];
     if (*n_out > capacity) return fail(ctx, KMC_E_OUT_TOO_SMALL, "export capacity smaller than the number of keys in the table");
     return KMC_OK;
+}
+
+extern "C" int32_t kmc_kmer_count(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t mode, uint64_t *keys, uint32_t *vals,
+                                  uint32_t log2_capacity, kmc_result *result)
+{
+    int32_t st = check_common(ctx, seqs, k);
+    if (st) return st;
+    if (!keys || !vals || !result) return fail(ctx, KMC_E_BAD_ARG, "keys / vals / result is NULL");
+    if (mode != KMC_FW && mode != KMC_CANON) return fail(ctx, KMC_E_BAD_ARG, "mode must be KMC_FW or KMC_CANON");
+    if (seqs->src_bits != 2) return fail(ctx, KMC_E_UNSUPPORTED, "the k-mer table needs a 2-bit source");
+    if (k > 32 || (k == 32 && mode == KMC_FW))
+        return fail(ctx, KMC_E_UNSUPPORTED, "the k-mer table supports K <= 31, and K = 32 for canonical k-mers");
+    return kmer_count<1>(ctx, seqs, k, mode, keys, vals, log2_capacity, result);
+}
+
+extern "C" int32_t kmc_kmer_count2(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t mode, uint64_t *keys, uint32_t *vals,
+                                   uint32_t log2_capacity, kmc_result *result)
+{
+    int32_t st = check_common(ctx, seqs, k);
+    if (st) return st;
+    if (!keys || !vals || !result) return fail(ctx, KMC_E_BAD_ARG, "keys / vals / result is NULL");
+    if (reinterpret_cast<uintptr_t>(keys) % 16) return fail(ctx, KMC_E_BAD_ARG, "the two-limb keys must be 16-byte aligned");
+    if (mode != KMC_FW && mode != KMC_CANON) return fail(ctx, KMC_E_BAD_ARG, "mode must be KMC_FW or KMC_CANON");
+    if (seqs->src_bits != 2) return fail(ctx, KMC_E_UNSUPPORTED, "the k-mer table needs a 2-bit source");
+    if (k < 33 || k > 64 || (k == 64 && mode == KMC_FW))
+        return fail(ctx, KMC_E_UNSUPPORTED, "the two-limb k-mer table supports K = 33..63, and K = 64 for canonical k-mers");
+    return kmer_count<2>(ctx, seqs, k, mode, keys, vals, log2_capacity, result);
+}
+
+extern "C" int32_t kmc_kmer_table_merge(kmc_ctx *ctx, uint64_t *keys, uint32_t *vals, uint32_t log2_capacity,
+                                        const uint64_t *src_keys, const uint32_t *src_vals, uint64_t n_src, uint64_t *n_new)
+{
+    return kmer_table_merge<1>(ctx, keys, vals, log2_capacity, src_keys, src_vals, n_src, n_new);
+}
+
+extern "C" int32_t kmc_kmer_table2_merge(kmc_ctx *ctx, uint64_t *keys, uint32_t *vals, uint32_t log2_capacity,
+                                         const uint64_t *src_keys, const uint32_t *src_vals, uint64_t n_src, uint64_t *n_new)
+{
+    if (ctx && (reinterpret_cast<uintptr_t>(keys) % 16 || reinterpret_cast<uintptr_t>(src_keys) % 16))
+        return fail(ctx, KMC_E_BAD_ARG, "the two-limb keys must be 16-byte aligned");
+    return kmer_table_merge<2>(ctx, keys, vals, log2_capacity, src_keys, src_vals, n_src, n_new);
+}
+
+extern "C" int32_t kmc_kmer_table_export(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
+                                         uint64_t *out_keys, uint32_t *out_vals, uint64_t capacity, uint64_t *n_out)
+{
+    return kmer_table_export<1>(ctx, keys, vals, log2_capacity, out_keys, out_vals, capacity, n_out);
+}
+
+extern "C" int32_t kmc_kmer_table2_export(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
+                                          uint64_t *out_keys, uint32_t *out_vals, uint64_t capacity, uint64_t *n_out)
+{
+    if (ctx && (reinterpret_cast<uintptr_t>(keys) % 16 || reinterpret_cast<uintptr_t>(out_keys) % 16))
+        return fail(ctx, KMC_E_BAD_ARG, "the two-limb keys must be 16-byte aligned");
+    return kmer_table_export<2>(ctx, keys, vals, log2_capacity, out_keys, out_vals, capacity, n_out);
 }

@@ -113,6 +113,12 @@ SIGNATURES = {
                                          C.POINTER(C.c_uint64)]),
     "kmc_kmer_table_export": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint64,
                                           C.POINTER(C.c_uint64)]),
+    "kmc_kmer_count2": (C.c_int32, [C.c_void_p, C.POINTER(kmc_seqs), C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_uint32,
+                                    C.POINTER(kmc_result)]),
+    "kmc_kmer_table2_merge": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint64,
+                                          C.POINTER(C.c_uint64)]),
+    "kmc_kmer_table2_export": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint64,
+                                           C.POINTER(C.c_uint64)]),
     "kmc_nccl_version": (C.c_int32, [C.POINTER(C.c_int32)]),
     "kmc_comm_unique_id": (C.c_int32, [C.c_void_p]),
     "kmc_comm_init_rank": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]),
@@ -125,6 +131,9 @@ SIGNATURES = {
     "kmc_kmer_owner": (C.c_uint32, [C.c_uint64, C.c_uint32]),
     "kmc_kmer_table_exchange": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32,
                                             C.POINTER(C.c_uint64)]),
+    "kmc_kmer_owner2": (C.c_uint32, [C.c_uint64, C.c_uint64, C.c_uint32]),
+    "kmc_kmer_table2_exchange": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32,
+                                             C.POINTER(C.c_uint64)]),
     "kmc_group_create": (C.c_int32, [C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_void_p)]),
     "kmc_group_destroy": (C.c_int32, [C.c_void_p]),
     "kmc_group_size": (C.c_int32, [C.c_void_p, C.POINTER(C.c_int32)]),
@@ -140,6 +149,8 @@ SIGNATURES = {
                                            C.POINTER(kmc_result)]),
     "kmc_group_kmer_table_exchange": (C.c_int32, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_uint32,
                                                   C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_uint32, C.POINTER(C.c_uint64)]),
+    "kmc_group_kmer_table2_exchange": (C.c_int32, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_uint32,
+                                                   C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_uint32, C.POINTER(C.c_uint64)]),
     "kmc_digest": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
     "kmc_timer_begin": (C.c_int32, [C.c_void_p]),
     "kmc_timer_end": (C.c_int32, [C.c_void_p, C.POINTER(C.c_float)]),

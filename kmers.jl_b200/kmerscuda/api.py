@@ -762,56 +762,80 @@ def composition(rs, K: int, *, canonical: bool = False, ctx: Optional[Context] =
 
 class KmerTable:
     """Exact k-mer counts on the device (kmc_kmer_count): an open-addressing table keyed by the k-mer,
-    the `Dict{Kmer,Int}` a user of the reference's iterators builds.  K <= 31 (forward) / 32 (canonical)."""
+    the `Dict{Kmer,Int}` a user of the reference's iterators builds.  K <= 31 (forward) / 32 (canonical).
 
-    def __init__(self, log2_capacity: int, ctx: Optional[Context] = None):
+    n_limbs=2 keys the table by two-limb k-mers (kmc_kmer_count2 and the other `*2` entry points): K = 33..63
+    (forward) / 64 (canonical), 20 bytes per slot."""
+
+    def __init__(self, log2_capacity: int, ctx: Optional[Context] = None, n_limbs: int = 1):
+        if n_limbs not in (1, 2):
+            raise ValueError(f"n_limbs must be 1 or 2, not {n_limbs}")
         self.ctx = ctx or default_context()
         self.log2_capacity = int(log2_capacity)
+        self.n_limbs = n_limbs
         n = 1 << self.log2_capacity
-        self.keys, self.vals = self.ctx.alloc(8 * n), self.ctx.alloc(4 * n)
-        self.ctx._check(self.ctx.lib.kmc_memset(self.ctx.handle, self.keys.ptr, 0xFF, 8 * n))
+        self.keys, self.vals = self.ctx.alloc(8 * n_limbs * n), self.ctx.alloc(4 * n)
+        self.ctx._check(self.ctx.lib.kmc_memset(self.ctx.handle, self.keys.ptr, 0xFF, 8 * n_limbs * n))
         self.ctx._check(self.ctx.lib.kmc_memset(self.ctx.handle, self.vals.ptr, 0, 4 * n))
         self.n_keys = 0
+
+    def _fn(self, name: str):
+        """The entry point `name` of this table's key width (kmc_kmer_count -> kmc_kmer_count2, ...)."""
+        if self.n_limbs == 2:
+            name = name.replace("kmc_kmer_table_", "kmc_kmer_table2_").replace("kmc_kmer_count", "kmc_kmer_count2")
+        return getattr(self.ctx.lib, name)
+
+    def _same_width(self, other: "KmerTable"):
+        if other.n_limbs != self.n_limbs:
+            raise ValueError(f"tables of {self.n_limbs} and {other.n_limbs} limbs cannot be combined")
 
     def count(self, rs, K: int, *, canonical: bool = True):
         """Adds every k-mer of the set.  Returns (k-mers counted, kernel_ms)."""
         _check_K(K)
         drs = rs if isinstance(rs, DeviceReadSet) else DeviceReadSet(self.ctx, rs)
         res = kmc_result()
-        self.ctx._check(self.ctx.lib.kmc_kmer_count(self.ctx.handle, C.byref(drs.desc), K, KMC_CANON if canonical else KMC_FW,
-                                                    self.keys.ptr, self.vals.ptr, self.log2_capacity, C.byref(res)))
+        self.ctx._check(self._fn("kmc_kmer_count")(self.ctx.handle, C.byref(drs.desc), K, KMC_CANON if canonical else KMC_FW,
+                                                   self.keys.ptr, self.vals.ptr, self.log2_capacity, C.byref(res)))
         self.n_keys += int(res.digest[0])
         return int(res.n_written), float(res.kernel_ms)
 
     def merge(self, other: "KmerTable"):
         """self[k] += other[k] for every key of `other` (same device): the merge step of a sharded count."""
+        self._same_width(other)
         n_new = C.c_uint64(0)
-        self.ctx._check(self.ctx.lib.kmc_kmer_table_merge(self.ctx.handle, self.keys.ptr, self.vals.ptr, self.log2_capacity,
-                                                          other.keys.ptr, other.vals.ptr, 1 << other.log2_capacity, C.byref(n_new)))
+        self.ctx._check(self._fn("kmc_kmer_table_merge")(self.ctx.handle, self.keys.ptr, self.vals.ptr, self.log2_capacity,
+                                                         other.keys.ptr, other.vals.ptr, 1 << other.log2_capacity, C.byref(n_new)))
         self.n_keys += int(n_new.value)
 
     def exchange(self, owned_log2_capacity: int) -> "KmerTable":
         """One process per GPU: send every (key, count) to the rank that owns the key (kmc_kmer_table_exchange over the
         context's communicator) and return this rank's owned table.  Collective."""
-        owned = KmerTable(owned_log2_capacity, ctx=self.ctx)
+        owned = KmerTable(owned_log2_capacity, ctx=self.ctx, n_limbs=self.n_limbs)
         self.ctx.sync()
         n_owned = C.c_uint64(0)
-        self.ctx._check(self.ctx.lib.kmc_kmer_table_exchange(self.ctx.handle, self.keys.ptr, self.vals.ptr, self.log2_capacity,
-                                                             owned.keys.ptr, owned.vals.ptr, owned_log2_capacity, C.byref(n_owned)))
+        self.ctx._check(self._fn("kmc_kmer_table_exchange")(self.ctx.handle, self.keys.ptr, self.vals.ptr, self.log2_capacity,
+                                                            owned.keys.ptr, owned.vals.ptr, owned_log2_capacity, C.byref(n_owned)))
         owned.n_keys = int(n_owned.value)
         return owned
 
     def items(self):
-        """(keys u64[n], counts u32[n]) sorted by key."""
+        """(keys, counts u32[n]) sorted by key: keys u64[n] for one limb; u64[n, 2] (limb 0 = head first) in Kmer order,
+        lexicographic on (limb 0, limb 1), for two."""
         n = max(self.n_keys, 1)
-        dk, dv = self.ctx.alloc(8 * n), self.ctx.alloc(4 * n)
+        L = self.n_limbs
+        dk, dv = self.ctx.alloc(8 * L * n), self.ctx.alloc(4 * n)
         n_out = C.c_uint64(0)
-        self.ctx._check(self.ctx.lib.kmc_kmer_table_export(self.ctx.handle, self.keys.ptr, self.vals.ptr, self.log2_capacity,
-                                                           dk.ptr, dv.ptr, n, C.byref(n_out)))
-        k, v = dk.download(np.uint64, int(n_out.value)), dv.download(np.uint32, int(n_out.value))
+        self.ctx._check(self._fn("kmc_kmer_table_export")(self.ctx.handle, self.keys.ptr, self.vals.ptr, self.log2_capacity,
+                                                          dk.ptr, dv.ptr, n, C.byref(n_out)))
+        m = int(n_out.value)
+        k, v = dk.download(np.uint64, L * m), dv.download(np.uint32, m)
         dk.free()
         dv.free()
-        order = np.argsort(k, kind="stable")
+        if L == 1:
+            order = np.argsort(k, kind="stable")
+            return k[order], v[order]
+        k = k.reshape(m, 2)
+        order = np.lexsort((k[:, 1], k[:, 0]))
         return k[order], v[order]
 
     def free(self):
@@ -907,12 +931,16 @@ class Group:
         """Every (key, count) of the per-device tables to its owner device (kmc_group_kmer_table_exchange);
         returns the owned tables, whose union is the count of the whole input."""
         n = len(self.ctx)
-        owned = [KmerTable(owned_log2_capacity, ctx=c) for c in self.ctx]
+        n_limbs = tables[0].n_limbs
+        for t in tables[1:]:
+            tables[0]._same_width(t)
+        owned = [KmerTable(owned_log2_capacity, ctx=c, n_limbs=n_limbs) for c in self.ctx]
         for c in self.ctx:
             c.sync()
         P = C.c_void_p * n
         n_owned = (C.c_uint64 * n)()
-        self._check(self.lib.kmc_group_kmer_table_exchange(
+        fn = self.lib.kmc_group_kmer_table2_exchange if n_limbs == 2 else self.lib.kmc_group_kmer_table_exchange
+        self._check(fn(
             self.handle, P(*[t.keys.ptr for t in tables]), P(*[t.vals.ptr for t in tables]), tables[0].log2_capacity,
             P(*[t.keys.ptr for t in owned]), P(*[t.vals.ptr for t in owned]), owned_log2_capacity, n_owned))
         for t, m in zip(owned, n_owned):
