@@ -584,148 +584,6 @@ int32_t kmc_base_hash(kmc_ctx *ctx, const uint64_t *kmers, uint64_t n, int32_t n
     return KMC_OK;
 }
 
-namespace {
-int32_t bucket_count_impl(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t bucket_bits, uint32_t *table, uint32_t n_parts,
-                          void *const *events, kmc_result *result);
-}
-
-int32_t kmc_bucket_count(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t bucket_bits, uint32_t *table,
-                         kmc_result *result)
-{
-    return bucket_count_impl(ctx, seqs, k, bucket_bits, table, 0, nullptr, result);
-}
-
-int32_t kmc_bucket_count_async(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t bucket_bits, uint32_t *table,
-                               uint32_t n_parts, void *const *events, kmc_result *result)
-{
-    if (!ctx) return KMC_E_BAD_ARG;
-    if (!events || n_parts < 1 || n_parts > 32 || (n_parts & (n_parts - 1)))
-        return fail(ctx, KMC_E_BAD_ARG, "n_parts must be a power of two <= 32 and events non-NULL");
-    for (uint32_t i = 0; i < n_parts; ++i)
-        if (!events[i]) return fail(ctx, KMC_E_BAD_ARG, "NULL event");
-    return bucket_count_impl(ctx, seqs, k, bucket_bits, table, n_parts, events, result);
-}
-
-namespace {
-// n_parts == 0: the synchronous call (kernel_ms measured); otherwise progress events and no synchronisation
-int32_t bucket_count_impl(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t bucket_bits, uint32_t *table, uint32_t n_parts,
-                          void *const *events, kmc_result *result)
-{
-    int32_t st = check_common(ctx, seqs, k);
-    if (st) return st;
-    if (!table || !result) return fail(ctx, KMC_E_BAD_ARG, "table / result is NULL");
-    if (bucket_bits < 1 || bucket_bits > 32) return fail(ctx, KMC_E_BAD_ARG, "bucket_bits must be in 1..32");
-    if (seqs->src_bits != 2) return fail(ctx, KMC_E_UNSUPPORTED, "bucket count needs a 2-bit source");
-    CU(cudaSetDevice(ctx->device));
-    result->n_written = 0;
-    result->err_seq = result->err_pos = 0;
-    result->err_sym = 0;
-    result->kernel_ms = 0.f;
-    const Geometry ge = geometry(k);
-    cudaStream_t stream = ctx->stream;
-    CU(cudaEventRecord(ctx->ev_k0, stream));
-    st = ensure_scratch(ctx, layout_scratch_bytes(seqs) + 256);
-    if (st) return st;
-    Scratch scratch{static_cast<char *>(ctx->scratch), ctx->scratch_bytes, 0};
-    Layout L;
-    st = plan_layout(ctx, seqs, k, ge, stream, KnownTotals(), scratch, &L);
-    if (st) return st;
-    result->n_written = L.total;
-    auto record_all = [&]() -> int32_t {
-        for (uint32_t i = 0; i < n_parts; ++i) CU(cudaEventRecord(static_cast<cudaEvent_t>(events[i]), stream));
-        return KMC_OK;
-    };
-    if (L.total == 0) return record_all();
-    ExtractParams p = base_params(seqs, k, ge, L, 0);
-    p.bucket_shift = static_cast<uint32_t>(64 - bucket_bits);
-    // Tables beyond L2 (B = 28 is 1 GiB): write the bucket ids out, bin them by their high bits, apply
-    // bin after bin (buckets.cu).  Needs 8 bytes per k-mer of temporary memory; without it (or for
-    // L2-sized tables) the kernel increments the table directly.
-    const uint64_t table_bytes = 4ull << bucket_bits;
-    const bool want_binned = table_bytes > (96ull << 20) && bucket_bits <= 32;
-
-    // the table is incremented directly by the extraction kernel
-    auto count_direct = [&](ExtractParams q, cudaStream_t s) -> int32_t {
-        int32_t rc = ensure_host_small(ctx); // allocates dev_small, where warm_table's sink lives
-        if (rc) return rc;
-        // a table that fits L2 is pulled into it first: increments that miss L2 serialise at DRAM latency
-        if (table_bytes <= (96ull << 20)) CU(warm_table(table, 1ull << bucket_bits, ctx->sm_count, warm_sink(ctx), s));
-        q.bucket_table = table;
-        ExtractLaunchFn fn = get_launcher(ge, MODE_BUCKETS, true, !L.uniform_len);
-        if (!fn) return fail(ctx, KMC_E_UNSUPPORTED, "no kernel for this K");
-        CU(fn(q, ctx->sm_count, s));
-        return KMC_OK;
-    };
-    // the exact binned path for the set (or piece of a uniform set) q describes: ids, histogram, scatter, apply
-    auto count_exact = [&](ExtractParams q, uint64_t windows, cudaStream_t s, uint32_t np, void *const *ev) -> int32_t {
-        AsyncBuf ids_buf, tmp_buf, matrix_buf, offs_buf, scan_buf; // freed (stream-ordered) on every way out
-        const uint64_t n_ids = (q.items + 1) * static_cast<uint64_t>(ge.g); // flat windows, rounded up to whole groups
-        const uint64_t cells = (static_cast<uint64_t>(1) << binned_count_bin_bits(bucket_bits)) * binned_count_blocks(n_ids);
-        cudaError_t e = ids_buf.alloc(ctx, round_up(n_ids * 4, 256), s);
-        if (e == cudaSuccess) e = tmp_buf.alloc(ctx, round_up(n_ids * 4, 256), s);
-        if (e == cudaSuccess) e = matrix_buf.alloc(ctx, (cells + 1) * 8, s);
-        if (e == cudaSuccess) e = offs_buf.alloc(ctx, (cells + 2) * 8, s);
-        if (e == cudaSuccess) e = scan_buf.alloc(ctx, (scan_tmp_elems(cells) + 1) * 8, s);
-        if (e != cudaSuccess) { // not enough memory for the binned path: direct increments
-            (void)cudaGetLastError();
-            int32_t rc = count_direct(q, s);
-            if (rc) return rc;
-            for (uint32_t i = 0; i < np; ++i) CU(cudaEventRecord(static_cast<cudaEvent_t>(ev[i]), s));
-            return KMC_OK;
-        }
-        // the flat id array is exactly the flat window array: every flat index < windows is written
-        // once (slots of partial groups that are not windows are not written and not binned)
-        q.out_a = ids_buf.as<uint64_t>();
-        q.vec_ok = 1;
-        ExtractLaunchFn fn = get_launcher(ge, MODE_BUCKET_IDS, true, !L.uniform_len);
-        if (!fn) return fail(ctx, KMC_E_UNSUPPORTED, "no kernel for this K");
-        CU(fn(q, ctx->sm_count, s));
-        CU(binned_count(ids_buf.as<uint32_t>(), windows, bucket_bits, table, tmp_buf.as<uint32_t>(), matrix_buf.as<uint64_t>(),
-                        offs_buf.as<uint64_t>(), scan_buf.as<uint64_t>(), ctx->sm_count, s, np, ev));
-        return KMC_OK;
-    };
-
-    bool done = false;
-    ExtractParams pa = p;
-    if (want_binned) set_iteration_strides(pa, ge.g);
-    if (want_binned && ge.n_limbs == 1 && L.uniform_len && binned_count_bin_bits(bucket_bits) == 6 && fused_bin_enabled() && pa.aligned &&
-        pa.al_tail == 0 && pa.items < 0xffffffffull - kTileItems) {
-        // One-limb k-mers over an aligned uniform set (C5): ids and bins from one kernel, bins of a fixed capacity and a
-        // spill list for the runs of a bin that filled up (buckets.cu).  Asynchronous like the exact path.
-        AsyncBuf bins_buf, state_buf;
-        const uint64_t cap = fused_bin_capacity(L.total);
-        cudaError_t e = bins_buf.alloc(ctx, fused_bin_buffer_ids(L.total) * 4, stream);
-        if (e == cudaSuccess) e = state_buf.alloc(ctx, fused_bin_state_bytes(), stream);
-        if (e != cudaSuccess) {
-            (void)cudaGetLastError(); // not enough memory: the exact path (which may end at direct increments)
-        } else {
-            st = ensure_host_small(ctx); // allocates dev_small, where the warm-up kernel's sink lives
-            if (st) return st;
-            CU(fused_bin_ids(pa, ge.nx, bucket_bits, bins_buf.as<uint32_t>(), cap, state_buf.as<unsigned long long>(), stream));
-            CU(fused_bin_apply(bins_buf.as<uint32_t>(), cap, state_buf.as<unsigned long long>(), bucket_bits, table, warm_sink(ctx),
-                               ctx->sm_count, stream, n_parts, events));
-            done = true;
-        }
-    }
-    if (!done && want_binned) {
-        st = count_exact(p, L.total, stream, n_parts, events);
-        if (st) return st;
-        done = true;
-    }
-    if (!done) {
-        st = count_direct(p, stream);
-        if (st) return st;
-        st = record_all();
-        if (st) return st;
-    }
-    if (n_parts) return KMC_OK; // asynchronous form: the caller waits for its events
-    CU(cudaEventRecord(ctx->ev_k1, stream));
-    CU(cudaStreamSynchronize(stream));
-    CU(cudaEventElapsedTime(&result->kernel_ms, ctx->ev_k0, ctx->ev_k1));
-    return KMC_OK;
-}
-} // namespace
-
 int32_t kmc_digest(kmc_ctx *ctx, const uint64_t *dptr, uint64_t n, uint64_t *out)
 {
     if (!ctx) return KMC_E_BAD_ARG;

@@ -535,5 +535,78 @@ cudaError_t partition(const Key *in, uint64_t n, int p, BinOf bin_of, Key *out, 
     }
 }
 
+// The binned path of a table too large for L2: one key per update is written out, the keys are partitioned by table slice,
+// and the slices are walked in groups, each group pulled into L2 and then given its keys.
+//
+// A table of up to kL2Budget bytes is updated directly: it stays in L2 (126 MB) beside the stream that updates it.
+constexpr uint64_t kL2Budget = 96ull << 20;
+
+// Table slice per bin: 2^22 counters = 16 MB of bucket table; 2^20 slots = 12 MB of one-limb, 20 MB of two-limb k-mer table.
+constexpr int kBucketSliceBits = 22, kKmerSliceBits = 20;
+
+// log2 of the bins of a table of 2^table_bits entries in slices of at most 2^slice_bits entries
+inline int bin_bits(int table_bits, int slice_bits)
+{
+    const int p = table_bits - slice_bits;
+    return p < kMinBits ? kMinBits : (p > kMaxBits ? kMaxBits : p);
+}
+
+// Bins applied per launch.  Measured on a B200: the bucket table (16 MB slices, increments) is fastest with 2 bins = 32 MB
+// per launch (1: +1 %, 4: +6 %, 8 = 128 MB: 2x slower -- the slices no longer fit L2); the one-limb k-mer table (12 MB
+// slices, a load and an increment per k-mer) keeps improving up to 8 bins = 96 MB (1: 10.7 ms, 2: 9.8, 4: 9.6, 8: 9.3 ms
+// per 480 M k-mers); 6 leaves room for the k-mer stream itself.  The two-limb table takes 3 bins = 60 MB.
+constexpr int kBucketGroup = 2;
+constexpr int kmer_group(int n_limbs) { return n_limbs == 1 ? 6 : 3; }
+
+// The temporaries of the binned path for up to n keys in 2^p bins: the keys as they are written (one per flat window),
+// the binned keys, the count matrix, its offsets and the scan scratch.  Stream-ordered, freed when this goes out of scope.
+template <typename Key> struct BinnedKeys {
+    AsyncBuf written, binned, matrix, offs, scan;
+    int p = 0;
+    uint64_t n_blocks = 0; // of the last partition: the keys of bin b are binned[offs[b * n_blocks] .. offs[(b + 1) * n_blocks])
+
+    // false when the memory is not there (the CUDA error is cleared): the caller then updates the table directly
+    bool alloc(kmc_ctx *ctx, uint64_t n, int bits, cudaStream_t stream)
+    {
+        p = bits;
+        const uint64_t key_bytes = (n * sizeof(Key) + 255) / 256 * 256, cells = matrix_cells<Key>(n, p);
+        cudaError_t e = written.alloc(ctx, key_bytes, stream);
+        if (e == cudaSuccess) e = binned.alloc(ctx, key_bytes, stream);
+        if (e == cudaSuccess) e = matrix.alloc(ctx, (cells + 1) * 8, stream);
+        if (e == cudaSuccess) e = offs.alloc(ctx, (cells + 2) * 8, stream);
+        if (e == cudaSuccess) e = scan.alloc(ctx, (scan_tmp_elems(cells) + 1) * 8, stream);
+        if (e != cudaSuccess) (void)cudaGetLastError();
+        return e == cudaSuccess;
+    }
+
+    // bins the first n written keys by bin_of
+    template <typename BinOf> cudaError_t partition(uint64_t n, BinOf bin_of, cudaStream_t stream)
+    {
+        n_blocks = blocks_for<Key>(n);
+        return binning::partition<Key>(written.as<Key>(), n, p, bin_of, binned.as<Key>(), matrix.as<uint64_t>(), offs.as<uint64_t>(),
+                                       scan.as<uint64_t>(), stream);
+    }
+};
+
+// Walks the bins [0, n_bins) in groups of `group`: apply(bin, bin_end) enqueues the warm-ups of the group's table slices and
+// the kernel that applies its keys.  events (may be NULL): events[i] is recorded once the i-th of n_parts equal ranges of
+// the table is final, i.e. once the bins [i * n_bins / n_parts, (i + 1) * n_bins / n_parts) are applied.
+template <typename Apply>
+cudaError_t apply_groups(int n_bins, int group, uint32_t n_parts, void *const *events, cudaStream_t stream, Apply apply)
+{
+    if (!events) n_parts = 0;
+    uint32_t parts_done = 0;
+    for (int b = 0; b < n_bins; b += group) {
+        const int b_end = b + group < n_bins ? b + group : n_bins;
+        cudaError_t e = apply(b, b_end);
+        if (e != cudaSuccess) return e;
+        while (parts_done < n_parts && static_cast<uint64_t>(parts_done + 1) * n_bins <= static_cast<uint64_t>(b_end) * n_parts) {
+            e = cudaEventRecord(static_cast<cudaEvent_t>(events[parts_done++]), stream);
+            if (e != cudaSuccess) return e;
+        }
+    }
+    return cudaGetLastError();
+}
+
 } // namespace binning
 } // namespace kmc

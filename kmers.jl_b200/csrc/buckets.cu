@@ -10,7 +10,8 @@
 //     then applied bin after bin, so that all SMs work on an L2-resident part of the table at a time.  The
 //     table is final range by range, which kmc_bucket_count_async reports through events so that the merge of
 //     several GPUs' tables can overlap the count.
-#include <cstdlib>
+// This file holds the whole count, from kmc_bucket_count / kmc_bucket_count_async to the last event; enqueue_count
+// chooses the path.
 #include <type_traits>
 
 #include "binning.cuh"
@@ -209,45 +210,6 @@ __global__ void __launch_bounds__(256) spill_apply_kernel(const uint32_t *__rest
         atomicAdd(table + spill[i], 1u);
 }
 
-} // namespace
-
-// ids[0..n) are bucket ids of `bucket_bits` bits; adds their histogram to table.  tmp: n u32 (binned ids),
-// matrix / offs: (n_bins * n_blocks + 1) u64 each, scan_tmp: scan_tmp_elems(n_bins * n_blocks) u64.
-cudaError_t binned_count(const uint32_t *ids, uint64_t n, int bucket_bits, uint32_t *table, uint32_t *binned, uint64_t *matrix,
-                         uint64_t *offs, uint64_t *scan_tmp, int sm_count, cudaStream_t stream, uint32_t n_parts, void *const *events)
-{
-    if (!events) n_parts = 0;
-    if (n == 0) {
-        for (uint32_t i = 0; i < n_parts; ++i) {
-            cudaError_t e = cudaEventRecord(static_cast<cudaEvent_t>(events[i]), stream);
-            if (e != cudaSuccess) return e;
-        }
-        return cudaSuccess;
-    }
-    const int p = binned_count_bin_bits(bucket_bits);
-    if (bucket_bits < p) return cudaErrorInvalidValue; // the caller bins only tables far larger than 2^p counters
-    const int n_bins = 1 << p, shift = bucket_bits - p;
-    const uint64_t n_blocks = binned_count_blocks(n);
-    cudaError_t e = binning::partition<uint32_t>(ids, n, p, binning::IdBin{shift}, binned, matrix, offs, scan_tmp, stream);
-    if (e != cudaSuccess) return e;
-    // offs has n_bins * n_blocks + 1 entries: offs[(bin + 1) * n_blocks] of the last bin is the total
-    const uint64_t slice = 1ull << shift; // counters per bin
-    const int group = apply_group(2); // bins applied per launch
-    uint32_t parts_done = 0;
-    for (int b = 0; b < n_bins; b += group) {
-        const int b_end = b + group < n_bins ? b + group : n_bins;
-        warm_slice_kernel<<<static_cast<unsigned>(sm_count * 8), 256, 0, stream>>>(table + static_cast<uint64_t>(b) * slice,
-                                                                                  slice * (b_end - b), reinterpret_cast<uint32_t *>(scan_tmp));
-        bin_apply_kernel<<<static_cast<unsigned>(sm_count * 16), 256, 0, stream>>>(binned, offs, n_blocks, b, b_end, table);
-        // range i of the table = bins [i * n_bins / n_parts, (i + 1) * n_bins / n_parts): final once they are applied
-        while (parts_done < n_parts && static_cast<uint64_t>(parts_done + 1) * n_bins <= static_cast<uint64_t>(b_end) * n_parts) {
-            e = cudaEventRecord(static_cast<cudaEvent_t>(events[parts_done++]), stream);
-            if (e != cudaSuccess) return e;
-        }
-    }
-    return cudaGetLastError();
-}
-
 uint64_t fused_bin_capacity(uint64_t n_ids)
 {
     const uint64_t cap = n_ids / binning::kTpBins + n_ids / (8 * binning::kTpBins) + 8192;
@@ -255,19 +217,14 @@ uint64_t fused_bin_capacity(uint64_t n_ids)
 }
 // ids the binned buffer holds: the 64 bins and a spill list long enough for every id of the call
 uint64_t fused_bin_buffer_ids(uint64_t n_ids) { return binning::kTpBins * fused_bin_capacity(n_ids) + n_ids + 4096; }
-uint64_t fused_bin_state_bytes() { return kStateWords * sizeof(unsigned long long); }
 
-// First half: one kernel bins the bucket ids of every window.  p: the parameter block of an aligned uniform set of
-// one-limb k-mers with whole groups (the caller has checked that), bucket_shift set.
-cudaError_t fused_bin_ids(ExtractParams p, int nx, int bucket_bits, uint32_t *binned, uint64_t cap, unsigned long long *state,
+// First half: one kernel bins the bucket ids of every window into the 64 bins.  p: the parameter block of an aligned uniform
+// set of one-limb k-mers with whole groups and fewer than 2^32 - kTileItems work items, strides and bucket_shift set (the
+// caller has checked that).  bin = id >> shift.
+cudaError_t fused_bin_ids(ExtractParams p, int nx, int shift, uint32_t *binned, uint64_t cap, unsigned long long *state,
                           cudaStream_t stream)
 {
-    const int pbits = binned_count_bin_bits(bucket_bits);
-    if (pbits != 6 || bucket_bits < pbits) return cudaErrorInvalidValue;
     const uint64_t tiles = (p.items + kTileItems - 1) / kTileItems;
-    if (tiles == 0 || tiles > 0x7fffffffull || p.items >= 0xffffffffull - kTileItems) return cudaErrorInvalidConfiguration;
-    set_iteration_strides(p, 8);
-    if (!p.aligned || p.al_tail) return cudaErrorInvalidValue; // whole groups only
     p.al_magic = aligned_magic(p.gprm);
     p.pf_tiles = 0;
     if (prefetch_enabled()) {
@@ -277,7 +234,7 @@ cudaError_t fused_bin_ids(ExtractParams p, int nx, int bucket_bits, uint32_t *bi
     cudaError_t e = cudaMemsetAsync(state, 0, kStateWords * sizeof(unsigned long long), stream);
     if (e == cudaSuccess) e = cudaMemsetAsync(state + kStateBinEnd, 0xff, binning::kTpBins * sizeof(unsigned long long), stream);
     if (e != cudaSuccess) return e;
-    const FusedBins f{binned, cap, state, bucket_bits - pbits};
+    const FusedBins f{binned, cap, state, shift};
     constexpr int smem = static_cast<int>(sizeof(binning::Scatter64Smem<uint32_t>));
     auto launch = [&](auto tag) -> cudaError_t {
         constexpr int NX = decltype(tag)::value;
@@ -294,53 +251,124 @@ cudaError_t fused_bin_ids(ExtractParams p, int nx, int bucket_bits, uint32_t *bi
     return cudaErrorInvalidValue;
 }
 
-// Second half: the spill list, then the bins in table order, as in binned_count.
-cudaError_t fused_bin_apply(const uint32_t *binned, uint64_t cap, const unsigned long long *state, int bucket_bits, uint32_t *table,
+// Second half: the spill list, then the bins in table order.
+cudaError_t fused_bin_apply(const uint32_t *binned, uint64_t cap, const unsigned long long *state, int shift, uint32_t *table,
                             uint32_t *sink, int sm_count, cudaStream_t stream, uint32_t n_parts, void *const *events)
 {
-    if (!events) n_parts = 0;
-    const int pbits = binned_count_bin_bits(bucket_bits);
-    const int n_bins = 1 << pbits, shift = bucket_bits - pbits;
     const uint64_t slice = 1ull << shift;
-    const int group = apply_group(2);
-    spill_apply_kernel<<<static_cast<unsigned>(sm_count * 8), 256, 0, stream>>>(binned + static_cast<uint64_t>(n_bins) * cap, state, table);
-    uint32_t parts_done = 0;
-    for (int b = 0; b < n_bins; b += group) {
-        const int b_end = b + group < n_bins ? b + group : n_bins;
-        warm_slice_kernel<<<static_cast<unsigned>(sm_count * 8), 256, 0, stream>>>(table + static_cast<uint64_t>(b) * slice,
-                                                                                  slice * (b_end - b), sink);
+    spill_apply_kernel<<<static_cast<unsigned>(sm_count * 8), 256, 0, stream>>>(binned + binning::kTpBins * cap, state, table);
+    auto apply = [&](int b, int b_end) {
+        const cudaError_t e = warm_table(table + static_cast<uint64_t>(b) * slice, slice * (b_end - b), sm_count, sink, stream);
+        if (e != cudaSuccess) return e;
         bin_apply_fused_kernel<<<static_cast<unsigned>(sm_count * 16), 256, 0, stream>>>(binned, cap, state, b, b_end, table);
-        while (parts_done < n_parts && static_cast<uint64_t>(parts_done + 1) * n_bins <= static_cast<uint64_t>(b_end) * n_parts) {
-            cudaError_t e = cudaEventRecord(static_cast<cudaEvent_t>(events[parts_done++]), stream);
-            if (e != cudaSuccess) return e;
+        return cudaGetLastError();
+    };
+    return binning::apply_groups(binning::kTpBins, binning::kBucketGroup, n_parts, events, stream, apply);
+}
+
+// Enqueues the count on the first path that applies:
+//   * no windows: nothing to count;
+//   * the table fits L2: the extraction kernel increments it directly (SINK_BUCKETS);
+//   * one-limb k-mers over an aligned uniform set in 64 bins (C5), and the fused bins fit in memory: ids and bins from one
+//     kernel, bins of a fixed capacity and a spill list for the runs of a bin that filled up;
+//   * the temporaries of the exact path fit in memory: ids written out (SINK_IDS), partitioned, applied bin after bin;
+//   * otherwise direct increments.
+// Every path records the n_parts progress events (events may be NULL) once their ranges of the table are final.
+int32_t enqueue_count(kmc_ctx *ctx, const Geometry &ge, const Layout &L, ExtractParams p, int bucket_bits, uint32_t *table,
+                      uint32_t n_parts, void *const *events, cudaStream_t stream)
+{
+    auto record_all = [&]() -> int32_t {
+        for (uint32_t i = 0; i < n_parts; ++i) CU(cudaEventRecord(static_cast<cudaEvent_t>(events[i]), stream));
+        return KMC_OK;
+    };
+    if (L.total == 0) return record_all();
+    int32_t st = ensure_host_small(ctx); // allocates dev_small, where the warm-up kernel's sink lives
+    if (st) return st;
+    const bool fits_l2 = (4ull << bucket_bits) <= binning::kL2Budget;
+    if (!fits_l2) {
+        const int pbits = binning::bin_bits(bucket_bits, binning::kBucketSliceBits), shift = bucket_bits - pbits;
+        ExtractParams pa = p;
+        set_iteration_strides(pa, ge.g);
+        if (ge.n_limbs == 1 && L.uniform_len && pbits == 6 && pa.aligned && pa.al_tail == 0 && pa.items < 0xffffffffull - kTileItems) {
+            AsyncBuf bins_buf, state_buf;
+            const uint64_t cap = fused_bin_capacity(L.total);
+            cudaError_t e = bins_buf.alloc(ctx, fused_bin_buffer_ids(L.total) * 4, stream);
+            if (e == cudaSuccess) e = state_buf.alloc(ctx, kStateWords * sizeof(unsigned long long), stream);
+            if (e == cudaSuccess) {
+                CU(fused_bin_ids(pa, ge.nx, shift, bins_buf.as<uint32_t>(), cap, state_buf.as<unsigned long long>(), stream));
+                CU(fused_bin_apply(bins_buf.as<uint32_t>(), cap, state_buf.as<unsigned long long>(), shift, table, warm_sink(ctx),
+                                   ctx->sm_count, stream, n_parts, events));
+                return KMC_OK;
+            }
+            (void)cudaGetLastError();
+        }
+        // the flat id array is exactly the flat window array: every flat index < windows is written once (slots of partial
+        // groups that are not windows are not written and not binned)
+        binning::BinnedKeys<uint32_t> bk;
+        if (bk.alloc(ctx, (L.items + 1) * static_cast<uint64_t>(ge.g), pbits, stream)) {
+            p.out_a = bk.written.as<uint64_t>();
+            p.vec_ok = 1;
+            ExtractLaunchFn fn = get_launcher(ge, MODE_BUCKET_IDS, true, !L.uniform_len);
+            if (!fn) return fail(ctx, KMC_E_UNSUPPORTED, "no kernel for this K");
+            CU(fn(p, ctx->sm_count, stream));
+            CU(bk.partition(L.total, binning::IdBin{shift}, stream));
+            const uint64_t slice = 1ull << shift;
+            auto apply = [&](int b, int b_end) {
+                const cudaError_t e = warm_table(table + static_cast<uint64_t>(b) * slice, slice * (b_end - b), ctx->sm_count,
+                                                 warm_sink(ctx), stream);
+                if (e != cudaSuccess) return e;
+                bin_apply_kernel<<<static_cast<unsigned>(ctx->sm_count * 16), 256, 0, stream>>>(bk.binned.as<uint32_t>(), bk.offs.as<uint64_t>(),
+                                                                                                bk.n_blocks, b, b_end, table);
+                return cudaGetLastError();
+            };
+            CU(binning::apply_groups(1 << pbits, binning::kBucketGroup, n_parts, events, stream, apply));
+            return KMC_OK;
         }
     }
-    return cudaGetLastError();
+    // a table that fits L2 is pulled into it first: increments that miss L2 serialise at DRAM latency
+    if (fits_l2) CU(warm_table(table, 1ull << bucket_bits, ctx->sm_count, warm_sink(ctx), stream));
+    p.bucket_table = table;
+    ExtractLaunchFn fn = get_launcher(ge, MODE_BUCKETS, true, !L.uniform_len);
+    if (!fn) return fail(ctx, KMC_E_UNSUPPORTED, "no kernel for this K");
+    CU(fn(p, ctx->sm_count, stream));
+    return record_all();
 }
 
-// KMC_FUSED_BIN=0 keeps every binned count on the exact three-pass path (A/B measurements, tests of both)
-bool fused_bin_enabled()
+// n_parts == 0: the synchronous call (kernel_ms measured); otherwise progress events and no synchronisation
+int32_t bucket_count(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t bucket_bits, uint32_t *table, uint32_t n_parts,
+                     void *const *events, kmc_result *result)
 {
-    static const bool on = [] {
-        const char *e = getenv("KMC_FUSED_BIN");
-        return !(e && e[0] == '0');
-    }();
-    return on;
+    int32_t st = check_common(ctx, seqs, k);
+    if (st) return st;
+    if (!table || !result) return fail(ctx, KMC_E_BAD_ARG, "table / result is NULL");
+    if (bucket_bits < 1 || bucket_bits > 32) return fail(ctx, KMC_E_BAD_ARG, "bucket_bits must be in 1..32");
+    if (seqs->src_bits != 2) return fail(ctx, KMC_E_UNSUPPORTED, "bucket count needs a 2-bit source");
+    CU(cudaSetDevice(ctx->device));
+    result->n_written = 0;
+    result->err_seq = result->err_pos = 0;
+    result->err_sym = 0;
+    result->kernel_ms = 0.f;
+    const Geometry ge = geometry(k);
+    cudaStream_t stream = ctx->stream;
+    CU(cudaEventRecord(ctx->ev_k0, stream));
+    st = ensure_scratch(ctx, layout_scratch_bytes(seqs) + 256);
+    if (st) return st;
+    Scratch scratch{static_cast<char *>(ctx->scratch), ctx->scratch_bytes, 0};
+    Layout L;
+    st = plan_layout(ctx, seqs, k, ge, stream, KnownTotals(), scratch, &L);
+    if (st) return st;
+    result->n_written = L.total;
+    ExtractParams p = base_params(seqs, k, ge, L, 0);
+    p.bucket_shift = static_cast<uint32_t>(64 - bucket_bits);
+    st = enqueue_count(ctx, ge, L, p, bucket_bits, table, n_parts, events, stream);
+    if (st || n_parts || L.total == 0) return st; // the asynchronous form: the caller waits for its events
+    CU(cudaEventRecord(ctx->ev_k1, stream));
+    CU(cudaStreamSynchronize(stream));
+    CU(cudaEventElapsedTime(&result->kernel_ms, ctx->ev_k0, ctx->ev_k1));
+    return KMC_OK;
 }
 
-// Bins applied per launch.  Measured on a B200 (KMC_APPLY_GROUP overrides, for experiments): the bucket table
-// (16 MB slices, increments) is fastest with 2 bins = 32 MB per launch (1: +1 %, 4: +6 %, 8 = 128 MB: 2x slower --
-// the slices no longer fit L2); the k-mer table (12 MB slices, a load and an increment per k-mer) keeps improving up to
-// 8 bins = 96 MB (1: 10.7 ms, 2: 9.8, 4: 9.6, 8: 9.3 ms per 480 M k-mers); 6 leaves room for the k-mer stream itself.
-int apply_group(int dflt)
-{
-    static const int env = [] {
-        const char *e = getenv("KMC_APPLY_GROUP");
-        const int v = e ? atoi(e) : 0;
-        return v < 0 ? 0 : (v > 64 ? 64 : v);
-    }();
-    return env ? env : dflt;
-}
+} // namespace
 
 cudaError_t warm_table(const uint32_t *table, uint64_t n_counters, int sm_count, uint32_t *sink, cudaStream_t stream)
 {
@@ -348,14 +376,23 @@ cudaError_t warm_table(const uint32_t *table, uint64_t n_counters, int sm_count,
     return cudaGetLastError();
 }
 
-int binned_count_bin_bits(int bucket_bits)
+} // namespace kmc
+
+using namespace kmc;
+
+extern "C" int32_t kmc_bucket_count(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t bucket_bits, uint32_t *table,
+                                    kmc_result *result)
 {
-    int p = bucket_bits - 22; // table slice per bin <= 2^22 counters = 16 MB
-    if (p < binning::kMinBits) p = binning::kMinBits;
-    if (p > binning::kMaxBits) p = binning::kMaxBits;
-    return p;
+    return bucket_count(ctx, seqs, k, bucket_bits, table, 0, nullptr, result);
 }
 
-uint64_t binned_count_blocks(uint64_t n) { return binning::blocks_for<uint32_t>(n); }
-
-} // namespace kmc
+extern "C" int32_t kmc_bucket_count_async(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t bucket_bits, uint32_t *table,
+                                          uint32_t n_parts, void *const *events, kmc_result *result)
+{
+    if (!ctx) return KMC_E_BAD_ARG;
+    if (!events || n_parts < 1 || n_parts > 32 || (n_parts & (n_parts - 1)))
+        return fail(ctx, KMC_E_BAD_ARG, "n_parts must be a power of two <= 32 and events non-NULL");
+    for (uint32_t i = 0; i < n_parts; ++i)
+        if (!events[i]) return fail(ctx, KMC_E_BAD_ARG, "NULL event");
+    return bucket_count(ctx, seqs, k, bucket_bits, table, n_parts, events, result);
+}

@@ -79,28 +79,9 @@ cudaError_t group_slots(const uint64_t *win_off, uint64_t n, int g, uint64_t *sl
 cudaError_t tile_first_reads(const uint64_t *item_off, uint64_t n_seqs, uint64_t tile_items, uint64_t n_tiles,
                              uint64_t *tile_first, cudaStream_t stream);
 
-// buckets.cu: histogram of n bucket ids into a table too large for L2, by binning the ids first
-int binned_count_bin_bits(int bucket_bits);
-int apply_group(int dflt); // bins applied per launch (KMC_APPLY_GROUP overrides the default, for experiments)
-uint64_t binned_count_blocks(uint64_t n);
-// pulls table[0..n_counters) into L2; sink: 4 bytes of device memory on the table's device (never written in practice)
+// buckets.cu: pulls table[0..n_counters) into L2; sink: 4 bytes of device memory on the table's device (never written in
+// practice)
 cudaError_t warm_table(const uint32_t *table, uint64_t n_counters, int sm_count, uint32_t *sink, cudaStream_t stream);
-// events (may be NULL): n_parts events, events[i] recorded once the i-th of n_parts equal ranges of the table is final
-cudaError_t binned_count(const uint32_t *ids, uint64_t n, int bucket_bits, uint32_t *table, uint32_t *binned, uint64_t *matrix,
-                         uint64_t *offs, uint64_t *scan_tmp, int sm_count, cudaStream_t stream, uint32_t n_parts = 0,
-                         void *const *events = nullptr);
-
-// The same count for one-limb k-mers over an aligned uniform set with whole groups, ids produced and binned by ONE kernel into
-// bins of a fixed capacity plus a spill list (buckets.cu): fused_bin_ids, then fused_bin_apply.  Nothing synchronises.
-struct ExtractParams;
-bool fused_bin_enabled();
-uint64_t fused_bin_capacity(uint64_t n_ids);   // ids per bin
-uint64_t fused_bin_buffer_ids(uint64_t n_ids); // ids of the binned buffer (64 bins + the spill list)
-uint64_t fused_bin_state_bytes();              // bytes of the cursor block
-cudaError_t fused_bin_ids(ExtractParams p, int nx, int bucket_bits, uint32_t *binned, uint64_t cap, unsigned long long *state,
-                          cudaStream_t stream);
-cudaError_t fused_bin_apply(const uint32_t *binned, uint64_t cap, const unsigned long long *state, int bucket_bits, uint32_t *table,
-                            uint32_t *sink, int sm_count, cudaStream_t stream, uint32_t n_parts, void *const *events);
 
 // misc_kernels.cu -----------------------------------------------------------------------------
 cudaError_t launch_fx_hash(const uint64_t *kmers, uint64_t n, int n_limbs, uint64_t h0, uint64_t *out, int sm_count,

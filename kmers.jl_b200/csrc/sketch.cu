@@ -529,56 +529,34 @@ static int32_t kmer_count(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t
     c.overflow = overflow;
     CU(cudaMemsetAsync(distinct, 0, 16, stream));
     // A table beyond L2 (12 bytes per slot for one limb, 20 for two): write the k-mers out, bin them by the table slice
-    // they fall into and insert slice after slice (bin_insert_kernel), a group of slices -- 72 MB of one-limb table, 60 MB
-    // of two-limb table -- per launch.  Needs 16 (32) bytes per k-mer of temporary memory; without it the k-mers are
-    // inserted as they are produced.
-    const uint64_t slot_bytes = 8 * NL + 4;
-    const uint64_t table_bytes = slot_bytes << log2_capacity;
-    int bin_bits = static_cast<int>(log2_capacity) - 20; // <= 2^20 slots = 12 (20) MB per slice
-    bin_bits = std::max(binning::kMinBits, std::min(binning::kMaxBits, bin_bits));
-    bool binned = table_bytes > (96ull << 20) && static_cast<int>(log2_capacity) > bin_bits;
-    AsyncBuf kmers_buf, binned_buf, matrix_buf, offs_buf, scan_buf;
-    const uint64_t n_flat = (L.items + 1) * static_cast<uint64_t>(ge.g); // flat windows, rounded up to whole groups
-    if (binned) {
-        const uint64_t cells = binning::matrix_cells<BinKey<NL>>(L.total, bin_bits);
-        cudaError_t e = kmers_buf.alloc(ctx, round_up(n_flat * sizeof(Key), 256), stream);
-        if (e == cudaSuccess) e = binned_buf.alloc(ctx, round_up(n_flat * sizeof(Key), 256), stream);
-        if (e == cudaSuccess) e = matrix_buf.alloc(ctx, (cells + 1) * 8, stream);
-        if (e == cudaSuccess) e = offs_buf.alloc(ctx, (cells + 2) * 8, stream);
-        if (e == cudaSuccess) e = scan_buf.alloc(ctx, (scan_tmp_elems(cells) + 1) * 8, stream);
-        if (e != cudaSuccess) {
-            (void)cudaGetLastError();
-            binned = false;
-        }
-    }
-    if (binned) {
-        p.out_a = static_cast<uint64_t *>(kmers_buf.p);
+    // they fall into and insert slice after slice (bin_insert_kernel), a group of slices per launch (binning.cuh).  Needs
+    // 16 (32) bytes per k-mer of temporary memory; without it the k-mers are inserted as they are produced.
+    const uint64_t table_bytes = (8 * NL + 4ull) << log2_capacity;
+    const int bin_bits = binning::bin_bits(static_cast<int>(log2_capacity), binning::kKmerSliceBits);
+    binning::BinnedKeys<BinKey<NL>> bk;
+    if (table_bytes > binning::kL2Budget && bk.alloc(ctx, (L.items + 1) * static_cast<uint64_t>(ge.g), bin_bits, stream)) {
+        p.out_a = bk.written.template as<uint64_t>();
         p.vec_ok = 1;
         ExtractLaunchFn xfn = get_launcher(ge, mode == KMC_CANON ? MODE_CANON : MODE_FW, false, !L.uniform_len);
         if (!xfn) return fail(ctx, KMC_E_UNSUPPORTED, "no kernel for this K");
         CU(xfn(p, ctx->sm_count, stream));
-        const BinKey<NL> *kmers = static_cast<const BinKey<NL> *>(kmers_buf.p);
-        BinKey<NL> *sorted = static_cast<BinKey<NL> *>(binned_buf.p);
-        uint64_t *offs = static_cast<uint64_t *>(offs_buf.p);
         if constexpr (NL == 1)
-            CU(binning::partition<BinKey<NL>>(kmers, L.total, bin_bits, binning::KmerHashBin{64 - bin_bits}, sorted,
-                                       static_cast<uint64_t *>(matrix_buf.p), offs, static_cast<uint64_t *>(scan_buf.p), stream));
+            CU(bk.partition(L.total, binning::KmerHashBin{64 - bin_bits}, stream));
         else
-            CU(binning::partition<BinKey<NL>>(kmers, L.total, bin_bits, binning::KmerHashBin2{64 - bin_bits}, sorted,
-                                       static_cast<uint64_t *>(matrix_buf.p), offs, static_cast<uint64_t *>(scan_buf.p), stream));
-        const uint64_t n_blocks = binning::blocks_for<BinKey<NL>>(L.total);
+            CU(bk.partition(L.total, binning::KmerHashBin2{64 - bin_bits}, stream));
+        const Key *sorted = bk.binned.template as<const Key>();
         const uint64_t slice = 1ull << (log2_capacity - bin_bits); // slots per bin
-        const int group = apply_group(NL == 1 ? 6 : 3);
-        for (int b = 0; b < (1 << bin_bits); b += group) {
-            const int b_end = std::min(b + group, 1 << bin_bits);
+        auto apply = [&](int b, int b_end) {
             const uint64_t slots = slice * static_cast<uint64_t>(b_end - b);
-            CU(warm_table(reinterpret_cast<const uint32_t *>(table_keys + static_cast<uint64_t>(b) * slice), 2 * NL * slots, ctx->sm_count,
-                          warm_sink(ctx), stream));
-            CU(warm_table(vals + static_cast<uint64_t>(b) * slice, slots, ctx->sm_count, warm_sink(ctx), stream));
+            cudaError_t e = warm_table(reinterpret_cast<const uint32_t *>(table_keys + static_cast<uint64_t>(b) * slice), 2 * NL * slots,
+                                       ctx->sm_count, warm_sink(ctx), stream);
+            if (e == cudaSuccess) e = warm_table(vals + static_cast<uint64_t>(b) * slice, slots, ctx->sm_count, warm_sink(ctx), stream);
+            if (e != cudaSuccess) return e;
             bin_insert_kernel<Key><<<static_cast<unsigned>(ctx->sm_count * 16), 256, 0, stream>>>(
-                reinterpret_cast<const Key *>(sorted), offs, n_blocks, b, b_end, table_keys, vals, log2_capacity, distinct, overflow);
-        }
-        CU(cudaGetLastError());
+                sorted, bk.offs.template as<uint64_t>(), bk.n_blocks, b, b_end, table_keys, vals, log2_capacity, distinct, overflow);
+            return cudaGetLastError();
+        };
+        CU(binning::apply_groups(1 << bin_bits, binning::kmer_group(NL), 0, nullptr, stream, apply));
     } else {
         const bool ragged = !L.uniform_len, canon = mode == KMC_CANON;
         ConsumeLaunchFn fn = NL == 1 ? consume_launcher<OP_TABLE>(ge, ragged, canon) : pick_consume_nx<2, OP_TABLE2>(ge.nx, ragged, canon);

@@ -492,7 +492,9 @@ def test_bucket_count_fused_bins_and_spill_list(kc):
         assert n == h.size and np.array_equal(np.nonzero(table)[0], idx) and np.array_equal(table[idx], cnt.astype(np.uint32))
 
 
-@pytest.mark.parametrize("k,bits", [(31, 20), (63, 12), (15, 28)])
+# (63, 27) and (21, 26): tables beyond L2 that the fused bins do not take, so the exact path bins the ids of
+# extract_aligned_kernel (88 windows per read, a multiple of G = 4) and of extract_kernel (130 windows, not a multiple of 8)
+@pytest.mark.parametrize("k,bits", [(31, 20), (63, 12), (15, 28), (63, 27), (21, 26)])
 def test_bucket_count(kc, k, bits):
     rng = np.random.default_rng(k)
     n_reads, length, stride = 20_000, 150, 5
@@ -508,50 +510,56 @@ def test_bucket_count(kc, k, bits):
 @pytest.mark.parametrize("bits,n_parts", [(20, 4), (26, 8), (27, 32), (26, 1)])
 def test_bucket_count_async_progress_events(kc, ctx, bits, n_parts):
     """kmc_bucket_count_async: same table as the synchronous call; every progress event completes; a range whose
-    event has fired is final (checked by copying it out on a second stream that only waits for that event)."""
+    event has fired is final (checked by copying it out on a second stream that only waits for that event).  At bits = 26
+    also over a ragged set, which the exact binned path counts (the uniform set takes the fused bins)."""
     import ctypes as C
     import torch
     from kmerscuda import _abi, sharding
     rng = np.random.default_rng(bits)
     n_reads, length, stride, k = 30_000, 150, 5, 31
     words = rng.integers(0, 2**64, size=n_reads * stride, dtype=np.uint64)
-    rs = kc.ReadSet(2, words, n_reads, uniform_len=length, uniform_stride_words=stride)
-    want, n, _ = kc.bucket_count(rs, k, bits, ctx=ctx)
-    drs = kc.DeviceReadSet(ctx, rs)
-    main, side = torch.cuda.Stream(), torch.cuda.Stream()
-    with torch.cuda.stream(main):
-        ctx.set_stream(main.cuda_stream)
-        try:
-            table = torch.zeros(1 << bits, dtype=torch.int32, device="cuda")
-            events = [torch.cuda.Event() for _ in range(n_parts)]
-            for e in events:
-                e.record(main)
-            handles = (C.c_void_p * n_parts)(*[C.c_void_p(e.cuda_event) for e in events])
-            res = _abi.kmc_result()
-            ctx._check(ctx.lib.kmc_bucket_count_async(ctx.handle, C.byref(drs.desc), k, bits, table.data_ptr(), n_parts, handles,
-                                                      C.byref(res)))
-            part = table.numel() // n_parts
-            copies = []
-            with torch.cuda.stream(side):
-                for i, e in enumerate(events):
-                    side.wait_event(e)
-                    copies.append(table[i * part:(i + 1) * part].clone())
-            side.synchronize()
-            main.synchronize()
-            assert all(e.query() for e in events)
-            assert int(res.n_written) == n
-            assert np.array_equal(table.cpu().numpy().view(np.uint32), want)
-            assert np.array_equal(torch.cat(copies).cpu().numpy().view(np.uint32), want)
-            # one rank: the overlapped count + merge helper is the same count
-            table.zero_()
-            assert sharding.count_and_merge_table(ctx, drs.desc, k, bits, table, n_parts=n_parts) == n
-            main.synchronize()
-            assert np.array_equal(table.cpu().numpy().view(np.uint32), want)
-            # argument checks
-            bad = (C.c_void_p * 3)(*[C.c_void_p(e.cuda_event) for e in events[:1] * 3])
-            assert ctx.lib.kmc_bucket_count_async(ctx.handle, C.byref(drs.desc), k, bits, table.data_ptr(), 3, bad, C.byref(res)) != 0
-        finally:
-            ctx.set_stream(None)
+    sets = [kc.ReadSet(2, words, n_reads, uniform_len=length, uniform_stride_words=stride)]
+    if bits == 26:
+        lens = [int(x) for x in rng.integers(0, 300, size=30_000)]
+        _, rwords, off, ln = make_ragged(rng, lens)
+        sets.append(kc.ReadSet(2, rwords, len(lens), seq_word_offset=off, seq_len=ln))
+    for rs in sets:
+        want, n, _ = kc.bucket_count(rs, k, bits, ctx=ctx)
+        drs = kc.DeviceReadSet(ctx, rs)
+        main, side = torch.cuda.Stream(), torch.cuda.Stream()
+        with torch.cuda.stream(main):
+            ctx.set_stream(main.cuda_stream)
+            try:
+                table = torch.zeros(1 << bits, dtype=torch.int32, device="cuda")
+                events = [torch.cuda.Event() for _ in range(n_parts)]
+                for e in events:
+                    e.record(main)
+                handles = (C.c_void_p * n_parts)(*[C.c_void_p(e.cuda_event) for e in events])
+                res = _abi.kmc_result()
+                ctx._check(ctx.lib.kmc_bucket_count_async(ctx.handle, C.byref(drs.desc), k, bits, table.data_ptr(), n_parts, handles,
+                                                          C.byref(res)))
+                part = table.numel() // n_parts
+                copies = []
+                with torch.cuda.stream(side):
+                    for i, e in enumerate(events):
+                        side.wait_event(e)
+                        copies.append(table[i * part:(i + 1) * part].clone())
+                side.synchronize()
+                main.synchronize()
+                assert all(e.query() for e in events)
+                assert int(res.n_written) == n
+                assert np.array_equal(table.cpu().numpy().view(np.uint32), want)
+                assert np.array_equal(torch.cat(copies).cpu().numpy().view(np.uint32), want)
+                # one rank: the overlapped count + merge helper is the same count
+                table.zero_()
+                assert sharding.count_and_merge_table(ctx, drs.desc, k, bits, table, n_parts=n_parts) == n
+                main.synchronize()
+                assert np.array_equal(table.cpu().numpy().view(np.uint32), want)
+                # argument checks
+                bad = (C.c_void_p * 3)(*[C.c_void_p(e.cuda_event) for e in events[:1] * 3])
+                assert ctx.lib.kmc_bucket_count_async(ctx.handle, C.byref(drs.desc), k, bits, table.data_ptr(), 3, bad, C.byref(res)) != 0
+            finally:
+                ctx.set_stream(None)
 
 
 # ----------------------------------------------- full-size properties (BASELINE config C2 shape)

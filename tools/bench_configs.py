@@ -145,13 +145,14 @@ def case_c4(ctx, steps, scale):
 
 
 def case_c5(ctx, steps, scale):
-    n_reads, length, stride, k = int(25_000_000 * scale), 150, 5, 31
-    wpr = length - k + 1
+    """K = 31 at B = 20 and 24 (direct increments) and 28 (fused bins); K = 63 at B = 28 (two limbs: the exact binned path)."""
+    n_reads, length, stride = int(25_000_000 * scale), 150, 5
     words = rand_words_2bit(n_reads * stride, 13)
     words.view(n_reads, stride)[:, stride - 1] &= (1 << (2 * (length - 32 * (stride - 1)))) - 1
     desc = _abi.kmc_seqs(words.data_ptr(), words.numel(), n_reads, None, None, length, stride, 2, 0)
     res = _abi.kmc_result()
-    for bits in (20, 24, 28):
+    for k, bits in ((31, 20), (31, 24), (31, 28), (63, 28)):
+        wpr = length - k + 1
         table = torch.zeros(1 << bits, dtype=torch.int32, device="cuda")
         torch.cuda.synchronize()
 
@@ -161,8 +162,8 @@ def case_c5(ctx, steps, scale):
                 raise RuntimeError(ctx.lib.kmc_last_error(ctx.handle).decode())
         med, mn = timed(ctx, step, steps)
         n = n_reads * wpr
-        emit("C5 (per-GPU part) canonical 31-mer bucket table, B=%d, %d x 150 bp reads" % (bits, n_reads), n,
-             (0.3125 + 8) * n, med, mn, {"table_bytes": 4 << bits})
+        emit("C5 (per-GPU part) canonical %d-mer bucket table, B=%d, %d x 150 bp reads" % (k, bits, n_reads), n,
+             (0.25 * length / wpr + 8) * n, med, mn, {"table_bytes": 4 << bits})
         del table
 
 
