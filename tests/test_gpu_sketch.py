@@ -130,10 +130,21 @@ def test_kmer_table_matches_unique_counts(kc, k, canonical):
         x.free()
 
 
-@pytest.mark.parametrize("k,canonical,log2cap,ragged", [(21, True, 23, False), (31, False, 24, True), (32, True, 28, True)])
+@pytest.mark.parametrize("k,canonical,log2cap,ragged", [(21, True, 24, False), (31, False, 24, True), (32, True, 28, True)])
 def test_kmer_table_beyond_l2_takes_the_binned_path(kc, k, canonical, log2cap, ragged):
-    """Tables larger than L2 are filled slice by slice from binned k-mers (64 bins for 2^23 / 2^24 slots, 256 for
-    2^28); the result is the same table content."""
+    """Tables larger than L2 (more than 96 MiB: 12 bytes per slot) are filled slice by slice from binned k-mers (64 bins
+    for 2^24 slots, 256 for 2^28), from a uniform and from ragged sets; the result is the same table content."""
+    count_twice(kc, k, canonical, log2cap, ragged)
+
+
+def test_kmer_table_at_exactly_the_l2_budget_streams(kc):
+    """2^23 one-limb slots are 96 MiB, exactly the L2 budget: the largest table that is still updated directly (the
+    binned path starts above it)."""
+    count_twice(kc, 21, True, 23, False)
+
+
+def count_twice(kc, k, canonical, log2cap, ragged):
+    """A 3000-read set from a 60 kbp genome counted into a fresh table of 2^log2cap slots, then once more."""
     rng = np.random.default_rng(900 + k)
     genome = rng.integers(0, 4, size=60_000).astype(np.uint64)
     n_reads = 3000
