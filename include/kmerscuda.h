@@ -272,6 +272,43 @@ int32_t kmc_kmer_table2_merge(kmc_ctx *ctx, uint64_t *keys, uint32_t *vals, uint
                               const uint64_t *src_keys /* [n_src][2] */, const uint32_t *src_vals, uint64_t n_src, uint64_t *n_new);
 int32_t kmc_kmer_table2_export(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
                                uint64_t *out_keys /* [capacity][2] */, uint32_t *out_vals, uint64_t capacity, uint64_t *n_out);
+/* Read-only queries of a table filled by kmc_kmer_count / kmc_kmer_count2 (or merged into).  Precondition: no count or
+ * merge into the same table is in flight -- calls on one context are stream ordered, so this holds unless another
+ * context writes the table.  A key that is not in the table has count 0.  Every entry point below returns
+ * KMC_E_BAD_ARG for a NULL pointer, log2_capacity outside 1..40, and two-limb keys / query / out_keys that are not
+ * 16-byte aligned.
+ *
+ * The count of every window of a read set: out_counts[i] (device u32[capacity]) = table[k-mer i], in the order
+ * kmc_extract writes the same k-mers (so out_counts[i] belongs to out.a[i]) -- the second pass of a k-mer-spectrum
+ * error corrector or read filter.  The k-mers must be looked up with the mode the table was counted with (KMC_FW or
+ * KMC_CANON); K, mode and source are checked as by kmc_kmer_count.  result->n_written = windows; capacity < windows is
+ * KMC_E_OUT_TOO_SMALL and nothing is written.  Tables of any size are probed directly. */
+int32_t kmc_kmer_lookup(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t mode, const uint64_t *keys, const uint32_t *vals,
+                        uint32_t log2_capacity, uint32_t *out_counts, uint64_t capacity, kmc_result *result);
+/* The same for a two-limb table (kmc_kmer_count2): K and mode as there, keys u64[2^cap][2] */
+int32_t kmc_kmer_lookup2(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t mode, const uint64_t *keys /* [2^cap][2] */,
+                         const uint32_t *vals, uint32_t log2_capacity, uint32_t *out_counts, uint64_t capacity, kmc_result *result);
+/* out_counts[i] = table[query[i]] for n keys in device memory (query u64[n] / u64[n][2]); n = 0 does nothing */
+int32_t kmc_kmer_table_get(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
+                           const uint64_t *query, uint64_t n, uint32_t *out_counts);
+int32_t kmc_kmer_table2_get(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
+                            const uint64_t *query /* [n][2] */, uint64_t n, uint32_t *out_counts);
+/* The count spectrum: hist[min(count, n_bins - 1)] += 1 for every key of the table, so the last bin holds every count
+ * of n_bins - 1 and more (bin 0 holds keys merged in with a zero count).  hist: device u64[n_bins], caller-zeroed; it
+ * accumulates, so after kmc_kmer_table_exchange the histograms of the owned tables summed over the ranks with
+ * kmc_allreduce_u64 are the spectrum of the whole input.  n_bins in 1..16384. */
+int32_t kmc_kmer_table_histogram(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity, uint64_t *hist,
+                                 uint32_t n_bins);
+int32_t kmc_kmer_table2_histogram(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity, uint64_t *hist,
+                                  uint32_t n_bins);
+/* kmc_kmer_table_export of the entries with min_count <= count <= max_count only (the solid k-mers); *n_out and
+ * KMC_E_OUT_TOO_SMALL as there, nothing is written past capacity.  min_count > max_count is KMC_E_BAD_ARG. */
+int32_t kmc_kmer_table_export_range(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
+                                    uint32_t min_count, uint32_t max_count, uint64_t *out_keys, uint32_t *out_vals,
+                                    uint64_t capacity, uint64_t *n_out);
+int32_t kmc_kmer_table2_export_range(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
+                                     uint32_t min_count, uint32_t max_count, uint64_t *out_keys /* [capacity][2] */,
+                                     uint32_t *out_vals, uint64_t capacity, uint64_t *n_out);
 
 /* ---- multi-GPU (SURVEY.md 8b / 8e) ---------------------------------------------------------------
  * The reference has no collective (it is single-threaded Julia); north_star shards reads over the GPUs of a box

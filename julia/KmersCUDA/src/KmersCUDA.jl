@@ -32,7 +32,7 @@ using Kmers: FwKmers, FwRvIterator, CanonicalKmers, UnambiguousKmers, SpacedKmer
 using Libdl
 
 export fx_hash_device, hash_device, extract, set_library!, minhash_sketch, composition, minimizers, count_kmers,
-    bucket_count, DeviceVector, Group, free!
+    bucket_count, DeviceVector, Group, free!, KmerCountTable, counts, spectrum
 
 # ---------------------------------------------------------------------------------------------
 # library handle
@@ -738,6 +738,128 @@ function count_kmers(it::Union{FwKmers{A, K}, CanonicalKmers{A, K}};
     keys, vals = Array(ok), Array(ov)
     foreach(free!, (dk, dv, ok, ov))
     # Kmer{A,K,N} is N UInt64 limbs, head first: the [N, n] export is a vector of n k-mers
+    kmers = reinterpret(T, keys)
+    return Dict{T, Int}(kmers[i] => Int(vals[i]) for i in eachindex(vals))
+end
+
+"""
+    t = KmerCountTable(Kmer{A,K}, log2_capacity)
+    count!(t, FwKmers{A,K}(seq) | CanonicalKmers{A,K}(seq))     # adds every k-mer (kmc_kmer_count / _count2)
+    counts(t, it) -> Vector{UInt32}                             # the count of every k-mer of `it`, in iteration order
+    get(t, kmers::Vector{<:Kmer}) -> Vector{UInt32}             # the count of each k-mer, 0 when absent
+    spectrum(t, n_bins) -> Vector{UInt64}                       # bin c + 1 = keys with count c, the last bin the rest
+    Dict(t; min_count = 1, max_count = typemax(UInt32))         # the keys whose count lies in [min_count, max_count]
+
+An exact k-mer count table that stays in device memory, so that it can be queried without copying it out: the second
+pass of a k-mer-spectrum error corrector (`counts`), the trusted / solid k-mers (`Dict` with bounds) and the count
+spectrum.  One limb for K <= 32, two for K = 33..64.  Every iterator counted into or looked up in one table must be
+of the same kind (forward or canonical).
+"""
+mutable struct KmerCountTable{T <: Kmer}
+    ctx::Context
+    log2_capacity::Int
+    keys::DeviceVector{UInt64}
+    vals::DeviceVector{UInt32}
+    mode::Int32                                  # the iterator kind counted so far, -1 before the first count!
+    n_keys::Int
+end
+
+function KmerCountTable(::Type{Kmer{A, K}}, log2_capacity::Integer; ctx::Context = default_context()) where {A <: NucleicAcidAlphabet{2}, K}
+    K <= 64 || throw(ArgumentError("KmerCountTable holds k-mers of one or two limbs (K <= 64)"))
+    T = derive_type(Kmer{A, K})
+    N = K <= 32 ? 1 : 2
+    dk, dv = DeviceVector{UInt64}(ctx, N << log2_capacity), DeviceVector{UInt32}(ctx, 1 << log2_capacity)
+    zero!(dk, 0xff)
+    zero!(dv)
+    return KmerCountTable{T}(ctx, Int(log2_capacity), dk, dv, Int32(-1), 0)   # (the DeviceVectors free themselves)
+end
+
+limbs(::KmerCountTable{Kmer{A, K, N}}) where {A, K, N} = N
+
+function check_mode!(t::KmerCountTable, mode::Int32)
+    t.mode == -1 && (t.mode = mode)
+    t.mode == mode || throw(ArgumentError("the table was counted from $(t.mode == KMC_CANON ? "canonical" : "forward") k-mers"))
+end
+
+function Base.count!(t::KmerCountTable{Kmer{A, K, N}}, it::Union{FwKmers{A, K}, CanonicalKmers{A, K}}) where {A, K, N}
+    mode = Int32(mode_of(typeof(it)))
+    check_mode!(t, mode)
+    res, ctx = KmcResult(), t.ctx
+    with_device_sequence(ctx, source(it)) do d
+        st = limbs(t) == 1 ?
+            ccall((:kmc_kmer_count, LIB[]), Int32, (Ptr{Cvoid}, Ptr{KmcSeqs}, Int32, Int32, Ptr{Cvoid}, Ptr{Cvoid}, UInt32, Ref{KmcResult}),
+                ctx.handle, d, K, mode, t.keys.ptr, t.vals.ptr, UInt32(t.log2_capacity), res) :
+            ccall((:kmc_kmer_count2, LIB[]), Int32, (Ptr{Cvoid}, Ptr{KmcSeqs}, Int32, Int32, Ptr{Cvoid}, Ptr{Cvoid}, UInt32, Ref{KmcResult}),
+                ctx.handle, d, K, mode, t.keys.ptr, t.vals.ptr, UInt32(t.log2_capacity), res)
+        st == KMC_OK || throw_status(ctx, st, res, A)
+    end
+    t.n_keys += Int(res.digest[1])
+    return t
+end
+
+function counts(t::KmerCountTable{Kmer{A, K, N}}, it::Union{FwKmers{A, K}, CanonicalKmers{A, K}}) where {A, K, N}
+    mode = Int32(mode_of(typeof(it)))
+    check_mode!(t, mode)
+    seq, res, ctx = source(it), KmcResult(), t.ctx
+    n = max(0, length(seq) - K + 1)
+    dout = DeviceVector{UInt32}(ctx, n)
+    with_device_sequence(ctx, seq) do d
+        st = limbs(t) == 1 ?
+            ccall((:kmc_kmer_lookup, LIB[]), Int32,
+                (Ptr{Cvoid}, Ptr{KmcSeqs}, Int32, Int32, Ptr{Cvoid}, Ptr{Cvoid}, UInt32, Ptr{Cvoid}, UInt64, Ref{KmcResult}),
+                ctx.handle, d, K, mode, t.keys.ptr, t.vals.ptr, UInt32(t.log2_capacity), dout.ptr, n, res) :
+            ccall((:kmc_kmer_lookup2, LIB[]), Int32,
+                (Ptr{Cvoid}, Ptr{KmcSeqs}, Int32, Int32, Ptr{Cvoid}, Ptr{Cvoid}, UInt32, Ptr{Cvoid}, UInt64, Ref{KmcResult}),
+                ctx.handle, d, K, mode, t.keys.ptr, t.vals.ptr, UInt32(t.log2_capacity), dout.ptr, n, res)
+        st == KMC_OK || throw_status(ctx, st, res, A)
+    end
+    out = Array(dout)
+    free!(dout)
+    return out
+end
+
+function Base.get(t::KmerCountTable{T}, kmers::Vector{T}) where {T <: Kmer}
+    ctx = t.ctx
+    dq, dout = upload(ctx, reinterpret(UInt64, kmers)), DeviceVector{UInt32}(ctx, length(kmers))
+    check(ctx, limbs(t) == 1 ?
+        ccall((:kmc_kmer_table_get, LIB[]), Int32, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, UInt32, Ptr{Cvoid}, UInt64, Ptr{Cvoid}),
+            ctx.handle, t.keys.ptr, t.vals.ptr, UInt32(t.log2_capacity), dq.ptr, UInt64(length(kmers)), dout.ptr) :
+        ccall((:kmc_kmer_table2_get, LIB[]), Int32, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, UInt32, Ptr{Cvoid}, UInt64, Ptr{Cvoid}),
+            ctx.handle, t.keys.ptr, t.vals.ptr, UInt32(t.log2_capacity), dq.ptr, UInt64(length(kmers)), dout.ptr))
+    out = Array(dout)
+    free!(dq)
+    free!(dout)
+    return out
+end
+
+function spectrum(t::KmerCountTable, n_bins::Integer)
+    ctx = t.ctx
+    dh = DeviceVector{UInt64}(ctx, n_bins)
+    zero!(dh)
+    check(ctx, limbs(t) == 1 ?
+        ccall((:kmc_kmer_table_histogram, LIB[]), Int32, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, UInt32, Ptr{Cvoid}, UInt32),
+            ctx.handle, t.keys.ptr, t.vals.ptr, UInt32(t.log2_capacity), dh.ptr, UInt32(n_bins)) :
+        ccall((:kmc_kmer_table2_histogram, LIB[]), Int32, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, UInt32, Ptr{Cvoid}, UInt32),
+            ctx.handle, t.keys.ptr, t.vals.ptr, UInt32(t.log2_capacity), dh.ptr, UInt32(n_bins)))
+    out = Array(dh)
+    free!(dh)
+    return out
+end
+
+function Base.Dict(t::KmerCountTable{T}; min_count::Integer = 1, max_count::Integer = typemax(UInt32)) where {T <: Kmer}
+    ctx, N, n = t.ctx, limbs(t), max(1, t.n_keys)
+    ok, ov, nout = DeviceVector{UInt64}(ctx, N * n), DeviceVector{UInt32}(ctx, n), Ref{UInt64}(0)
+    check(ctx, limbs(t) == 1 ?
+        ccall((:kmc_kmer_table_export_range, LIB[]), Int32,
+            (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, UInt32, UInt32, UInt32, Ptr{Cvoid}, Ptr{Cvoid}, UInt64, Ptr{UInt64}),
+            ctx.handle, t.keys.ptr, t.vals.ptr, UInt32(t.log2_capacity), UInt32(min_count), UInt32(max_count), ok.ptr, ov.ptr, UInt64(n), nout) :
+        ccall((:kmc_kmer_table2_export_range, LIB[]), Int32,
+            (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, UInt32, UInt32, UInt32, Ptr{Cvoid}, Ptr{Cvoid}, UInt64, Ptr{UInt64}),
+            ctx.handle, t.keys.ptr, t.vals.ptr, UInt32(t.log2_capacity), UInt32(min_count), UInt32(max_count), ok.ptr, ov.ptr, UInt64(n), nout))
+    m = Int(nout[])
+    keys, vals = Array(truncate!(ok, N * m)), Array(truncate!(ov, m))
+    free!(ok)
+    free!(ov)
     kmers = reinterpret(T, keys)
     return Dict{T, Int}(kmers[i] => Int(vals[i]) for i in eachindex(vals))
 end

@@ -55,6 +55,29 @@ end
     @test_throws ArgumentError KmersCUDA.count_kmers(CanonicalDNAMers{65}(s))
 end
 
+@testset "KmerCountTable: per-window counts, get, spectrum, solid k-mers" begin
+    genome = randdnaseq(RNG, 3_000)
+    s = LongDNA{2}(reduce(*, [genome[i:i+299] for i in rand(RNG, 1:2700, 30)]))
+    q = LongDNA{2}(genome[1:1000] * randdnaseq(RNG, 1000))      # half of its k-mers are absent
+    for (K, canonical) in ((21, true), (31, false), (47, true), (63, false))
+        it(x) = canonical ? CanonicalDNAMers{K}(x) : FwDNAMers{K}(x)
+        want = Dict{eltype(it(s)), Int}()
+        for m in it(s)
+            want[m] = get(want, m, 0) + 1
+        end
+        t = KmerCountTable(Kmer{DNAAlphabet{2}, K}, 14)
+        count!(t, it(s))
+        @test counts(t, it(q)) == [get(want, m, 0) for m in it(q)]
+        ks = collect(it(q))
+        @test get(t, ks) == [get(want, m, 0) for m in ks]
+        h = spectrum(t, 8)
+        @test h == [Base.count(c -> min(c, 7) == b, values(want)) for b in 0:7]
+        @test Dict(t) == want
+        @test Dict(t; min_count = 2, max_count = 5) == filter(p -> 2 <= p.second <= 5, want)
+        @test_throws ArgumentError counts(t, canonical ? FwDNAMers{K}(q) : CanonicalDNAMers{K}(q))
+    end
+end
+
 @testset "LongSubSeq views (reference: test/runtests.jl:154-169)" begin
     s2 = LongDNA{2}(randdnaseq(RNG, 1000))
     s4 = LongDNA{4}(s2); s4[500] = DNA_N

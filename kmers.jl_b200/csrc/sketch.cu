@@ -13,6 +13,9 @@
 //                       kmc_kmer_table_merge / _export move entries between tables (multi-GPU merge)
 //   kmc_kmer_count2     the same table for two-limb k-mers, K = 33..64 (table_keys.cuh): 16-byte keys, claimed by
 //                       one 128-bit compare-and-swap; kmc_kmer_table2_merge / _export
+//   kmc_kmer_lookup(2)  read-only queries of a counted table: the count of every window of a read set (in
+//                       kmc_extract's order), of a list of keys (_get), the count spectrum (_histogram) and the
+//                       keys whose count lies in a range (_export_range)
 //
 // Both run consume_kernel: the same (read, group slot) work items, block load and static funnel
 // shifts as extract_kernel (kmer_core.cuh), with the stores replaced by a small functor.
@@ -38,7 +41,16 @@ namespace kmc {
 
 namespace {
 
-enum : int { OP_HASH_HIST = 0, OP_HASH_BELOW = 1, OP_COMPOSITION = 2, OP_COMPOSITION_SHARED = 3, OP_TABLE = 4, OP_TABLE2 = 5 };
+enum : int {
+    OP_HASH_HIST = 0,
+    OP_HASH_BELOW = 1,
+    OP_COMPOSITION = 2,
+    OP_COMPOSITION_SHARED = 3,
+    OP_TABLE = 4,
+    OP_TABLE2 = 5,
+    OP_LOOKUP = 6,
+    OP_LOOKUP2 = 7
+};
 
 // kEmptyKey (table_keys.cuh) is never a k-mer: one limb, K <= 31, or K = 32 canonical (the all-T 32-mer is not
 // canonical); two limbs {~0, ~0}, K <= 63, or K = 64 canonical.
@@ -101,6 +113,24 @@ __device__ __forceinline__ int table_add(ulonglong2 *keys, uint32_t *vals, uint3
     return kTableFull;
 }
 
+// table[key], 0 for a key that is not in the table: the probe of table_add without its atomics.  Precondition: no
+// count or merge into the same table is in flight (calls on one context are stream ordered), so a two-limb slot read
+// by one 16-byte load is never half written.  A full table that lacks the key ends after 2^log2cap probes.
+template <typename Key>
+__device__ __forceinline__ uint32_t table_find(const Key *__restrict__ keys, const uint32_t *__restrict__ vals, uint32_t log2cap,
+                                               Key key, uint64_t hash)
+{
+    const uint64_t mask = (1ull << log2cap) - 1;
+    uint64_t slot = hash >> (64 - log2cap);
+    for (uint64_t probes = 0; probes <= mask; ++probes) {
+        const Key cur = keys[slot];
+        if (key_free(cur)) return 0;
+        if (key_equal(cur, key)) return vals[slot];
+        slot = (slot + 1) & mask;
+    }
+    return 0;
+}
+
 // adds the new keys a thread has seen to *distinct: one atomic per warp (all 32 lanes must call)
 __device__ __forceinline__ void add_distinct(unsigned long long *distinct, uint32_t n_new)
 {
@@ -122,6 +152,7 @@ struct ConsumeParams {
     unsigned long long *distinct;  // OP_TABLE: keys in the table
     uint32_t *overflow;            // OP_TABLE*: set when a k-mer found no slot
     ulonglong2 *keys2;             // OP_TABLE2: two-limb keys, ulonglong2[2^log2cap] ({~0, ~0} = free), vals = table
+    uint32_t *out_counts;          // OP_LOOKUP*: u32 per window, at its flat window index (kmc_extract's order)
 };
 
 constexpr int kSharedCompositionMax = 4096; // 4^6 counters = 16 KB of shared memory
@@ -137,6 +168,7 @@ __global__ void __launch_bounds__(kBlockThreads) consume_kernel(const ExtractPar
     constexpr int G = GroupOf<N>::G;
     __shared__ TileShared<RAGGED> sh;
     constexpr bool SHARED_HIST = (OP == OP_COMPOSITION_SHARED || OP == OP_HASH_HIST);
+    constexpr bool LOOKUP = (OP == OP_LOOKUP || OP == OP_LOOKUP2);
     __shared__ uint32_t s_hist[SHARED_HIST ? kSharedCompositionMax : 1];
     const uint64_t tile_base = static_cast<uint64_t>(blockIdx.x) * kTileItems;
     if (SHARED_HIST) {
@@ -175,6 +207,7 @@ __global__ void __launch_bounds__(kBlockThreads) consume_kernel(const ExtractPar
         if (jhi > jlo) {
             uint64_t fw[G][N], rv[G][N];
             block_kmers<N, NX, G, true, CANON>(x, p.s0, p.head_mask, fw, rv);
+            uint32_t found[LOOKUP ? G : 1]; // OP_LOOKUP*: the counts of the item's windows [jlo, jhi)
 #pragma unroll
             for (int j = 0; j < G; ++j) {
                 if (j < jlo || j >= jhi) continue;
@@ -183,6 +216,14 @@ __global__ void __launch_bounds__(kBlockThreads) consume_kernel(const ExtractPar
                 uint64_t a[N];
 #pragma unroll
                 for (int i = 0; i < N; ++i) a[i] = take_fw ? fw[j][i] : rv[j][i];
+                if constexpr (OP == OP_LOOKUP) {
+                    found[j] = table_find<unsigned long long>(c.keys, c.table, c.log2cap, a[N - 1], fx_hash<N>(a, 0));
+                    continue;
+                } else if constexpr (OP == OP_LOOKUP2) {
+                    const ulonglong2 key = make_ulonglong2(a[0], a[N - 1]);
+                    found[j] = table_find(c.keys2, c.table, c.log2cap, key, key_hash(key));
+                    continue;
+                }
                 if (OP == OP_HASH_HIST) {
                     atomicAdd(s_hist + (fx_hash<N>(a, 0) >> c.shift), 1u);
                 } else if (OP == OP_HASH_BELOW) {
@@ -204,6 +245,21 @@ __global__ void __launch_bounds__(kBlockThreads) consume_kernel(const ExtractPar
                     atomicAdd(c.table + a[N - 1], 1u); // as_integer(kmer): K <= 14, one limb
                 } else {
                     atomicAdd(s_hist + a[N - 1], 1u);
+                }
+            }
+            if constexpr (LOOKUP) {
+                // a whole group is 4 G bytes at a multiple of 4 G: one vector store when the base allows it (p.vec_ok)
+                uint32_t *dst = c.out_counts + (ALIGNED ? item : cur.q) * G;
+                if (jlo == 0 && jhi == G && p.vec_ok && (G == 8 || G == 4)) {
+                    uint64_t w[G / 2];
+#pragma unroll
+                    for (int t = 0; t < G / 2; ++t) w[t] = found[2 * t] | (static_cast<uint64_t>(found[2 * t + 1]) << 32);
+                    if (G == 8) st_v4(reinterpret_cast<uint64_t *>(dst), w[0], w[1 % (G / 2)], w[2 % (G / 2)], w[3 % (G / 2)]);
+                    else st_v2(reinterpret_cast<uint64_t *>(dst), w[0], w[1 % (G / 2)]);
+                } else {
+#pragma unroll
+                    for (int j = 0; j < G; ++j)
+                        if (j >= jlo && j < jhi) dst[j] = found[j];
                 }
             }
         }
@@ -309,16 +365,19 @@ __global__ void __launch_bounds__(256) bin_insert_kernel(const Key *__restrict__
     add_distinct(distinct, n_new);
 }
 
-template <typename Key>
+// RANGE: only the entries with min_count <= count <= max_count
+template <typename Key, bool RANGE = false>
 __global__ void __launch_bounds__(256) table_export_kernel(const Key *__restrict__ keys, const uint32_t *__restrict__ vals,
                                                            uint64_t n_slots, Key *__restrict__ out_keys,
                                                            uint32_t *__restrict__ out_vals, uint64_t capacity,
-                                                           unsigned long long *cursor)
+                                                           unsigned long long *cursor, uint32_t min_count = 0,
+                                                           uint32_t max_count = ~0u)
 {
     for (uint64_t i = static_cast<uint64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < n_slots;
          i += static_cast<uint64_t>(gridDim.x) * blockDim.x) {
         const Key key = keys[i];
         if (key_free(key)) continue;
+        if (RANGE && (vals[i] < min_count || vals[i] > max_count)) continue;
         const uint32_t active = __activemask(); // warp-aggregated append: one atomic per converged group
         const int leader = __ffs(active) - 1;
         unsigned long long base = 0;
@@ -330,6 +389,54 @@ __global__ void __launch_bounds__(256) table_export_kernel(const Key *__restrict
             out_vals[at] = vals[i];
         }
     }
+}
+
+// out[i] = table[query[i]], 0 for a key that is not in the table
+template <typename Key>
+__global__ void __launch_bounds__(256) table_get_kernel(const Key *__restrict__ keys, const uint32_t *__restrict__ vals, uint32_t log2cap,
+                                                        const Key *__restrict__ query, uint64_t n, uint32_t *__restrict__ out)
+{
+    for (uint64_t i = static_cast<uint64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < n;
+         i += static_cast<uint64_t>(gridDim.x) * blockDim.x) {
+        const Key key = query[i];
+        out[i] = table_find(keys, vals, log2cap, key, key_hash(key));
+    }
+}
+
+// The count spectrum: hist[min(count, n_bins - 1)] += 1 for every key of the table.  Each block counts into n_bins
+// shared counters (dynamic shared memory) and adds its non-zero bins once.  Most keys of a read set share a few small
+// counts, so the lanes of a warp that fall into one bin add together (one shared atomic per distinct bin).  A thread
+// loads kHistUnroll slots before it counts any, to keep enough loads in flight for a pass bound by HBM.
+constexpr int kHistUnroll = 4;
+
+template <typename Key>
+__global__ void __launch_bounds__(256) table_histogram_kernel(const Key *__restrict__ keys, const uint32_t *__restrict__ vals,
+                                                              uint64_t n_slots, unsigned long long *hist, uint32_t n_bins)
+{
+    extern __shared__ uint32_t s_bins[];
+    for (uint32_t b = threadIdx.x; b < n_bins; b += blockDim.x) s_bins[b] = 0;
+    __syncthreads();
+    const uint64_t step = static_cast<uint64_t>(gridDim.x) * blockDim.x * kHistUnroll;
+    for (uint64_t base = static_cast<uint64_t>(blockIdx.x) * blockDim.x * kHistUnroll + threadIdx.x; base < n_slots; base += step) {
+        uint32_t bin[kHistUnroll];
+#pragma unroll
+        for (int u = 0; u < kHistUnroll; ++u) {
+            const uint64_t i = base + static_cast<uint64_t>(u) * blockDim.x;
+            const bool inside = i < n_slots;
+            const Key key = inside ? keys[i] : Key{};
+            const uint32_t val = inside ? vals[i] : 0u;
+            bin[u] = inside && !key_free(key) ? min(val, n_bins - 1) : ~0u; // ~0: no key
+        }
+        const uint32_t active = __activemask();
+#pragma unroll
+        for (int u = 0; u < kHistUnroll; ++u) {
+            const uint32_t peers = __match_any_sync(active, bin[u]);
+            if (bin[u] != ~0u && (threadIdx.x & 31) == static_cast<unsigned>(__ffs(peers) - 1)) atomicAdd(s_bins + bin[u], __popc(peers));
+        }
+    }
+    __syncthreads();
+    for (uint32_t b = threadIdx.x; b < n_bins; b += blockDim.x)
+        if (s_bins[b]) atomicAdd(hist + b, static_cast<unsigned long long>(s_bins[b]));
 }
 
 } // namespace
@@ -599,14 +706,16 @@ static int32_t kmer_table_merge(kmc_ctx *ctx, uint64_t *keys, uint32_t *vals, ui
     return st;
 }
 
-template <int NL>
+// RANGE: kmc_kmer_table(2)_export_range, the entries whose count lies in [min_count, max_count]
+template <int NL, bool RANGE = false>
 static int32_t kmer_table_export(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity, uint64_t *out_keys,
-                                 uint32_t *out_vals, uint64_t capacity, uint64_t *n_out)
+                                 uint32_t *out_vals, uint64_t capacity, uint64_t *n_out, uint32_t min_count = 0, uint32_t max_count = ~0u)
 {
     using Key = TableKey<NL>;
     if (!ctx) return KMC_E_BAD_ARG;
     if (!keys || !vals || !n_out || (capacity && (!out_keys || !out_vals))) return fail(ctx, KMC_E_BAD_ARG, "NULL buffer");
     if (log2_capacity < 1 || log2_capacity > 40) return fail(ctx, KMC_E_BAD_ARG, "log2_capacity must be in 1..40");
+    if (min_count > max_count) return fail(ctx, KMC_E_BAD_ARG, "min_count is larger than max_count");
     CU(cudaSetDevice(ctx->device));
     int32_t st = ensure_scratch(ctx, 1024);
     if (st) return st;
@@ -617,9 +726,9 @@ static int32_t kmer_table_export(kmc_ctx *ctx, const uint64_t *keys, const uint3
     CU(cudaMemsetAsync(cursor, 0, 8, stream));
     const uint64_t n_slots = 1ull << log2_capacity;
     const uint64_t blocks = std::min<uint64_t>((n_slots + 255) / 256, static_cast<uint64_t>(ctx->sm_count) * 16);
-    table_export_kernel<Key><<<static_cast<unsigned>(blocks), 256, 0, stream>>>(reinterpret_cast<const Key *>(keys), vals, n_slots,
-                                                                                 reinterpret_cast<Key *>(out_keys), out_vals, capacity,
-                                                                                 cursor);
+    table_export_kernel<Key, RANGE><<<static_cast<unsigned>(blocks), 256, 0, stream>>>(
+        reinterpret_cast<const Key *>(keys), vals, n_slots, reinterpret_cast<Key *>(out_keys), out_vals, capacity, cursor, min_count,
+        max_count);
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(&ctx->host_small[100], cursor, 8, cudaMemcpyDeviceToHost, stream));
     CU(cudaStreamSynchronize(stream));
@@ -628,31 +737,204 @@ static int32_t kmer_table_export(kmc_ctx *ctx, const uint64_t *keys, const uint3
     return KMC_OK;
 }
 
-extern "C" int32_t kmc_kmer_count(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t mode, uint64_t *keys, uint32_t *vals,
+// The checks a count into a table of NL limbs and a lookup in it share, past their NULL checks: 16-byte aligned
+// two-limb keys, the mode, a 2-bit source and a K of the table's width
+template <int NL>
+static int32_t check_table_kmers(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t mode, const uint64_t *keys)
+{
+    if (NL == 2 && reinterpret_cast<uintptr_t>(keys) % 16) return fail(ctx, KMC_E_BAD_ARG, "the two-limb keys must be 16-byte aligned");
+    if (mode != KMC_FW && mode != KMC_CANON) return fail(ctx, KMC_E_BAD_ARG, "mode must be KMC_FW or KMC_CANON");
+    if (seqs->src_bits != 2) return fail(ctx, KMC_E_UNSUPPORTED, "the k-mer table needs a 2-bit source");
+    if (NL == 1 && (k > 32 || (k == 32 && mode == KMC_FW)))
+        return fail(ctx, KMC_E_UNSUPPORTED, "the k-mer table supports K <= 31, and K = 32 for canonical k-mers");
+    if (NL == 2 && (k < 33 || k > 64 || (k == 64 && mode == KMC_FW)))
+        return fail(ctx, KMC_E_UNSUPPORTED, "the two-limb k-mer table supports K = 33..63, and K = 64 for canonical k-mers");
+    return KMC_OK;
+}
+
+template <int NL>
+static int32_t kmer_count_checked(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t mode, uint64_t *keys, uint32_t *vals,
                                   uint32_t log2_capacity, kmc_result *result)
 {
     int32_t st = check_common(ctx, seqs, k);
     if (st) return st;
     if (!keys || !vals || !result) return fail(ctx, KMC_E_BAD_ARG, "keys / vals / result is NULL");
-    if (mode != KMC_FW && mode != KMC_CANON) return fail(ctx, KMC_E_BAD_ARG, "mode must be KMC_FW or KMC_CANON");
-    if (seqs->src_bits != 2) return fail(ctx, KMC_E_UNSUPPORTED, "the k-mer table needs a 2-bit source");
-    if (k > 32 || (k == 32 && mode == KMC_FW))
-        return fail(ctx, KMC_E_UNSUPPORTED, "the k-mer table supports K <= 31, and K = 32 for canonical k-mers");
-    return kmer_count<1>(ctx, seqs, k, mode, keys, vals, log2_capacity, result);
+    st = check_table_kmers<NL>(ctx, seqs, k, mode, keys);
+    if (st) return st;
+    return kmer_count<NL>(ctx, seqs, k, mode, keys, vals, log2_capacity, result);
+}
+
+extern "C" int32_t kmc_kmer_count(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t mode, uint64_t *keys, uint32_t *vals,
+                                  uint32_t log2_capacity, kmc_result *result)
+{
+    return kmer_count_checked<1>(ctx, seqs, k, mode, keys, vals, log2_capacity, result);
 }
 
 extern "C" int32_t kmc_kmer_count2(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t mode, uint64_t *keys, uint32_t *vals,
                                    uint32_t log2_capacity, kmc_result *result)
 {
+    return kmer_count_checked<2>(ctx, seqs, k, mode, keys, vals, log2_capacity, result);
+}
+
+// kmc_kmer_lookup (NL = 1) and kmc_kmer_lookup2 (NL = 2): the count of every window, direct probes at any table size
+template <int NL>
+static int32_t kmer_lookup(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t mode, const uint64_t *keys, const uint32_t *vals,
+                           uint32_t log2_capacity, uint32_t *out_counts, uint64_t capacity, kmc_result *result)
+{
     int32_t st = check_common(ctx, seqs, k);
     if (st) return st;
-    if (!keys || !vals || !result) return fail(ctx, KMC_E_BAD_ARG, "keys / vals / result is NULL");
-    if (reinterpret_cast<uintptr_t>(keys) % 16) return fail(ctx, KMC_E_BAD_ARG, "the two-limb keys must be 16-byte aligned");
-    if (mode != KMC_FW && mode != KMC_CANON) return fail(ctx, KMC_E_BAD_ARG, "mode must be KMC_FW or KMC_CANON");
-    if (seqs->src_bits != 2) return fail(ctx, KMC_E_UNSUPPORTED, "the k-mer table needs a 2-bit source");
-    if (k < 33 || k > 64 || (k == 64 && mode == KMC_FW))
-        return fail(ctx, KMC_E_UNSUPPORTED, "the two-limb k-mer table supports K = 33..63, and K = 64 for canonical k-mers");
-    return kmer_count<2>(ctx, seqs, k, mode, keys, vals, log2_capacity, result);
+    if (!keys || !vals || !out_counts || !result) return fail(ctx, KMC_E_BAD_ARG, "keys / vals / out_counts / result is NULL");
+    st = check_table_kmers<NL>(ctx, seqs, k, mode, keys);
+    if (st) return st;
+    if (log2_capacity < 1 || log2_capacity > 40) return fail(ctx, KMC_E_BAD_ARG, "log2_capacity must be in 1..40");
+    CU(cudaSetDevice(ctx->device));
+    memset(result, 0, sizeof *result);
+    const Geometry ge = geometry(k);
+    if (ge.n_limbs != NL) return fail(ctx, KMC_E_UNSUPPORTED, "no kernel for this K");
+    cudaStream_t stream = ctx->stream;
+    CU(cudaEventRecord(ctx->ev_k0, stream));
+    st = ensure_scratch(ctx, layout_scratch_bytes(seqs) + 256);
+    if (st) return st;
+    Scratch scratch{static_cast<char *>(ctx->scratch), ctx->scratch_bytes, 0};
+    Layout L;
+    st = plan_layout(ctx, seqs, k, ge, stream, KnownTotals(), scratch, &L);
+    if (st) return st;
+    result->n_written = L.total;
+    if (capacity < L.total) return fail(ctx, KMC_E_OUT_TOO_SMALL, "out_counts capacity smaller than the number of windows");
+    if (L.total == 0) return KMC_OK;
+    ExtractParams p = base_params(seqs, k, ge, L, 0);
+    p.vec_ok = reinterpret_cast<uintptr_t>(out_counts) % (4u * ge.g) == 0;
+    ConsumeParams c{};
+    c.table = const_cast<uint32_t *>(vals); // read only: OP_LOOKUP* never writes the table
+    if constexpr (NL == 1)
+        c.keys = reinterpret_cast<unsigned long long *>(const_cast<uint64_t *>(keys));
+    else
+        c.keys2 = reinterpret_cast<ulonglong2 *>(const_cast<uint64_t *>(keys));
+    c.log2cap = log2_capacity;
+    c.out_counts = out_counts;
+    ConsumeLaunchFn fn = pick_consume_nx<NL, NL == 1 ? OP_LOOKUP : OP_LOOKUP2>(ge.nx, !L.uniform_len, mode == KMC_CANON);
+    if (!fn) return fail(ctx, KMC_E_UNSUPPORTED, "no kernel for this K");
+    CU(fn(p, c, stream));
+    CU(cudaEventRecord(ctx->ev_k1, stream));
+    CU(cudaStreamSynchronize(stream));
+    CU(cudaEventElapsedTime(&result->kernel_ms, ctx->ev_k0, ctx->ev_k1));
+    return KMC_OK;
+}
+
+// the argument checks every read-only query of a table shares
+template <int NL>
+static int32_t check_table_query(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity)
+{
+    if (!ctx) return KMC_E_BAD_ARG;
+    if (!keys || !vals) return fail(ctx, KMC_E_BAD_ARG, "NULL table");
+    if (log2_capacity < 1 || log2_capacity > 40) return fail(ctx, KMC_E_BAD_ARG, "log2_capacity must be in 1..40");
+    if (NL == 2 && reinterpret_cast<uintptr_t>(keys) % 16) return fail(ctx, KMC_E_BAD_ARG, "the two-limb keys must be 16-byte aligned");
+    return KMC_OK;
+}
+
+template <int NL>
+static int32_t kmer_table_get(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity, const uint64_t *query,
+                              uint64_t n, uint32_t *out_counts)
+{
+    using Key = TableKey<NL>;
+    int32_t st = check_table_query<NL>(ctx, keys, vals, log2_capacity);
+    if (st) return st;
+    if (n && (!query || !out_counts)) return fail(ctx, KMC_E_BAD_ARG, "query / out_counts is NULL");
+    if (NL == 2 && reinterpret_cast<uintptr_t>(query) % 16) return fail(ctx, KMC_E_BAD_ARG, "the two-limb keys must be 16-byte aligned");
+    if (n == 0) return KMC_OK;
+    CU(cudaSetDevice(ctx->device));
+    cudaStream_t stream = ctx->stream;
+    const uint64_t blocks = std::min<uint64_t>((n + 255) / 256, static_cast<uint64_t>(ctx->sm_count) * 16);
+    table_get_kernel<Key><<<static_cast<unsigned>(blocks), 256, 0, stream>>>(reinterpret_cast<const Key *>(keys), vals, log2_capacity,
+                                                                              reinterpret_cast<const Key *>(query), n, out_counts);
+    CU(cudaGetLastError());
+    CU(cudaStreamSynchronize(stream));
+    return KMC_OK;
+}
+
+constexpr uint32_t kMaxHistBins = 16384; // 64 KB of shared counters per block
+
+template <int NL>
+static int32_t kmer_table_histogram(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity, uint64_t *hist,
+                                    uint32_t n_bins)
+{
+    using Key = TableKey<NL>;
+    int32_t st = check_table_query<NL>(ctx, keys, vals, log2_capacity);
+    if (st) return st;
+    if (!hist) return fail(ctx, KMC_E_BAD_ARG, "hist is NULL");
+    if (n_bins < 1 || n_bins > kMaxHistBins) return fail(ctx, KMC_E_BAD_ARG, "n_bins must be in 1..16384");
+    CU(cudaSetDevice(ctx->device));
+    cudaStream_t stream = ctx->stream;
+    const size_t smem = 4ull * n_bins;
+    CU(cudaFuncSetAttribute(table_histogram_kernel<Key>, cudaFuncAttributeMaxDynamicSharedMemorySize, 4 * kMaxHistBins));
+    const uint64_t n_slots = 1ull << log2_capacity;
+    const uint64_t blocks = std::min<uint64_t>((n_slots + 256 * kHistUnroll - 1) / (256 * kHistUnroll), static_cast<uint64_t>(ctx->sm_count) * 8);
+    table_histogram_kernel<Key><<<static_cast<unsigned>(blocks), 256, smem, stream>>>(
+        reinterpret_cast<const Key *>(keys), vals, n_slots, reinterpret_cast<unsigned long long *>(hist), n_bins);
+    CU(cudaGetLastError());
+    CU(cudaStreamSynchronize(stream));
+    return KMC_OK;
+}
+
+template <int NL>
+static int32_t kmer_table_export_range(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
+                                       uint32_t min_count, uint32_t max_count, uint64_t *out_keys, uint32_t *out_vals, uint64_t capacity,
+                                       uint64_t *n_out)
+{
+    if (ctx && NL == 2 && (reinterpret_cast<uintptr_t>(keys) % 16 || reinterpret_cast<uintptr_t>(out_keys) % 16))
+        return fail(ctx, KMC_E_BAD_ARG, "the two-limb keys must be 16-byte aligned");
+    return kmer_table_export<NL, true>(ctx, keys, vals, log2_capacity, out_keys, out_vals, capacity, n_out, min_count, max_count);
+}
+
+extern "C" int32_t kmc_kmer_lookup(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t mode, const uint64_t *keys, const uint32_t *vals,
+                                   uint32_t log2_capacity, uint32_t *out_counts, uint64_t capacity, kmc_result *result)
+{
+    return kmer_lookup<1>(ctx, seqs, k, mode, keys, vals, log2_capacity, out_counts, capacity, result);
+}
+
+extern "C" int32_t kmc_kmer_lookup2(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t mode, const uint64_t *keys,
+                                    const uint32_t *vals, uint32_t log2_capacity, uint32_t *out_counts, uint64_t capacity,
+                                    kmc_result *result)
+{
+    return kmer_lookup<2>(ctx, seqs, k, mode, keys, vals, log2_capacity, out_counts, capacity, result);
+}
+
+extern "C" int32_t kmc_kmer_table_get(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
+                                      const uint64_t *query, uint64_t n, uint32_t *out_counts)
+{
+    return kmer_table_get<1>(ctx, keys, vals, log2_capacity, query, n, out_counts);
+}
+
+extern "C" int32_t kmc_kmer_table2_get(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
+                                       const uint64_t *query, uint64_t n, uint32_t *out_counts)
+{
+    return kmer_table_get<2>(ctx, keys, vals, log2_capacity, query, n, out_counts);
+}
+
+extern "C" int32_t kmc_kmer_table_histogram(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
+                                            uint64_t *hist, uint32_t n_bins)
+{
+    return kmer_table_histogram<1>(ctx, keys, vals, log2_capacity, hist, n_bins);
+}
+
+extern "C" int32_t kmc_kmer_table2_histogram(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
+                                             uint64_t *hist, uint32_t n_bins)
+{
+    return kmer_table_histogram<2>(ctx, keys, vals, log2_capacity, hist, n_bins);
+}
+
+extern "C" int32_t kmc_kmer_table_export_range(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
+                                               uint32_t min_count, uint32_t max_count, uint64_t *out_keys, uint32_t *out_vals,
+                                               uint64_t capacity, uint64_t *n_out)
+{
+    return kmer_table_export_range<1>(ctx, keys, vals, log2_capacity, min_count, max_count, out_keys, out_vals, capacity, n_out);
+}
+
+extern "C" int32_t kmc_kmer_table2_export_range(kmc_ctx *ctx, const uint64_t *keys, const uint32_t *vals, uint32_t log2_capacity,
+                                                uint32_t min_count, uint32_t max_count, uint64_t *out_keys, uint32_t *out_vals,
+                                                uint64_t capacity, uint64_t *n_out)
+{
+    return kmer_table_export_range<2>(ctx, keys, vals, log2_capacity, min_count, max_count, out_keys, out_vals, capacity, n_out);
 }
 
 extern "C" int32_t kmc_kmer_table_merge(kmc_ctx *ctx, uint64_t *keys, uint32_t *vals, uint32_t log2_capacity,

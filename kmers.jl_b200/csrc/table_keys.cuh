@@ -17,6 +17,8 @@ constexpr uint64_t kEmptyKey = ~0ull;
 
 __host__ __device__ __forceinline__ bool key_free(uint64_t k) { return k == kEmptyKey; }
 __host__ __device__ __forceinline__ bool key_free(ulonglong2 k) { return k.x == kEmptyKey && k.y == kEmptyKey; }
+__host__ __device__ __forceinline__ bool key_equal(uint64_t a, uint64_t b) { return a == b; }
+__host__ __device__ __forceinline__ bool key_equal(ulonglong2 a, ulonglong2 b) { return a.x == b.x && a.y == b.y; }
 
 // fx_hash(k-mer, 0) (src/kmer.jl:255-261): its top bits pick the table slot (and the bin of the binned insert), a
 // second mix of it the owner rank of the multi-GPU exchange (comm.cu)

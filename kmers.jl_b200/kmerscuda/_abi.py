@@ -119,7 +119,19 @@ SIGNATURES = {
                                           C.POINTER(C.c_uint64)]),
     "kmc_kmer_table2_export": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint64,
                                            C.POINTER(C.c_uint64)]),
-    "kmc_nccl_version": (C.c_int32, [C.POINTER(C.c_int32)]),
+    "kmc_kmer_lookup": (C.c_int32, [C.c_void_p, C.POINTER(kmc_seqs), C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_uint32,
+                                    C.c_void_p, C.c_uint64, C.POINTER(kmc_result)]),
+    "kmc_kmer_lookup2": (C.c_int32, [C.c_void_p, C.POINTER(kmc_seqs), C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_uint32,
+                                     C.c_void_p, C.c_uint64, C.POINTER(kmc_result)]),
+    "kmc_kmer_table_get": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint64, C.c_void_p]),
+    "kmc_kmer_table2_get": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint64, C.c_void_p]),
+    "kmc_kmer_table_histogram": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32]),
+    "kmc_kmer_table2_histogram": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32]),
+    "kmc_kmer_table_export_range": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p,
+                                                C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]),
+    "kmc_kmer_table2_export_range": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p,
+                                                 C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]),
+    "kmc_nccl_version":(C.c_int32, [C.POINTER(C.c_int32)]),
     "kmc_comm_unique_id": (C.c_int32, [C.c_void_p]),
     "kmc_comm_init_rank": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]),
     "kmc_comm_destroy": (C.c_int32, [C.c_void_p]),

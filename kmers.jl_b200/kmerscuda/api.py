@@ -782,7 +782,8 @@ class KmerTable:
     def _fn(self, name: str):
         """The entry point `name` of this table's key width (kmc_kmer_count -> kmc_kmer_count2, ...)."""
         if self.n_limbs == 2:
-            name = name.replace("kmc_kmer_table_", "kmc_kmer_table2_").replace("kmc_kmer_count", "kmc_kmer_count2")
+            name = (name.replace("kmc_kmer_table_", "kmc_kmer_table2_").replace("kmc_kmer_count", "kmc_kmer_count2")
+                    .replace("kmc_kmer_lookup", "kmc_kmer_lookup2"))
         return getattr(self.ctx.lib, name)
 
     def _same_width(self, other: "KmerTable"):
@@ -818,15 +819,64 @@ class KmerTable:
         owned.n_keys = int(n_owned.value)
         return owned
 
-    def items(self):
+    def lookup(self, rs, K: int, *, canonical: bool = True, device_out: bool = False):
+        """The count of every window of the set (kmc_kmer_lookup): u32[windows] in `extract` order, so element i is the
+        count of extract(...).kmers[i] (0 for a k-mer the table does not hold).  Look up with the mode the table was
+        counted with.  device_out=True leaves the counts on the device and returns their DeviceBuffer."""
+        _check_K(K)
+        drs = rs if isinstance(rs, DeviceReadSet) else DeviceReadSet(self.ctx, rs)
+        n = int(drs.host.window_counts(K).sum())
+        out = self.ctx.alloc(4 * max(n, 1))
+        res = kmc_result()
+        self.ctx._check(self._fn("kmc_kmer_lookup")(self.ctx.handle, C.byref(drs.desc), K, KMC_CANON if canonical else KMC_FW,
+                                                    self.keys.ptr, self.vals.ptr, self.log2_capacity, out.ptr, n, C.byref(res)))
+        if device_out:
+            return out
+        counts = out.download(np.uint32, n)
+        out.free()
+        return counts
+
+    def get(self, keys: np.ndarray) -> np.ndarray:
+        """table[key] for every key (kmc_kmer_table_get): keys u64[n] for one limb, u64[n, 2] for two; u32[n], 0 for a key
+        that is not in the table."""
+        keys = np.ascontiguousarray(keys, dtype=np.uint64)
+        if keys.ndim != self.n_limbs or (self.n_limbs == 2 and keys.shape[1] != 2):
+            raise ValueError(f"a table of {self.n_limbs} limbs takes keys of shape {'(n,)' if self.n_limbs == 1 else '(n, 2)'}")
+        n = keys.shape[0]
+        dq, dout = self.ctx.to_device(keys), self.ctx.alloc(4 * max(n, 1))
+        self.ctx._check(self._fn("kmc_kmer_table_get")(self.ctx.handle, self.keys.ptr, self.vals.ptr, self.log2_capacity, dq.ptr, n,
+                                                       dout.ptr))
+        counts = dout.download(np.uint32, n)
+        dq.free()
+        dout.free()
+        return counts
+
+    def histogram(self, n_bins: int = 256) -> np.ndarray:
+        """The count spectrum (kmc_kmer_table_histogram): u64[n_bins], bin c = keys with count c, the last bin every
+        count of n_bins - 1 and more."""
+        h = self.ctx.alloc(8 * n_bins)
+        self.ctx._check(self.ctx.lib.kmc_memset(self.ctx.handle, h.ptr, 0, 8 * n_bins))
+        self.ctx._check(self._fn("kmc_kmer_table_histogram")(self.ctx.handle, self.keys.ptr, self.vals.ptr, self.log2_capacity,
+                                                             h.ptr, n_bins))
+        out = h.download(np.uint64, n_bins)
+        h.free()
+        return out
+
+    def items(self, min_count: Optional[int] = None, max_count: Optional[int] = None):
         """(keys, counts u32[n]) sorted by key: keys u64[n] for one limb; u64[n, 2] (limb 0 = head first) in Kmer order,
-        lexicographic on (limb 0, limb 1), for two."""
+        lexicographic on (limb 0, limb 1), for two.  With min_count / max_count only the keys whose count lies in
+        [min_count, max_count] (kmc_kmer_table_export_range; the solid k-mers)."""
         n = max(self.n_keys, 1)
         L = self.n_limbs
         dk, dv = self.ctx.alloc(8 * L * n), self.ctx.alloc(4 * n)
         n_out = C.c_uint64(0)
-        self.ctx._check(self._fn("kmc_kmer_table_export")(self.ctx.handle, self.keys.ptr, self.vals.ptr, self.log2_capacity,
-                                                          dk.ptr, dv.ptr, n, C.byref(n_out)))
+        if min_count is None and max_count is None:
+            self.ctx._check(self._fn("kmc_kmer_table_export")(self.ctx.handle, self.keys.ptr, self.vals.ptr, self.log2_capacity,
+                                                              dk.ptr, dv.ptr, n, C.byref(n_out)))
+        else:
+            lo, hi = 0 if min_count is None else int(min_count), 2**32 - 1 if max_count is None else int(max_count)
+            self.ctx._check(self._fn("kmc_kmer_table_export_range")(self.ctx.handle, self.keys.ptr, self.vals.ptr,
+                                                                    self.log2_capacity, lo, hi, dk.ptr, dv.ptr, n, C.byref(n_out)))
         m = int(n_out.value)
         k, v = dk.download(np.uint64, L * m), dv.download(np.uint32, m)
         dk.free()
