@@ -236,6 +236,30 @@ int32_t kmc_minimizers(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t w,
 int32_t kmc_minhash_sketch(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t mode, uint64_t s,
                            uint64_t *out_hashes, kmc_result *result);
 
+/* The bottom-s sketch of every sequence of the set on its own: row i of out_hashes (device u64[n_seqs][s]) holds,
+ * ascending, exactly what kmc_minhash_sketch returns for a set made of sequence i alone; out_n[i] (device u32[n_seqs])
+ * is its length: min(s, distinct k-mers of sequence i), 0 for a sequence shorter than K.  Slots past out_n[i] are ~0.
+ * KMC_FW / KMC_CANON, 2-bit sources, K <= 64, single sequences, uniform and ragged sets, first_symbol_offset views.
+ * result->n_written = sum of out_n; result->kernel_ms as for the other consumers; result->digest[0] = rounds run past
+ * the first, result->digest[1] = sequences those rounds sketched again (sequences whose repeats left fewer than s
+ * distinct k-mers below their first hash limit).  s < 1, n_seqs * s * 8 overflowing u64, a mode other than KMC_FW /
+ * KMC_CANON and NULL pointers are KMC_E_BAD_ARG; K > 64 and other sources are KMC_E_UNSUPPORTED; n_seqs = 0 writes
+ * nothing.  Temporary memory: 32 bytes per sequence and 16 bytes per candidate (about s + 4 sqrt(s) + 16 per long
+ * sequence, every window of a sequence of fewer than about 2s + 8 sqrt(s) + 32 windows) plus the sort's scratch. */
+int32_t kmc_minhash_sketch_each(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t mode, uint64_t s,
+                                uint64_t *out_hashes, uint32_t *out_n, kmc_result *result);
+
+/* Every sketch of list A against every sketch of list B (device rows of s u64, ascending and distinct, lengths a_n /
+ * b_n; a length above s is read as s; A and B may be the same arrays).  For pair (i, j), at i * n_b + j (device u32):
+ *   shared[]        = |A_i ∩ B_j|
+ *   shared_bottom[] = |S_s(A_i ∪ B_j) ∩ A_i ∩ B_j|, S_s = the s smallest values   (Mash's estimator numerator)
+ * so the Mash Jaccard estimate is shared_bottom / min(s, n_A + n_B - shared).  Either output may be NULL.  s in
+ * 1..16384 (KMC_E_UNSUPPORTED above, KMC_E_BAD_ARG for 0); n_a = 0 or n_b = 0 does nothing.  No row is read past its
+ * length, whatever the rows contain.  Synchronises. */
+int32_t kmc_minhash_compare(kmc_ctx *ctx, const uint64_t *a, const uint32_t *a_n, uint64_t n_a,
+                            const uint64_t *b, const uint32_t *b_n, uint64_t n_b, uint64_t s,
+                            uint32_t *shared, uint32_t *shared_bottom);
+
 /* k-mer composition vector: table[as_integer(kmer)] += 1 for every k-mer of the set
  * (docs/src/composition.md:28-39 counts FwDNAMers{4}; as_integer: src/kmer.jl:305-326), forward
  * (KMC_FW) or canonical (KMC_CANON) k-mers, K <= 14.  table: device u32[4^K], caller-zeroed

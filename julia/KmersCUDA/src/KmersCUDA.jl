@@ -31,7 +31,7 @@ using Kmers
 using Kmers: FwKmers, FwRvIterator, CanonicalKmers, UnambiguousKmers, SpacedKmers, Kmer, derive_type
 using Libdl
 
-export fx_hash_device, hash_device, extract, set_library!, minhash_sketch, composition, minimizers, count_kmers,
+export fx_hash_device, hash_device, extract, set_library!, minhash_sketch, minhash_sketches, minhash_compare, composition, minimizers, count_kmers,
     bucket_count, DeviceVector, Group, free!, KmerCountTable, counts, spectrum
 
 # ---------------------------------------------------------------------------------------------
@@ -648,6 +648,61 @@ function minhash_sketch(it::Union{FwKmers{A, K}, CanonicalKmers{A, K}}, s::Integ
     free!(dout)
     return out
 end
+
+"""
+    minhash_sketches(seqs::AbstractVector{<:LongSequence}, K, s; canonical = true) -> Vector{Vector{UInt64}}
+
+The bottom-`s` sketch of every sequence on its own, in one call (`kmc_minhash_sketch_each`): element `i` is what
+`minhash_sketch(CanonicalKmers{A,K}(seqs[i]), s)` returns (`FwKmers` with `canonical = false`).
+"""
+function minhash_sketches(seqs::AbstractVector{S}, K::Integer, s::Integer; canonical::Bool = true,
+        ctx::Context = default_context()) where {S <: LongSequence{<:NucleicAcidAlphabet{2}}}
+    n = length(seqs)
+    n == 0 && return Vector{UInt64}[]
+    pk = pack_reads(seqs)
+    dw, doff, dlen = upload(ctx, pk.words), upload(ctx, pk.woff), upload(ctx, pk.lens)
+    drows = DeviceVector{UInt64}(ctx, n * s)
+    dn = DeviceVector{UInt32}(ctx, n)
+    res = KmcResult()
+    d = Ref(KmcSeqs(dw.ptr, length(pk.words), n, doff.ptr, dlen.ptr, 0, 0, UInt32(2), 0))
+    st = ccall((:kmc_minhash_sketch_each, LIB[]), Int32,
+        (Ptr{Cvoid}, Ptr{KmcSeqs}, Int32, Int32, UInt64, Ptr{Cvoid}, Ptr{Cvoid}, Ref{KmcResult}),
+        ctx.handle, d, K, canonical ? KMC_CANON : KMC_FW, s, drows.ptr, dn.ptr, res)
+    st == KMC_OK || throw_status(ctx, st, res, eltype(S))
+    rows, lens = reshape(Array(drows), Int(s), n), Array(dn)
+    foreach(free!, (dw, doff, dlen, drows, dn))
+    return [rows[1:lens[i], i] for i in 1:n]
+end
+
+"""
+    minhash_compare(a::Vector{Vector{UInt64}}, b = a, s) -> (shared::Matrix{UInt32}, shared_bottom::Matrix{UInt32})
+
+Every sketch of `a` against every sketch of `b` (`kmc_minhash_compare`): `shared[i, j] = |a[i] ∩ b[j]|` and
+`shared_bottom[i, j]` = how many of those are among the `s` smallest values of `a[i] ∪ b[j]`.  The Mash Jaccard
+estimate is `shared_bottom / min(s, length(a[i]) + length(b[j]) - shared)`; sketches are ascending and distinct, as
+`minhash_sketches` returns them, and are read up to `s` values.
+"""
+function minhash_compare(a::AbstractVector{<:AbstractVector{UInt64}}, b::AbstractVector{<:AbstractVector{UInt64}}, s::Integer;
+        ctx::Context = default_context())
+    na, nb = length(a), length(b)
+    (na == 0 || nb == 0) && return (zeros(UInt32, na, nb), zeros(UInt32, na, nb))
+    pack(v) = (m = fill(typemax(UInt64), Int(s), length(v));
+               for (i, x) in enumerate(v); k = min(length(x), s); m[1:k, i] .= x[1:k]; end;
+               (vec(m), UInt32[min(length(x), s) for x in v]))
+    ra, la = pack(a)
+    rb, lb = pack(b)
+    da, dla, db, dlb = upload(ctx, ra), upload(ctx, la), upload(ctx, rb), upload(ctx, lb)
+    dsh, dbt = DeviceVector{UInt32}(ctx, na * nb), DeviceVector{UInt32}(ctx, na * nb)
+    check(ctx, ccall((:kmc_minhash_compare, LIB[]), Int32,
+        (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, UInt64, Ptr{Cvoid}, Ptr{Cvoid}, UInt64, UInt64, Ptr{Cvoid}, Ptr{Cvoid}),
+        ctx.handle, da.ptr, dla.ptr, na, db.ptr, dlb.ptr, nb, s, dsh.ptr, dbt.ptr))
+    # the library writes pair (i, j) at i * nb + j: row-major, so the column-major result is transposed
+    shared = permutedims(reshape(Array(dsh), nb, na))
+    bottom = permutedims(reshape(Array(dbt), nb, na))
+    foreach(free!, (da, dla, db, dlb, dsh, dbt))
+    return shared, bottom
+end
+minhash_compare(a::AbstractVector{<:AbstractVector{UInt64}}, s::Integer; kw...) = minhash_compare(a, a, s; kw...)
 
 """
     composition(FwKmers{A,K}(seq) | CanonicalKmers{A,K}(seq)) -> Vector{UInt32}  (length 4^K, K <= 14)

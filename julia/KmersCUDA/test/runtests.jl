@@ -135,3 +135,21 @@ end
     @test_throws BioSequences.EncodeError KmersCUDA.collect(SpacedDNAMers{3, 4}("TAGAWWWW"))
     @test KmersCUDA.collect(each_codon(DNA, "TGACGATCGAC")) == collect(each_codon(DNA, "TGACGATCGAC"))
 end
+
+@testset "minhash_sketches == minhash_sketch per sequence; minhash_compare == set definitions" begin
+    seqs = [LongDNA{2}(randdnaseq(RNG, len)) for len in (0, 10, 20, 21, 500, 5_000, 50_000)]
+    for canonical in (true, false), s in (1, 10, 1000)
+        rows = KmersCUDA.minhash_sketches(seqs, 21, s; canonical)
+        for (i, q) in enumerate(seqs)
+            it = canonical ? CanonicalDNAMers{21}(q) : FwDNAMers{21}(q)
+            @test rows[i] == KmersCUDA.minhash_sketch(it, s)
+            @test rows[i] == first(sort!(unique(fx_hash.(collect(it)))), s)
+        end
+        shared, bottom = KmersCUDA.minhash_compare(rows, s)
+        for i in eachindex(rows), j in eachindex(rows)
+            x, y = Set(rows[i]), Set(rows[j])
+            @test shared[i, j] == length(x ∩ y)
+            @test bottom[i, j] == length(Set(first(sort!(collect(x ∪ y)), s)) ∩ x ∩ y)
+        end
+    end
+end

@@ -91,6 +91,12 @@ template <int G, int BPS> struct AlignedLocator {
         uint32_t gi;
         return bit_of(item, gi);
     }
+    // the read that owns the item: the quotient bit_of computes
+    KMC_DEV uint32_t read_of(uint32_t item) const
+    {
+        const uint32_t r = __umulhi(item, magic);
+        return item - r * gprm >= gprm ? r + 1 : r;
+    }
 };
 
 // reversebits(x, BitsPerSymbol{2}) on a 32-bit word: reverse the order of the 16 two-bit groups.

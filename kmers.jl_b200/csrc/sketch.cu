@@ -4,6 +4,9 @@
 //                       `sketch(fx_hash, CanonicalDNAMers{16}(seq), 1000)` (docs/src/minhash.md:31-36;
 //                       MinHash.jl is not vendored: the published bottom-s definition is restated --
 //                       the s smallest DISTINCT hash values over all k-mers, ascending)
+//   kmc_minhash_sketch_each  the same sketch of every sequence of the set on its own, in one call (per-sequence hash
+//                       limits, candidates in per-sequence segments, cub's segmented sort; kmc_minhash_compare
+//                       compares the rows, compare.cu)
 //   kmc_composition     k-mer composition vector -- `counts[as_integer(kmer) + 1] += 1` over
 //                       FwDNAMers{K} (docs/src/composition.md:28-39), K <= 14
 //   kmc_kmer_count      exact k-mer counts keyed by the k-mer itself (the `Dict{Kmer,Int}` a user of the
@@ -28,6 +31,7 @@
 // array), and if duplicates left fewer than s distinct values the threshold moves up and (3)-(4)
 // repeat.  The k-mers are read twice (2 x 0.25 B/symbol) and nothing proportional to them is written.
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_segmented_sort.cuh>
 #include <cub/device/device_select.cuh>
 
 #include <algorithm>
@@ -49,7 +53,9 @@ enum : int {
     OP_TABLE = 4,
     OP_TABLE2 = 5,
     OP_LOOKUP = 6,
-    OP_LOOKUP2 = 7
+    OP_LOOKUP2 = 7,
+    OP_SKETCH_COUNT = 8,
+    OP_SKETCH_APPEND = 9
 };
 
 // kEmptyKey (table_keys.cuh) is never a k-mer: one limb, K <= 31, or K = 32 canonical (the all-T 32-mer is not
@@ -153,6 +159,9 @@ struct ConsumeParams {
     uint32_t *overflow;            // OP_TABLE*: set when a k-mer found no slot
     ulonglong2 *keys2;             // OP_TABLE2: two-limb keys, ulonglong2[2^log2cap] ({~0, ~0} = free), vals = table
     uint32_t *out_counts;          // OP_LOOKUP*: u32 per window, at its flat window index (kmc_extract's order)
+    const uint64_t *seq_lim;       // OP_SKETCH_*: per sequence, keep h < lim (~0: every k-mer; 0: skip the sequence)
+    unsigned long long *seq_cnt;   // OP_SKETCH_COUNT: candidates per sequence
+    unsigned long long *seq_cursor; // OP_SKETCH_APPEND: next free candidate slot of each sequence (starts at its offset)
 };
 
 constexpr int kSharedCompositionMax = 4096; // 4^6 counters = 16 KB of shared memory
@@ -169,6 +178,7 @@ __global__ void __launch_bounds__(kBlockThreads) consume_kernel(const ExtractPar
     __shared__ TileShared<RAGGED> sh;
     constexpr bool SHARED_HIST = (OP == OP_COMPOSITION_SHARED || OP == OP_HASH_HIST);
     constexpr bool LOOKUP = (OP == OP_LOOKUP || OP == OP_LOOKUP2);
+    constexpr bool SKETCH = (OP == OP_SKETCH_COUNT || OP == OP_SKETCH_APPEND);
     __shared__ uint32_t s_hist[SHARED_HIST ? kSharedCompositionMax : 1];
     const uint64_t tile_base = static_cast<uint64_t>(blockIdx.x) * kTileItems;
     if (SHARED_HIST) {
@@ -194,20 +204,33 @@ __global__ void __launch_bounds__(kBlockThreads) consume_kernel(const ExtractPar
         if (item >= p.items) break;
         int jlo, jhi;
         uint32_t x[NX];
+        uint64_t seq = 0, lim = 0; // OP_SKETCH_*: the item's sequence and its limit (0: skipped this round)
         if (ALIGNED) {
             jlo = 0;
             jhi = (p.al_tail != 0 && static_cast<uint32_t>(item) == n_items32 - 1u) ? static_cast<int>(p.al_tail) : G;
+            if constexpr (SKETCH) {
+                seq = items.read_of(static_cast<uint32_t>(item));
+                lim = __ldg(c.seq_lim + seq);
+                if (lim == 0) jhi = 0;
+            }
             load_block_at<NX>(p, items.bit_of(static_cast<uint32_t>(item)), inside, x);
         } else {
             cur.locate(p, item, li, sh);
             jlo = cur.jlo;
             jhi = cur.jhi;
+            if constexpr (SKETCH) {
+                seq = cur.r;
+                lim = __ldg(c.seq_lim + seq);
+                if (lim == 0) jhi = jlo;
+            }
             if (jhi > jlo) load_block<NX>(p.w32, p.nw32, cur.bit(p), x);
         }
         if (jhi > jlo) {
             uint64_t fw[G][N], rv[G][N];
             block_kmers<N, NX, G, true, CANON>(x, p.s0, p.head_mask, fw, rv);
             uint32_t found[LOOKUP ? G : 1]; // OP_LOOKUP*: the counts of the item's windows [jlo, jhi)
+            uint64_t hs[OP == OP_SKETCH_APPEND ? G : 1]; // OP_SKETCH_APPEND: the hashes of the windows
+            uint32_t take = 0;                            // OP_SKETCH_*: bit j = window j is a candidate
 #pragma unroll
             for (int j = 0; j < G; ++j) {
                 if (j < jlo || j >= jhi) continue;
@@ -222,6 +245,11 @@ __global__ void __launch_bounds__(kBlockThreads) consume_kernel(const ExtractPar
                 } else if constexpr (OP == OP_LOOKUP2) {
                     const ulonglong2 key = make_ulonglong2(a[0], a[N - 1]);
                     found[j] = table_find(c.keys2, c.table, c.log2cap, key, key_hash(key));
+                    continue;
+                } else if constexpr (SKETCH) {
+                    const uint64_t h = fx_hash<N>(a, 0);
+                    if (h < lim || lim == ~0ull) take |= 1u << j;
+                    if constexpr (OP == OP_SKETCH_APPEND) hs[j] = h;
                     continue;
                 }
                 if (OP == OP_HASH_HIST) {
@@ -245,6 +273,37 @@ __global__ void __launch_bounds__(kBlockThreads) consume_kernel(const ExtractPar
                     atomicAdd(c.table + a[N - 1], 1u); // as_integer(kmer): K <= 14, one limb
                 } else {
                     atomicAdd(s_hist + a[N - 1], 1u);
+                }
+            }
+            if constexpr (SKETCH) {
+                // The lanes of a warp that hold candidates of one sequence add them with one atomic: the counts (<= G)
+                // are summed bit by bit over the lanes of the same sequence (__match_any_sync), and the appending
+                // lanes write at their prefix from the base the first of them reserved.
+                const uint32_t active = __activemask();
+                if (__any_sync(active, take != 0)) {
+                    constexpr int kCountBits = G >= 8 ? 4 : G >= 4 ? 3 : G >= 2 ? 2 : 1;
+                    static_assert(G < 16, "a lane's candidate count fits kCountBits bits");
+                    const uint32_t lane = threadIdx.x & 31;
+                    const uint32_t peers = __match_any_sync(active, static_cast<unsigned long long>(seq));
+                    const int leader = __ffs(peers) - 1;
+                    const uint32_t n_take = __popc(take), lower = peers & ((1u << lane) - 1u);
+                    uint32_t total = 0, before = 0;
+#pragma unroll
+                    for (int b = 0; b < kCountBits; ++b) {
+                        const uint32_t m = __ballot_sync(active, (n_take >> b) & 1u) & peers;
+                        total += static_cast<uint32_t>(__popc(m)) << b;
+                        before += static_cast<uint32_t>(__popc(m & lower)) << b;
+                    }
+                    if constexpr (OP == OP_SKETCH_COUNT) {
+                        if (static_cast<int>(lane) == leader && total) atomicAdd(c.seq_cnt + seq, static_cast<unsigned long long>(total));
+                    } else {
+                        unsigned long long base = 0;
+                        if (static_cast<int>(lane) == leader && total) base = atomicAdd(c.seq_cursor + seq, static_cast<unsigned long long>(total));
+                        uint64_t at = __shfl_sync(active, base, leader) + before;
+#pragma unroll
+                        for (int j = 0; j < G; ++j)
+                            if ((take >> j) & 1u) c.cand[at++] = hs[j];
+                    }
                 }
             }
             if constexpr (LOOKUP) {
@@ -439,6 +498,70 @@ __global__ void __launch_bounds__(256) table_histogram_kernel(const Key *__restr
         if (s_bins[b]) atomicAdd(hist + b, static_cast<unsigned long long>(s_bins[b]));
 }
 
+// ---- a bottom-s sketch per sequence (kmc_minhash_sketch_each) ----------------------------------------------------
+// The first limit of each sequence: every k-mer when its windows are few against s, otherwise the hash below which
+// s + 4 sqrt(s) + 16 of its windows are expected (windows hash uniformly), so that distinct k-mers below it fall short of
+// s only when repeats remove that margin -- and the retry catches those.  No windows: an empty row, no candidates.
+__global__ void sketch_limits_kernel(const uint64_t *__restrict__ win_off, uint64_t wpr, uint64_t n, uint64_t s,
+                                     uint64_t *__restrict__ lim)
+{
+    for (uint64_t i = static_cast<uint64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < n;
+         i += static_cast<uint64_t>(gridDim.x) * blockDim.x) {
+        const uint64_t w = win_off ? win_off[i + 1] - win_off[i] : wpr;
+        const double want = static_cast<double>(s) + 4.0 * sqrt(static_cast<double>(s)) + 16.0;
+        const double frac = w ? want / static_cast<double>(w) : 1.0;
+        lim[i] = frac >= 0.5 ? ~0ull : static_cast<uint64_t>(frac * 18446744073709551616.0);
+    }
+}
+
+// the segment offsets of sequences [seg0, seg0 + nseg] relative to the first one, as the int offsets cub takes
+__global__ void segment_offsets_kernel(const uint64_t *__restrict__ off, uint64_t seg0, uint64_t nseg, int *__restrict__ out)
+{
+    const uint64_t base = off[seg0];
+    for (uint64_t i = static_cast<uint64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i <= nseg;
+         i += static_cast<uint64_t>(gridDim.x) * blockDim.x)
+        out[i] = static_cast<int>(off[seg0 + i] - base);
+}
+
+// One warp per sequence of the round (lim != 0): its sorted candidates [off[i], off[i+1]) give the first min(s, distinct)
+// distinct values to row i, the rest of the row is ~0 and out_n[i] its length.  A row that is final adds its length to
+// *n_total.  A row with fewer than s distinct candidates under a limit below ~0 may be missing values above the limit: its
+// limit becomes 4x (then ~0) and it is counted in *n_retry; every other sequence gets limit 0, which the next round skips.
+__global__ void __launch_bounds__(256) sketch_finish_kernel(const uint64_t *__restrict__ sorted, const uint64_t *__restrict__ off,
+                                                            uint64_t *__restrict__ lim, uint64_t n, uint64_t s, int round,
+                                                            uint64_t *__restrict__ out_hashes, uint32_t *__restrict__ out_n,
+                                                            unsigned long long *n_retry, unsigned long long *n_total)
+{
+    const uint32_t lane = threadIdx.x & 31;
+    const uint64_t warps = static_cast<uint64_t>(gridDim.x) * (blockDim.x / 32);
+    for (uint64_t i = (static_cast<uint64_t>(blockIdx.x) * blockDim.x + threadIdx.x) / 32; i < n; i += warps) {
+        const uint64_t l = lim[i];
+        if (l == 0) continue;
+        const uint64_t beg = off[i], end = off[i + 1];
+        uint64_t *row = out_hashes + i * s;
+        uint64_t distinct = 0;
+        for (uint64_t p0 = beg; p0 < end && distinct < s; p0 += 32) {
+            const uint64_t q = p0 + lane;
+            const bool in = q < end;
+            const uint64_t v = in ? sorted[q] : 0;
+            const bool keep = in && (q == beg || sorted[q - 1] != v);
+            const uint32_t m = __ballot_sync(0xffffffffu, keep);
+            const uint64_t rank = distinct + __popc(m & ((1u << lane) - 1u));
+            if (keep && rank < s) row[rank] = v;
+            distinct += __popc(m);
+        }
+        const uint64_t nd = distinct < s ? distinct : s;
+        for (uint64_t t = nd + lane; t < s; t += 32) row[t] = ~0ull;
+        if (lane == 0) {
+            out_n[i] = static_cast<uint32_t>(nd);
+            const bool retry = distinct < s && l != ~0ull;
+            lim[i] = retry ? (round == 0 && l < (1ull << 62) ? 4 * l : ~0ull) : 0;
+            if (retry) atomicAdd(n_retry, 1ull);
+            else atomicAdd(n_total, static_cast<unsigned long long>(nd));
+        }
+    }
+}
+
 } // namespace
 
 } // namespace kmc
@@ -537,6 +660,131 @@ extern "C" int32_t kmc_minhash_sketch(kmc_ctx *ctx, const kmc_seqs *seqs, int32_
         }
         want = cum + 2 * (s - distinct) + 1; // at least one more bucket
     }
+    CU(cudaEventRecord(ctx->ev_k1, stream));
+    CU(cudaStreamSynchronize(stream));
+    CU(cudaEventElapsedTime(&result->kernel_ms, ctx->ev_k0, ctx->ev_k1));
+    return KMC_OK;
+}
+
+// Every sequence's own sketch in one pass per round over the set (DESIGN.md 3.2d): per-sequence limits, a count pass
+// (OP_SKETCH_COUNT) and a scan give each sequence a segment of the candidate array, an append pass (OP_SKETCH_APPEND)
+// fills the segments, cub's segmented sort orders them and sketch_finish_kernel takes each row's distinct prefix.  Rows
+// whose repeats left fewer than s distinct candidates go round again with a higher limit; the others are skipped.
+extern "C" int32_t kmc_minhash_sketch_each(kmc_ctx *ctx, const kmc_seqs *seqs, int32_t k, int32_t mode, uint64_t s,
+                                           uint64_t *out_hashes, uint32_t *out_n, kmc_result *result)
+{
+    int32_t st = check_common(ctx, seqs, k);
+    if (st) return st;
+    if (!out_hashes || !out_n || !result) return fail(ctx, KMC_E_BAD_ARG, "out_hashes / out_n / result is NULL");
+    if (mode != KMC_FW && mode != KMC_CANON) return fail(ctx, KMC_E_BAD_ARG, "mode must be KMC_FW or KMC_CANON");
+    if (seqs->src_bits != 2) return fail(ctx, KMC_E_UNSUPPORTED, "the sketch needs a 2-bit source");
+    if (k > 64) return fail(ctx, KMC_E_UNSUPPORTED, "the sketch supports K <= 64");
+    if (s < 1) return fail(ctx, KMC_E_BAD_ARG, "the sketch size must be at least 1");
+    const uint64_t n = seqs->n_seqs;
+    if (n && s > ~0ull / 8 / n) return fail(ctx, KMC_E_BAD_ARG, "n_seqs * s * 8 bytes overflows");
+    memset(result, 0, sizeof *result);
+    if (n == 0) return KMC_OK;
+    CU(cudaSetDevice(ctx->device));
+    const Geometry ge = geometry(k);
+    const bool canon = mode == KMC_CANON;
+    cudaStream_t stream = ctx->stream;
+    CU(cudaEventRecord(ctx->ev_k0, stream));
+    st = ensure_scratch(ctx, layout_scratch_bytes(seqs) + 1024);
+    if (st) return st;
+    st = ensure_host_small(ctx);
+    if (st) return st;
+    Scratch scratch{static_cast<char *>(ctx->scratch), ctx->scratch_bytes, 0};
+    unsigned long long *counters = static_cast<unsigned long long *>(scratch.take(32)); // n_retry, n_total
+    Layout L;
+    st = plan_layout(ctx, seqs, k, ge, stream, KnownTotals(), scratch, &L);
+    if (st) return st;
+    ExtractParams p = base_params(seqs, k, ge, L, 0);
+    const bool ragged = !L.uniform_len;
+    ConsumeLaunchFn count = consume_launcher<OP_SKETCH_COUNT>(ge, ragged, canon);
+    ConsumeLaunchFn append = consume_launcher<OP_SKETCH_APPEND>(ge, ragged, canon);
+    if (!count || !append) return fail(ctx, KMC_E_UNSUPPORTED, "no kernel for this K");
+
+    AsyncBuf lim, cnt, off, cursor, scan_tmp;
+    CU(lim.alloc(ctx, n * 8, stream));
+    CU(cnt.alloc(ctx, n * 8, stream));
+    CU(off.alloc(ctx, (n + 1) * 8, stream));
+    CU(cursor.alloc(ctx, n * 8, stream));
+    CU(scan_tmp.alloc(ctx, scan_tmp_elems(n) * 8, stream));
+    const unsigned blocks = static_cast<unsigned>(std::min<uint64_t>((n + 255) / 256, static_cast<uint64_t>(ctx->sm_count) * 16));
+    sketch_limits_kernel<<<blocks, 256, 0, stream>>>(L.win_off, L.wpr, n, s, lim.as<uint64_t>());
+    CU(cudaGetLastError());
+    CU(cudaMemsetAsync(counters, 0, 16, stream));
+    ConsumeParams c{};
+    c.seq_lim = lim.as<uint64_t>();
+    c.seq_cnt = cnt.as<unsigned long long>();
+    c.seq_cursor = cursor.as<unsigned long long>();
+    constexpr int kMaxRounds = 3; // the first limit, 4x, ~0: the last round flags nothing
+    for (int round = 0; round < kMaxRounds; ++round) {
+        // (1) candidates per sequence, their offsets and total
+        CU(cudaMemsetAsync(cnt.p, 0, n * 8, stream));
+        CU(count(p, c, stream));
+        CU(inclusive_offsets_u64(cnt.as<uint64_t>(), off.as<uint64_t>(), n, scan_tmp.as<uint64_t>(), stream));
+        CU(cudaMemcpyAsync(&ctx->host_small[100], off.as<uint64_t>() + n, 8, cudaMemcpyDeviceToHost, stream));
+        CU(cudaStreamSynchronize(stream));
+        const uint64_t total = ctx->host_small[100];
+        // (2) the candidates into their segments
+        AsyncBuf cand, sorted;
+        CU(cand.alloc(ctx, total * 8, stream));
+        CU(sorted.alloc(ctx, total * 8, stream));
+        c.cand = cand.as<uint64_t>();
+        CU(cudaMemcpyAsync(cursor.p, off.p, n * 8, cudaMemcpyDeviceToDevice, stream));
+        CU(append(p, c, stream));
+        // (3) sort every segment: cub counts items and segments in int, so runs of whole segments of at most 2^31 - 1
+        // candidates each (one download of the offsets when the total is larger)
+        if (total) {
+            std::vector<uint64_t> h_off;
+            if (total > 0x7fffffffull || n > 0x7fffffffull) {
+                h_off.resize(n + 1);
+                CU(cudaMemcpyAsync(h_off.data(), off.p, (n + 1) * 8, cudaMemcpyDeviceToHost, stream));
+                CU(cudaStreamSynchronize(stream));
+            }
+            AsyncBuf seg_off, sort_tmp;
+            const uint64_t max_run = std::min<uint64_t>(n, 0x7ffffffeull);
+            CU(seg_off.alloc(ctx, (max_run + 1) * 4, stream));
+            size_t tmp_bytes = 0;
+            CU(cub::DeviceSegmentedSort::SortKeys(nullptr, tmp_bytes, cand.as<const uint64_t>(), sorted.as<uint64_t>(),
+                                                  static_cast<int>(std::min<uint64_t>(total, 0x7fffffffull)), static_cast<int>(max_run),
+                                                  seg_off.as<int>(), seg_off.as<int>() + 1, stream));
+            CU(sort_tmp.alloc(ctx, tmp_bytes, stream));
+            for (uint64_t seg0 = 0; seg0 < n;) {
+                uint64_t seg1 = n;
+                if (!h_off.empty()) {
+                    seg1 = seg0 + 1;
+                    if (h_off[seg1] - h_off[seg0] > 0x7fffffffull)
+                        return fail(ctx, KMC_E_UNSUPPORTED, "a sequence has more than 2^31 - 1 sketch candidates");
+                    while (seg1 < n && seg1 - seg0 < max_run && h_off[seg1 + 1] - h_off[seg0] <= 0x7fffffffull) ++seg1;
+                }
+                const uint64_t items = h_off.empty() ? total : h_off[seg1] - h_off[seg0];
+                const uint64_t base = h_off.empty() ? 0 : h_off[seg0];
+                const unsigned ob = static_cast<unsigned>(std::min<uint64_t>((seg1 - seg0 + 256) / 256, static_cast<uint64_t>(ctx->sm_count) * 16));
+                segment_offsets_kernel<<<ob, 256, 0, stream>>>(off.as<uint64_t>(), seg0, seg1 - seg0, seg_off.as<int>());
+                CU(cudaGetLastError());
+                if (items)
+                    CU(cub::DeviceSegmentedSort::SortKeys(sort_tmp.p, tmp_bytes, cand.as<const uint64_t>() + base, sorted.as<uint64_t>() + base,
+                                                          static_cast<int>(items), static_cast<int>(seg1 - seg0), seg_off.as<int>(),
+                                                          seg_off.as<int>() + 1, stream));
+                seg0 = seg1;
+            }
+        }
+        // (4) the rows; sequences left short go round again
+        CU(cudaMemsetAsync(counters, 0, 8, stream));
+        const unsigned fb = static_cast<unsigned>(std::min<uint64_t>((n + 7) / 8, static_cast<uint64_t>(ctx->sm_count) * 32));
+        sketch_finish_kernel<<<fb, 256, 0, stream>>>(sorted.as<uint64_t>(), off.as<uint64_t>(), lim.as<uint64_t>(), n, s, round,
+                                                     out_hashes, out_n, counters, counters + 1);
+        CU(cudaGetLastError());
+        CU(cudaMemcpyAsync(&ctx->host_small[100], counters, 16, cudaMemcpyDeviceToHost, stream));
+        CU(cudaStreamSynchronize(stream));
+        const uint64_t n_retry = ctx->host_small[100];
+        if (n_retry == 0) break;
+        result->digest[0] += 1;       // rounds past the first
+        result->digest[1] += n_retry; // sequences sketched again
+    }
+    result->n_written = ctx->host_small[101];
     CU(cudaEventRecord(ctx->ev_k1, stream));
     CU(cudaStreamSynchronize(stream));
     CU(cudaEventElapsedTime(&result->kernel_ms, ctx->ev_k0, ctx->ev_k1));

@@ -105,6 +105,10 @@ SIGNATURES = {
                                    C.POINTER(kmc_out), C.POINTER(kmc_result)]),
     "kmc_minhash_sketch": (C.c_int32, [C.c_void_p, C.POINTER(kmc_seqs), C.c_int32, C.c_int32, C.c_uint64, C.c_void_p,
                                        C.POINTER(kmc_result)]),
+    "kmc_minhash_sketch_each": (C.c_int32, [C.c_void_p, C.POINTER(kmc_seqs), C.c_int32, C.c_int32, C.c_uint64, C.c_void_p,
+                                            C.c_void_p, C.POINTER(kmc_result)]),
+    "kmc_minhash_compare": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint64,
+                                        C.c_uint64, C.c_void_p, C.c_void_p]),
     "kmc_composition": (C.c_int32, [C.c_void_p, C.POINTER(kmc_seqs), C.c_int32, C.c_int32, C.c_void_p,
                                     C.POINTER(kmc_result)]),
     "kmc_kmer_count": (C.c_int32, [C.c_void_p, C.POINTER(kmc_seqs), C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_uint32,

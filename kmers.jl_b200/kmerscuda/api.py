@@ -740,6 +740,83 @@ def minhash_sketch(rs, K: int, s: int, *, canonical: bool = True, ctx: Optional[
     return out
 
 
+def minhash_sketches(rs, K: int, s: int, *, canonical: bool = True, ctx: Optional[Context] = None, stats: bool = False):
+    """The bottom-s sketch of every sequence of the set on its own (kmc_minhash_sketch_each): row i of the u64[n_seqs, s]
+    array is what `minhash_sketch` returns for sequence i alone, padded with ~0; the u32[n_seqs] array holds the row
+    lengths.  stats=True adds a dict: device ms, rounds run past the first and sequences those rounds sketched again."""
+    _check_K(K)
+    ctx = ctx or default_context()
+    drs = rs if isinstance(rs, DeviceReadSet) else DeviceReadSet(ctx, rs)
+    n, s = drs.host.n_seqs, int(s)
+    dh = ctx.alloc(max(n * max(s, 0), 1) * 8)
+    dn = ctx.alloc(max(n, 1) * 4)
+    res = kmc_result()
+    try:
+        ctx._check(ctx.lib.kmc_minhash_sketch_each(ctx.handle, C.byref(drs.desc), K, KMC_CANON if canonical else KMC_FW, s, dh.ptr,
+                                                   dn.ptr, C.byref(res)))
+        rows = dh.download(np.uint64, n * s).reshape(n, s)
+        lens = dn.download(np.uint32, n)
+    finally:
+        dh.free()
+        dn.free()
+    if stats:
+        return rows, lens, {"kernel_ms": float(res.kernel_ms), "extra_rounds": int(res.digest[0]), "resketched": int(res.digest[1]),
+                            "n_written": int(res.n_written)}
+    return rows, lens
+
+
+def minhash_compare(a, a_n, b=None, b_n=None, *, ctx: Optional[Context] = None):
+    """Every sketch of A against every sketch of B (kmc_minhash_compare).  a: u64[n_a, s] rows, ascending and distinct
+    (as `minhash_sketches` returns them), a_n their lengths (a length above s is read as s); b=None compares A with
+    itself.  Returns (shared, shared_bottom), u32[n_a, n_b]: |A_i ∩ B_j| and the number of those among the s smallest
+    values of A_i ∪ B_j."""
+    ctx = ctx or default_context()
+    a = np.ascontiguousarray(a, dtype=np.uint64)
+    a_n = np.ascontiguousarray(a_n, dtype=np.uint32)
+    same = b is None
+    if same:
+        b, b_n = a, a_n
+    b = np.ascontiguousarray(b, dtype=np.uint64)
+    b_n = np.ascontiguousarray(b_n, dtype=np.uint32)
+    if a.ndim != 2 or b.ndim != 2 or a.shape[1] != b.shape[1]:
+        raise ValueError("a and b must be 2-D with the same sketch size s (columns)")
+    if a_n.shape != (a.shape[0],) or b_n.shape != (b.shape[0],):
+        raise ValueError("a_n / b_n must hold one length per row")
+    n_a, n_b, s = a.shape[0], b.shape[0], a.shape[1]
+    bufs = [ctx.to_device(a), ctx.to_device(a_n)]
+    bufs += bufs if same else [ctx.to_device(b), ctx.to_device(b_n)]
+    d_sh, d_bt = ctx.alloc(max(n_a * n_b, 1) * 4), ctx.alloc(max(n_a * n_b, 1) * 4)
+    try:
+        ctx._check(ctx.lib.kmc_minhash_compare(ctx.handle, bufs[0].ptr, bufs[1].ptr, n_a, bufs[2].ptr, bufs[3].ptr, n_b, s,
+                                               d_sh.ptr, d_bt.ptr))
+        shared = d_sh.download(np.uint32, n_a * n_b).reshape(n_a, n_b)
+        bottom = d_bt.download(np.uint32, n_a * n_b).reshape(n_a, n_b)
+    finally:
+        for d in bufs + [d_sh, d_bt]:
+            d.free()
+    return shared, bottom
+
+
+def mash_jaccard(shared, shared_bottom, a_n, b_n, s: int):
+    """Mash's Jaccard estimate per pair: shared_bottom / min(s, n_A + n_B - shared), with the lengths read as at most s
+    (0 where both sketches are empty).  Shapes as `minhash_compare` returns them."""
+    na = np.minimum(np.asarray(a_n, dtype=np.int64), s)[:, None]
+    nb = np.minimum(np.asarray(b_n, dtype=np.int64), s)[None, :]
+    denom = np.minimum(s, na + nb - np.asarray(shared, dtype=np.int64))
+    j = np.zeros(denom.shape, dtype=np.float64)
+    np.divide(np.asarray(shared_bottom, dtype=np.float64), denom, out=j, where=denom > 0)
+    return j
+
+
+def mash_distance(j, K: int):
+    """Mash distance from the Jaccard estimate: -ln(2j / (1 + j)) / K, and 1 where j = 0."""
+    j = np.asarray(j, dtype=np.float64)
+    d = np.ones(j.shape, dtype=np.float64)
+    pos = j > 0
+    d[pos] = -np.log(2.0 * j[pos] / (1.0 + j[pos])) / K
+    return d
+
+
 def composition(rs, K: int, *, canonical: bool = False, ctx: Optional[Context] = None, table: Optional[DeviceBuffer] = None):
     """k-mer composition vector: counts[as_integer(kmer)] over every k-mer of the set
     (docs/src/composition.md:28-39), u32[4^K], K <= 14."""
