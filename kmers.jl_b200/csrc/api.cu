@@ -94,6 +94,8 @@ int32_t plan_layout(kmc_ctx *ctx, const kmc_seqs *s, int k, const Geometry &ge, 
 {
     L->uniform_len = (s->seq_len == nullptr);
     L->uniform_off = (s->seq_word_offset == nullptr);
+    L->tile_first = nullptr;
+    L->tile_buf.reset(); // (a pipeline slot's layout of its previous chunk, whose launches are enqueued)
     const uint64_t G = static_cast<uint64_t>(ge.g);
     if (L->uniform_len) {
         L->wpr = s->uniform_len >= static_cast<uint64_t>(k) ? s->uniform_len - k + 1 : 0;
@@ -133,7 +135,11 @@ int32_t plan_layout(kmc_ctx *ctx, const kmc_seqs *s, int k, const Geometry &ge, 
     const uint64_t tiles = (L->items + kTileItems - 1) / kTileItems;
     if (tiles) {
         uint64_t *tile_first = static_cast<uint64_t *>(scratch.take((tiles + 1) * 8));
-        if (!tile_first) return fail(ctx, KMC_E_BAD_ARG, "internal: scratch window too small");
+        if (!tile_first) { // more tiles than tiles_upper_bound(): sequences that overlap in the buffer
+            L->tile_buf = std::make_shared<AsyncBuf>();
+            CU(L->tile_buf->alloc(ctx, (tiles + 1) * 8, stream));
+            tile_first = L->tile_buf->as<uint64_t>();
+        }
         CU(tile_first_reads(item_off, n, kTileItems, tiles, tile_first, stream));
         L->tile_first = tile_first;
     }

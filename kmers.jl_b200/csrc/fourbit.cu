@@ -341,6 +341,12 @@ int32_t fourbit_phase_a(kmc_ctx *ctx, const kmc_seqs *s, int32_t k, int32_t mode
         const uint64_t tiles = (L.items + kTileItems - 1) / kTileItems;
         st->total_dev = static_cast<unsigned long long *>(scratch.take(8));
         st->tile_state = static_cast<unsigned long long *>(scratch.take(8 * (tiles + 2)));
+        st->tile_state_buf.reset();
+        if (st->total_dev && !st->tile_state) { // more tiles than tiles_upper_bound(): sequences that overlap in the buffer
+            st->tile_state_buf = std::make_shared<AsyncBuf>();
+            CU(st->tile_state_buf->alloc(ctx, 8 * (tiles + 2), stream));
+            st->tile_state = st->tile_state_buf->as<unsigned long long>();
+        }
         if (!st->total_dev || !st->tile_state) return fail(ctx, KMC_E_BAD_ARG, "internal: scratch window too small");
         if (count_first || !out) {
             CU(cudaMemsetAsync(st->total_dev, 0, 8, stream));

@@ -51,6 +51,7 @@ struct FourBitState {
     uint32_t *bad = nullptr;
     uint32_t *err = nullptr; // ASCII UnambiguousKmers: hard-error flags (bytes outside the skipping table)
     unsigned long long *tile_state = nullptr; // UnambiguousKmers: look-back descriptors of compact_kernel
+    std::shared_ptr<AsyncBuf> tile_state_buf; // tile_state when the scratch window cannot hold it (overlapping sequences)
     unsigned long long *total_dev = nullptr;  // UnambiguousKmers: emitted k-mers (device)
     LinPlan lin;                              // UnambiguousKmers: the source-order compaction, when the layout allows it
     bool counted = false;                     // host_small[0] holds the count when phase A has completed

@@ -3,6 +3,7 @@
 // side of the kernel parameter block.  Nothing here computes k-mers on the host.
 #pragma once
 #include <cstring>
+#include <memory>
 
 #include "extract_kernels.cuh"
 #include "kmc_internal.h"
@@ -66,10 +67,15 @@ struct Layout {
     const uint64_t *win_off = nullptr;  // device, ragged
     const uint64_t *item_off = nullptr; // device, ragged
     const uint64_t *tile_first = nullptr; // device, ragged
+    // tile_first when the scratch window cannot hold it (sequences that overlap in the buffer can have more windows
+    // than the buffer has symbols): a temporary from the context's pool, freed (stream-ordered) with the last copy of
+    // the Layout, so after the launches that read it have been enqueued
+    std::shared_ptr<AsyncBuf> tile_buf;
 };
 
-// upper bound of the tiles any layout of this set can need (windows <= symbols, at most two
-// partial group slots per sequence), for scratch sizing before the exact totals are known
+// upper bound of the tiles a layout of sequences that do not overlap in the buffer can need (windows <= symbols, at
+// most two partial group slots per sequence), for scratch sizing before the exact totals are known.  Overlapping
+// sequences can need more: plan_layout() then takes the tile array from the context's pool.
 inline uint64_t tiles_upper_bound(const kmc_seqs *s)
 {
     const uint64_t spu = s->src_bits == 8 ? 1 : s->src_bits == 4 ? 16 : 32; // symbols per unit of n_words
